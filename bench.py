@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- accel_update throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step is ONE accel_update in steady state (subspace full, one eviction per
 call) on synthetic fp64 vectors, n = 2^28, mvec = 10, vtol = 0.01
@@ -51,7 +51,36 @@ def parse_args():
     ap.add_argument("--no-pageable", action="store_true", help="skip the pageable-host-memory e2e figure")
     ap.add_argument("--no-probe", action="store_true", help="skip the cross-rank oracle parity probe")
     ap.add_argument("--no-sweep", action="store_true", help="skip the mvec 2/5/10/20 sweep (N = 1 only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the corrected f of the last timed step to DIR/f.npy (float64; "
+                         "a fixed sample of %d elements when f is longer, see dump_index)" % DUMP_MAX)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1 (the number of timed accel_update calls)")
+    return args
+
+
+# --dump-outputs keeps at most this many doubles (32 MiB), so that two builds can be compared output for output
+DUMP_MAX = 1 << 22
+
+
+def dump_index(n: int):
+    """The positions of a length-n output that --dump-outputs writes, in increasing order: all of them up to
+    DUMP_MAX, else one position drawn with a fixed seed from each of DUMP_MAX equal blocks, so every run
+    with the same n samples the same positions."""
+    import numpy as np
+    if n <= DUMP_MAX:
+        return np.arange(n, dtype=np.int64)
+    edges = np.arange(DUMP_MAX + 1, dtype=np.int64) * n // DUMP_MAX
+    u = np.random.default_rng(12345).random(DUMP_MAX)
+    return edges[:-1] + (u * np.diff(edges)).astype(np.int64)
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def algorithmic_bytes(n: int, m: int) -> int:
@@ -130,12 +159,14 @@ class ClockSampler:
 # --------------------------------------------------------------------------
 # the reference arm / cpu baseline: the reference's own serial C accel_update
 # --------------------------------------------------------------------------
-def cpu_reference_run(n_full: int, mvec: int, steps: int, warmup: int, budget_s: float, n_cap: int = 1 << 26):
+def cpu_reference_run(n_full: int, mvec: int, steps: int, warmup: int, budget_s: float, n_cap: int = 1 << 26,
+                      dump_dir: str | None = None):
     """Time the reference's C accel_update (1 thread: the reference is serial) on a bounded sample
     of the workload: the largest power-of-two length <= n_cap (2^26: BASELINE.md section 3; the
     unmodified source overflows int at (mvec+1)*n >= 2^31, src-C/...c:235,241) whose whole run fits
     in ~budget_s.  Returns updates/s scaled linearly to n_full, labelled as extrapolated, beside
-    the real per-call time of the sample."""
+    the real per-call time of the sample.  With dump_dir, the last timed call's corrected f (of the
+    sample's length) is written there as f.npy."""
     import numpy as np
     from oracle import api
     calls = steps + warmup + mvec + 2
@@ -158,6 +189,8 @@ def cpu_reference_run(n_full: int, mvec: int, steps: int, warmup: int, budget_s:
         acc.accel_update(pool[k % len(pool)])
         k += 1
     dt = time.perf_counter() - t0
+    if dump_dir:
+        write_outputs(dump_dir, {"f": pool[(k - 1) % len(pool)][dump_index(n_s)]})
     nvec = acc.num_vec()
     acc.close()
     ups_sample = steps / dt
@@ -176,7 +209,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    res = cpu_reference_run(args.n, args.mvec, args.steps, args.warmup, budget_s=240.0)
+    res = cpu_reference_run(args.n, args.mvec, args.steps, args.warmup, budget_s=240.0, dump_dir=args.dump_outputs)
     line = {
         "impl": "reference",
         "metric": "accel_update/sec", "value": res["value"], "unit": "updates/s",
@@ -393,6 +426,21 @@ def example_probe(world, rank, local_rank):
             "device_errors": [d["error"] for d in parts], "ok": bool(ok)}
 
 
+def sample_of_slabs(f, lo, hi, n, world, torch):
+    """The dump_index(n) elements of the global vector whose elements lo:hi this rank holds in f (device), on
+    every rank.  Slabs are contiguous and in rank order, so the ranks' parts join in index order."""
+    import numpy as np
+    idx = dump_index(n)
+    mine = idx[(idx >= lo) & (idx < hi)] - lo
+    part = f.index_select(0, torch.from_numpy(mine).to(f.device)).cpu().numpy()
+    if world == 1:
+        return part
+    import torch.distributed as dist
+    parts = [None] * world
+    dist.all_gather_object(parts, part)
+    return np.concatenate(parts)
+
+
 def time_updates(acc, pool, k, steps, stream, torch):
     ev0 = torch.cuda.Event(enable_timing=True)
     ev1 = torch.cuda.Event(enable_timing=True)
@@ -536,6 +584,10 @@ def run_ours(args):
     t_wall1 = time.time()
     elapsed_ms = max_over_ranks(ev0.elapsed_time(ev1))
     launches = acc.launch_count() - launches0
+    if args.dump_outputs:                         # before the steps below overwrite the pool buffers in place
+        f_last = sample_of_slabs(pool[(k - 1) % pool_n], lo, hi, n, world, torch)
+        if rank == 0:
+            write_outputs(args.dump_outputs, {"f": f_last})
 
     # Per-kernel durations (roofline): the same steps again with a CUDA event pair around every
     # launch (the library's timing mode, events on the handle's stream).  Kept out of the headline

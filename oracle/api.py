@@ -17,6 +17,8 @@ from . import build as _build
 
 _dbl_p = C.POINTER(C.c_double)
 _int_p = C.POINTER(C.c_int)
+# the reference's dp hook: double dp(int n, double *x, double *y)
+DP_FUNC = C.CFUNCTYPE(C.c_double, C.c_int, _dbl_p, _dbl_p)
 
 
 def _dp(a: np.ndarray):
@@ -38,6 +40,8 @@ def oracle_lib() -> C.CDLL:
             getattr(lib, name).argtypes = [C.c_void_p]
         lib.orc_nka_accel_update.restype = None
         lib.orc_nka_accel_update.argtypes = [C.c_void_p, _dbl_p]
+        lib.orc_nka_set_dp.restype = None
+        lib.orc_nka_set_dp.argtypes = [C.c_void_p, C.c_void_p]
         lib.orc_nka_set_vec_tol.restype = None
         lib.orc_nka_set_vec_tol.argtypes = [C.c_void_p, C.c_double]
         for name in ("orc_nka_num_vec", "orc_nka_max_vec", "orc_nka_defined", "orc_nka_ndrop_last",
@@ -80,13 +84,18 @@ class OracleNKA:
     """The restatement, with the reference C header's call shapes.
 
     dotmode 0 = the reference's serial sum, 1 = long double accumulation.
-    flavour 0 = C correction statement, 1 = Fortran association."""
+    flavour 0 = C correction statement, 1 = Fortran association.
+    dp = a dot product with the signature of the reference's `dp` hook (a ctypes function
+    pointer, e.g. DP_FUNC(callable)); it replaces every dot product, as in the reference."""
 
-    def __init__(self, vlen: int, mvec: int, vtol: float = 0.01, dotmode: int = 0, flavour: int = 0):
+    def __init__(self, vlen: int, mvec: int, vtol: float = 0.01, dotmode: int = 0, flavour: int = 0, dp=None):
         self._lib = oracle_lib()
         self._h = self._lib.orc_nka_init(vlen, mvec, vtol, dotmode, flavour)
         if not self._h:
             raise ValueError("orc_nka_init rejected its arguments")
+        self._dp = dp                      # keeps a Python callback alive as long as the handle
+        if dp is not None:
+            self._lib.orc_nka_set_dp(self._h, C.cast(dp, C.c_void_p))
         self.vlen, self.mvec = vlen, mvec
 
     def accel_update(self, f: np.ndarray) -> None:
@@ -139,7 +148,6 @@ class OracleNKA:
 
 
 _ref_lib = None
-_DPFUNC = C.CFUNCTYPE(C.c_double, C.c_int, _dbl_p, _dbl_p)
 
 
 def ref_lib() -> C.CDLL | None:

@@ -33,7 +33,8 @@
  *   - slots are 0-based with -1 as the end marker in every flavour;
  *   - the dot product is selectable: 0 = the reference's serial left-to-right
  *     sum (src-C/...c:200-208), 1 = long double accumulation (the arbiter for
- *     n > 2^18, SURVEY.md section 7 hard part 3);
+ *     n > 2^18, SURVEY.md section 7 hard part 3); orc_nka_set_dp installs a
+ *     caller's dp hook instead, as the reference's nka_init does;
  *   - `flavour` picks the correction statement: 0 = C  f += c*(v-w)
  *     (src-C/...c:423), 1 = Fortran  f = f - c*w + c*v (src-F08/...F90:397);
  *   - set_vec_tol/defined exist (Fortran API) although the C header lacks them.
@@ -54,6 +55,7 @@ typedef struct orc_nka {
   int mvec, nslot;       /* nslot = mvec + 1 */
   double vtol;
   int dotmode;           /* 0 serial double, 1 long double */
+  double (*dp)(int, double *, double *);   /* the reference's dp hook; NULL = dotmode */
   int flavour;           /* 0 C, 1 Fortran association in the correction */
   int subspace, pending;
   int first, last, free;
@@ -89,6 +91,8 @@ static double dot_ld(size_t n, const double *a, const double *b)
 
 static double dot(const orc_nka *st, const double *a, const double *b)
 {
+  /* src-C/...c:227-231: a caller-supplied dp replaces every dot product */
+  if (st->dp) return st->dp((int)st->vlen, (double *)a, (double *)b);
   return st->dotmode == 1 ? dot_ld(st->vlen, a, b) : dot_serial(st->vlen, a, b);
 }
 
@@ -101,6 +105,12 @@ double orc_dp_long_double(int len, double *x, double *y)
 }
 
 /* ---- life cycle -------------------------------------------------------- */
+
+/* The reference's dp argument of nka_init (src-C/...c:227-231), set after init; NULL restores dotmode. */
+void orc_nka_set_dp(orc_nka *st, double (*dp)(int, double *, double *))
+{
+  st->dp = dp;
+}
 
 void orc_nka_restart(orc_nka *st);
 

@@ -18,6 +18,10 @@ Writes, next to this file:
   (the oracle port is bit-identical to the reference, so a digest pins it).
 * ``accel_small.npz``        -- full correction vectors for the scenarios with
   n <= 128, for eyeballing and for tolerance tests without the oracle.
+* ``accel_dp_golden.json``   -- the same digests for DP_SCENARIOS with a long-double
+  dot product handed to the reference through its ``dp`` hook: the arbiter the GPU
+  tests compare with.  ``--dp-from-port`` writes this file alone from the port
+  (dotmode = 1) where the reference is not at hand; its "source" field says which.
 """
 from __future__ import annotations
 
@@ -39,9 +43,30 @@ from oracle import api, build  # noqa: E402
 import scenarios as S  # noqa: E402
 
 REF = "/root/reference"
+DP_SCENARIOS = ["picard_n500_m5_v2"]
+
+
+def _digests(acc, ops) -> dict:
+    outs, nvecs = S.run_ops(acc, ops)
+    acc.close()
+    return {"num_vec": nvecs, "sha256": [hashlib.sha256(o.tobytes()).hexdigest() for o in outs]}
+
+
+def write_dp_golden(from_port: bool) -> None:
+    gold = {"source": "oracle port, dotmode=1 (long-double dots)" if from_port
+            else "compiled reference src-C, long-double dp through nka_init's dp hook"}
+    for name in DP_SCENARIOS:
+        n, mvec, vtol, mk = S.SCENARIOS[name]
+        acc = api.OracleNKA(n, mvec, vtol, dotmode=1) if from_port else api.RefNKA(n, mvec, vtol, long_double_dp=True)
+        gold[name] = {"n": n, "mvec": mvec, "vtol": vtol, **_digests(acc, mk())}
+    with open(os.path.join(HERE, "accel_dp_golden.json"), "w") as fh:
+        json.dump(gold, fh, indent=0)
 
 
 def main() -> None:
+    if "--dp-from-port" in sys.argv:
+        write_dp_golden(from_port=True)
+        return
     if not build.reference_available():
         raise SystemExit("needs /root/reference (build container only)")
     built = build.build_all()
@@ -90,6 +115,7 @@ def main() -> None:
     with open(os.path.join(HERE, "accel_golden.json"), "w") as fh:
         json.dump(gold, fh, indent=0)
     np.savez_compressed(os.path.join(HERE, "accel_small.npz"), **small)
+    write_dp_golden(from_port=False)
     print("wrote goldens for %d scenarios" % len(gold))
 
 

@@ -2,12 +2,13 @@
 
 Per scenario: how far the CUDA path is from the long-double arbiter and from the unmodified
 (serial-sum) reference, beside the tolerance that was applied.  Written at session end to
-gpurun_out/parity_errors.json (scratch that comes back from the GPU box) and merged into
+build/parity_errors.json (a run's output, kept out of git); tools/merge_parity.py merges it into
 profiles/parity_errors.json (the copy that is committed)."""
 import json
 import os
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+PATH = os.path.join(ROOT, "build", "parity_errors.json")
 _PARITY = {}
 WHAT = ("max over the calls of a scenario of ||got - ref|| / max(||ref||, ||f_in||); arbiter = the reference "
         "algorithm with long-double dot products (its dp hook), serial = the unmodified reference (serial sums)")
@@ -20,19 +21,17 @@ def record_parity(name: str, **fields) -> None:
 def flush() -> None:
     if not _PARITY:
         return
-    for d in ("gpurun_out", "profiles"):
-        try:
-            os.makedirs(os.path.join(ROOT, d), exist_ok=True)
-            path = os.path.join(ROOT, d, "parity_errors.json")
-            old = {}
-            if os.path.exists(path):
-                try:
-                    with open(path) as fh:
-                        old = json.load(fh).get("scenarios", {})
-                except Exception:
-                    old = {}
-            old.update(_PARITY)
-            with open(path, "w") as fh:
-                json.dump({"what": WHAT, "scenarios": dict(sorted(old.items()))}, fh, indent=1)
-        except OSError:
-            pass
+    try:
+        os.makedirs(os.path.dirname(PATH), exist_ok=True)
+        old = {}
+        if os.path.exists(PATH):
+            try:
+                with open(PATH) as fh:
+                    old = json.load(fh).get("scenarios", {})
+            except Exception:
+                old = {}
+        old.update(_PARITY)
+        with open(PATH, "w") as fh:
+            json.dump({"what": WHAT, "scenarios": dict(sorted(old.items()))}, fh, indent=1)
+    except OSError:
+        pass

@@ -190,7 +190,7 @@ def tolerances(serial, arbiter, inputs, factor=4.0):
     Factor 4: call by call the CUDA path is at most 2.6 times as far from the arbiter as the
     reference's serial run has been up to that call (contraction_n50_m8; 2.3 for
     contraction_n200_m5; 0.57 for collinear_n300_m6; every other scenario passes at the plain 1e-12) --
-    `worst_ratio_to_reference_spread` in profiles/parity_errors.json, written by the GPU run; a
+    `worst_ratio_to_reference_spread` in profiles/parity_errors.json, merged from the GPU run's table; a
     factor of 2 fails those two.  The
     sensitivity is carried forward as a running maximum because a perturbed stored
     vector keeps influencing later calls.  Returns (scales, rel_tols)."""

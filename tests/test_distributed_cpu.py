@@ -2,7 +2,8 @@
 
 The CUDA path cannot run here, so this checks what surrounds it: the slab partition, the
 id exchange over torch.distributed, and -- with the REFERENCE's own C accelerator driven
-through its `dp` hook by a gloo all-reduce -- that "each rank updates its slab, dot products
+through its `dp` hook by a gloo all-reduce (oracle/_ref, when built; else the port, pinned
+bit-identical to it, through the same hook) -- that "each rank updates its slab, dot products
 are summed over ranks" reproduces the serial full-vector update exactly as the reference
 promises (src-F08-vector/README.md:16-22).  That is the contract libnka_b200's NCCL path
 implements on the GPUs (checked for real by tests/test_gpu_multi.py)."""
@@ -54,33 +55,40 @@ def _worker(rank, world, port, n, mvec, q):
         uid = exchange_unique_id()
         lo, hi = slab_bounds(n, world, rank)
         lib = api.ref_lib()
-        have_ref = lib is not None
         flags = [None] * world
-        dist.all_gather_object(flags, have_ref)
-        results = {"uid": uid, "bounds": (lo, hi)}
+        dist.all_gather_object(flags, lib is not None)
+        results = {"uid": uid, "bounds": (lo, hi), "impl": "reference" if all(flags) else "port"}
+
+        def global_dot(length, x, y):
+            a = np.ctypeslib.as_array(x, shape=(length,)) if length else np.zeros(0)
+            b = np.ctypeslib.as_array(y, shape=(length,)) if length else np.zeros(0)
+            t = torch.tensor([float(np.dot(a, b))], dtype=torch.float64)
+            dist.all_reduce(t)
+            return float(t.item())
+
+        cb = api.DP_FUNC(global_dot)
         if all(flags):
-            DP = C.CFUNCTYPE(C.c_double, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double))
-
-            def global_dot(length, x, y):
-                a = np.ctypeslib.as_array(x, shape=(length,)) if length else np.zeros(0)
-                b = np.ctypeslib.as_array(y, shape=(length,)) if length else np.zeros(0)
-                t = torch.tensor([float(np.dot(a, b))], dtype=torch.float64)
-                dist.all_reduce(t)
-                return float(t.item())
-
-            cb = DP(global_dot)
             h = lib.nka_init(hi - lo, mvec, 0.01, C.cast(cb, C.c_void_p))
-            rng = np.random.default_rng(77)
-            outs, nvec = [], []
-            for t in range(mvec + 5):
-                full = rng.uniform(-0.5, 0.5, n) * 0.8 ** t
-                mine = np.ascontiguousarray(full[lo:hi])
-                lib.nka_accel_update(h, mine.ctypes.data_as(C.POINTER(C.c_double)))
-                outs.append(mine)
-                nvec.append(lib.nka_num_vec(h))
+            update = lambda f: lib.nka_accel_update(h, f.ctypes.data_as(C.POINTER(C.c_double)))
+            num_vec = lambda: lib.nka_num_vec(h)
+        else:
+            # without the compiled reference: the port, which routes every dot product through the same hook
+            acc = api.OracleNKA(hi - lo, mvec, 0.01, dp=cb)
+            update, num_vec = acc.accel_update, acc.num_vec
+        rng = np.random.default_rng(77)
+        outs, nvec = [], []
+        for t in range(mvec + 5):
+            full = rng.uniform(-0.5, 0.5, n) * 0.8 ** t
+            mine = np.ascontiguousarray(full[lo:hi])
+            update(mine)
+            outs.append(mine)
+            nvec.append(num_vec())
+        if all(flags):
             lib.nka_delete(h)
-            results["outs"] = outs
-            results["nvec"] = nvec
+        else:
+            acc.close()
+        results["outs"] = outs
+        results["nvec"] = nvec
         q.put((rank, results))
     finally:
         dist.destroy_process_group()
@@ -90,6 +98,7 @@ def test_two_rank_slab_update_equals_serial_update():
     import torch.multiprocessing as mp
     from oracle import api
     n, mvec, world = 1001, 4, 2
+    api.oracle_lib()            # built here, once: two ranks compiling it at the same time could load a partial file
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
@@ -103,8 +112,7 @@ def test_two_rank_slab_update_equals_serial_update():
     # the 128-byte id reached both ranks unchanged
     assert got[0]["uid"] == got[1]["uid"] and len(got[0]["uid"]) == 128
     assert got[0]["bounds"][1] == got[1]["bounds"][0]
-    if "outs" not in got[0]:
-        pytest.skip("oracle/_ref not built in this tree")
+    assert got[0]["impl"] == got[1]["impl"]
     # serial reference on the full vectors (long-double dots: summation order differs across the split)
     ser = api.OracleNKA(n, mvec, 0.01, dotmode=1)
     rng = np.random.default_rng(77)

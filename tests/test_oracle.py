@@ -1,9 +1,11 @@
 """Pin the oracle: the C restatement against the reference's own golden
 tables and against outputs of the compiled reference (SURVEY.md 8c).
 
-CPU only.  The goldens under tests/golden/ were produced from /root/reference
-by tests/golden/make_golden.py; nothing here reads /root/reference.
+CPU only.  The goldens under tests/golden/ were produced by tests/golden/make_golden.py
+from the reference's sources and compiled library (accel_dp_golden.json names its own
+source); nothing here reads the reference's sources.
 """
+import ctypes as C
 import hashlib
 import json
 import os
@@ -109,11 +111,25 @@ def test_flavours_differ_only_by_rounding():
         assert np.linalg.norm(x - y) <= 1e-14 * np.linalg.norm(x)
 
 
+with open(os.path.join(GOLD, "accel_dp_golden.json")) as _fh:
+    _GOLD_DP = json.load(_fh)
+
+
 def test_compiled_reference_matches_port_when_present():
-    """If oracle/_ref/libnka_ref.so travelled with the tree, cross-check live."""
-    if api.ref_lib() is None:
-        pytest.skip("oracle/_ref not built in this tree")
+    """The long-double arbiter (the port with dotmode = 1, and the port with the same dot product
+    handed to its dp hook) reproduces the stored digests of every call and num_vec; the file's
+    "source" says what produced them.  If oracle/_ref/libnka_ref.so travelled with the tree, the
+    reference itself is cross-checked live as well, in serial mode and through its dp hook."""
     n, mvec, vtol, mk = S.SCENARIOS["picard_n500_m5_v2"]
+    g = _GOLD_DP["picard_n500_m5_v2"]
+    assert (g["n"], g["mvec"], g["vtol"]) == (n, mvec, vtol)
+    hook = C.cast(api.oracle_lib().orc_dp_long_double, C.c_void_p)
+    for acc in (api.OracleNKA(n, mvec, vtol, dotmode=1), api.OracleNKA(n, mvec, vtol, dp=hook)):
+        outs, nvecs = S.run_ops(acc, mk())
+        assert nvecs == g["num_vec"]
+        assert [hashlib.sha256(o.tobytes()).hexdigest() for o in outs] == g["sha256"]
+    if api.ref_lib() is None:
+        return
     a, nva = S.run_ops(api.RefNKA(n, mvec, vtol), mk())
     b, nvb = S.run_ops(api.OracleNKA(n, mvec, vtol), mk())
     assert nva == nvb

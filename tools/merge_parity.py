@@ -1,10 +1,10 @@
-"""Merge the achieved-error table a GPU run brought back (gpurun_out/parity_errors.json) into the committed copy
+"""Merge the achieved-error table of a GPU test run (build/parity_errors.json) into the committed copy
 (profiles/parity_errors.json): entries of the new run replace older ones of the same name."""
 import json
 import os
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-new = json.load(open(os.path.join(ROOT, "gpurun_out", "parity_errors.json")))
+new = json.load(open(os.path.join(ROOT, "build", "parity_errors.json")))
 path = os.path.join(ROOT, "profiles", "parity_errors.json")
 old = json.load(open(path)) if os.path.exists(path) else {"what": new["what"], "scenarios": {}}
 old["what"] = new["what"]
