@@ -154,6 +154,7 @@ struct nka_state {
   bool pending = false;
   int ub_len = 0;
   bool lazy = true;             // skip the doomed oldest column in pass A (single GPU only)
+  bool poison = false;          // NKA_POISON_ALLOC=1 (tests): data buffers start as NaN bytes, see poison_fill
   // the reference's dp hook: global sum of each partial dot product through a host callback
   double (*dp)(int, double*, double*) = nullptr;
   double (*dp_ctx)(int, double*, double*, void*) = nullptr;
@@ -392,6 +393,15 @@ static bool peer_setup(NKA st)
 // ---------------------------------------------------------------------------
 // construction / destruction
 // ---------------------------------------------------------------------------
+// Test switch NKA_POISON_ALLOC=1: fill a freshly allocated data buffer with 0xFF bytes (a NaN for
+// fp64) instead of leaving it as cudaMalloc returns it, which usually reads as zero.  A kernel that
+// reads a value it has not written then yields NaN in place of a silent zero.  Only buffers of
+// values are filled: never the state, the ticket or anything else read as an index or a counter.
+static void poison_fill(NKA st, void* p, size_t bytes)
+{
+  if (st->poison) CUDA_CHECK(cudaMemsetAsync(p, 0xFF, bytes, st->stream));
+}
+
 extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void* stream)
 {
   // preconditions: src-C/...c:217-219 ; src-F08/nka_type.F90:190-191,205
@@ -421,6 +431,7 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
   for (int i = 0; i <= NKA_MAXSLOT; ++i)
     for (int v = 0; v < 3; ++v) { st->occ_a[i][v] = -1; st->occ_b[i][v] = -1; }
   if (const char* e = getenv("NKA_LAZY_LAST")) st->lazy = atoi(e) != 0;      // ablation switch
+  if (const char* e = getenv("NKA_POISON_ALLOC")) st->poison = atoi(e) != 0;
 
   const size_t colbytes = st->ld * sizeof(double);
   const size_t poolbytes = colbytes * (size_t)(mvec + 1);
@@ -439,6 +450,10 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
   CUDA_CHECK(cudaMalloc(&st->ticket, sizeof(unsigned)));
   CUDA_CHECK(cudaMemsetAsync(st->ticket, 0, sizeof(unsigned), st->stream));
   CUDA_CHECK(cudaMemsetAsync(st->dots, 0, 2 * NKA_MAXSLOT * sizeof(double), st->stream));
+  poison_fill(st, st->W, poolbytes);
+  poison_fill(st, st->Z, poolbytes);
+  poison_fill(st, st->partials, (size_t)st->max_grid * 2 * NKA_MAXSLOT * sizeof(double));
+  poison_fill(st, st->dots, 2 * NKA_MAXSLOT * sizeof(double));
   nka_init_kernel<<<1, 32, 0, st->stream>>>(st->S, mvec, vtol, st->lazy ? 1 : 0);
   CUDA_CHECK(cudaGetLastError());
   st->launches += 1;
@@ -690,7 +705,10 @@ extern "C" void nka_accel_update_host(NKA st, double* f)
   NkaRange nvtx("nka:accel_update(host f: h2d | sweeps | d2h, pipelined)");
   const size_t n = st->vlen;
   const size_t bytes = n * sizeof(double);
-  if (!st->fstage) CUDA_CHECK(cudaMalloc(&st->fstage, bytes ? bytes : 16));
+  if (!st->fstage) {
+    CUDA_CHECK(cudaMalloc(&st->fstage, bytes ? bytes : 16));
+    poison_fill(st, st->fstage, bytes ? bytes : 16);
+  }
   if (st->host_chunk_bytes == 0) {
     st->host_chunk_bytes = NKA_HOST_CHUNK_BYTES;
     if (const char* e = getenv("NKA_HOST_CHUNK_BYTES")) if (atoll(e) >= 128) st->host_chunk_bytes = (size_t)atoll(e);   // tests

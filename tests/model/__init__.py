@@ -33,13 +33,16 @@ def lib():
             getattr(L, nm).restype = None
         for nm in ("model_num_vec", "model_defined", "model_bound_violations", "model_error", "model_ndrop_last",
                    "model_relaxed_last", "model_evicted_last", "model_host_pending", "model_dev_pending",
-                   "model_list_len", "model_ub_len"):
+                   "model_list_len", "model_ub_len", "model_plan_a_ncol", "model_plan_a_skip_last",
+                   "model_plan_b_nz", "model_plan_b_has_pair", "model_plan_b_write_f", "model_plan_m_n"):
             getattr(L, nm).argtypes = [C.c_void_p]
             getattr(L, nm).restype = C.c_int
         L.model_mat_entries.argtypes = [C.c_void_p]
         L.model_mat_entries.restype = C.c_ulonglong
         L.model_fixups.argtypes = [C.c_void_p]
         L.model_fixups.restype = C.c_ulonglong
+        L.model_plan_a_submask.argtypes = [C.c_void_p]
+        L.model_plan_a_submask.restype = C.c_ulonglong
         L.model_set_lazy.argtypes = [C.c_void_p, C.c_int]
         L.model_set_lazy.restype = None
         L.model_min_margin.argtypes = [C.c_void_p]
@@ -79,6 +82,17 @@ class ModelNKA:
     def dev_pending(self): return self._lib.model_dev_pending(self._h)
     def list_len(self): return self._lib.model_list_len(self._h)
     def ub_len(self): return self._lib.model_ub_len(self._h)
+
+    def plan_a(self):
+        """Plan A as the next pass A reads it: (ncol, skip_last, submask)."""
+        L = self._lib
+        return L.model_plan_a_ncol(self._h), L.model_plan_a_skip_last(self._h), L.model_plan_a_submask(self._h)
+
+    def plan_b(self):
+        """Plans B and M as the last update left them: (nz, has_pair, write_f, planM.n)."""
+        L = self._lib
+        return (L.model_plan_b_nz(self._h), L.model_plan_b_has_pair(self._h), L.model_plan_b_write_f(self._h),
+                L.model_plan_m_n(self._h))
 
     def __del__(self):
         try:

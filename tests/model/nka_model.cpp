@@ -16,6 +16,15 @@
 
 #include "../../nka_b200/csrc/nka_state.h"
 
+// How the state step is executed: by one thread here; tests/model/lanes_test.cpp runs it on
+// several host threads instead, to check that the result does not depend on the lane count.
+typedef int (*ModelStepFn)(NkaDevState& S, NkaStepScratch& X, const double* dots, int have_last);
+
+static int serial_step(NkaDevState& S, NkaStepScratch& X, const double* dots, int have_last)
+{
+  return nka_state_step(S, X, dots, NKA_MAXSLOT, have_last, NkaSerial());
+}
+
 struct Model {
   size_t n, ld;
   int mvec;
@@ -30,6 +39,7 @@ struct Model {
   unsigned long long mat_entries;
   unsigned long long fixups;
   bool lazy;
+  ModelStepFn step;
 };
 
 static void pass_a(Model* m, const double* f)
@@ -105,7 +115,9 @@ static void pass_b(Model* m, double* f)
 
 extern "C" {
 
-Model* model_init(size_t n, int mvec, double vtol)
+// poison = 1: the state and the step's scratch start as 0xFF bytes (NaN doubles, -1 ints), as
+// uninitialised device memory may, so that init has to set everything the step reads.
+Model* model_init_ex(size_t n, int mvec, double vtol, int poison)
 {
   if (mvec < 1 || mvec + 1 > NKA_MAXSLOT || !(vtol > 0.0)) return nullptr;
   Model* m = new Model();
@@ -113,10 +125,17 @@ Model* model_init(size_t n, int mvec, double vtol)
   m->mvec = mvec;
   m->W.assign(m->ld * (mvec + 1), 0.0);
   m->Z.assign(m->ld * (mvec + 1), 0.0);
+  if (poison) {
+    memset(&m->S, 0xFF, sizeof m->S);
+    memset(&m->scratch, 0xFF, sizeof m->scratch);
+  }
   nka_state_init(m->S, mvec, vtol);
   m->pending = false; m->ub_len = 0; m->bound_violations = 0; m->mat_entries = 0; m->fixups = 0; m->lazy = true;
+  m->step = serial_step;
   return m;
 }
+
+Model* model_init(size_t n, int mvec, double vtol) { return model_init_ex(n, mvec, vtol, 0); }
 
 void model_delete(Model* m) { delete m; }
 
@@ -130,16 +149,16 @@ void model_accel_update(Model* m, double* f)
   if (L > 0) {
     pass_a(m, f);
     NkaDevState copy = m->S;                       // the device works on a staged copy
-    if (nka_state_step(copy, m->scratch, m->dots, NKA_MAXSLOT, 0, NkaSerial())) {
+    if (m->step(copy, m->scratch, m->dots, 0)) {
       if (!may_skip) m->bound_violations++;        // the host must have queued the fix-up kernel
       m->S.need_fixup = 1;
       fixup(m, f);
       copy = m->S;
-      if (nka_state_step(copy, m->scratch, m->dots, NKA_MAXSLOT, 1, NkaSerial())) m->bound_violations++;
+      if (m->step(copy, m->scratch, m->dots, 1)) m->bound_violations++;
     }
     m->S = copy;
   } else {
-    nka_state_step(m->S, m->scratch, m->dots, NKA_MAXSLOT, 1, NkaSerial());
+    m->step(m->S, m->scratch, m->dots, 1);
   }
   pass_b(m, f);
   if (m->pending) m->ub_len = L + 1 < m->mvec + 1 ? L + 1 : m->mvec + 1;
@@ -181,5 +200,15 @@ int model_host_pending(Model* m) { return m->pending ? 1 : 0; }
 int model_dev_pending(Model* m) { return m->S.pending; }
 int model_list_len(Model* m) { int n = 0; for (int k = m->S.first; k != NKA_NIL; k = m->S.next[k]) ++n; return n; }
 int model_ub_len(Model* m) { return m->ub_len; }
+
+// The plans, for tests that work out which kernel instantiation and body the device runs:
+// plan A as pass A will read it on the next update, plans B and M as the last update left them.
+int model_plan_a_ncol(Model* m) { return m->S.planA.ncol; }
+int model_plan_a_skip_last(Model* m) { return m->S.planA.skip_last; }
+unsigned long long model_plan_a_submask(Model* m) { return m->S.planA.submask; }
+int model_plan_b_nz(Model* m) { return m->S.planB.nz; }
+int model_plan_b_has_pair(Model* m) { return m->S.planB.has_pair; }
+int model_plan_b_write_f(Model* m) { return m->S.planB.write_f; }
+int model_plan_m_n(Model* m) { return m->S.planM.n; }
 
 }  // extern "C"
