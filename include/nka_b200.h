@@ -62,6 +62,28 @@ void *nka_get_stream (NKA);
 /* Block until everything queued on the handle's stream has finished. */
 void nka_synchronize (NKA);
 
+/* ---- CUDA graphs -------------------------------------------------------- */
+/* nka_accel_update_dev (and nka_accel_update with a device pointer,
+ * nka_accel_update_vec), nka_relax, nka_restart and nka_set_vec_tol can be
+ * captured in a stream capture (cudaStreamBeginCapture, torch.cuda.graph) of
+ * the handle's stream, which must be set with nka_set_stream before the
+ * capture begins (not the legacy default stream).  The graph holds f's device
+ * address.  A capture does not run anything: it leaves nka_launch_count and the
+ * timing unchanged.  The first capture switches the handle for good to the
+ * capacity shape, a launch shape valid for any list state (pass A at full width,
+ * the fix-up kernel always queued, pass B at mvec pairs), for eager calls too;
+ * in steady state it is the shape an eager call uses anyway.  Calls that
+ * synchronise or stage through the host abort with a message while the
+ * handle's stream captures: nka_accel_update_host (and a host pointer), an
+ * update on a handle with a dot-product callback, nka_num_vec, nka_defined,
+ * nka_get_state, nka_timing_*, nka_set_stream, nka_synchronize,
+ * nka_set_dot_prod*, nka_comm_init / nka_comm_adopt.  With several ranks,
+ * every rank captures and replays the same graphs in the same order.
+ * Returns 1 while the handle's stream is capturing, 0 when it is not, -1 when
+ * the handle is on the legacy default stream while a blocking stream captures
+ * (nothing can be queued on the handle then). */
+int nka_stream_capturing (NKA);
+
 /* ---- multi-GPU: one process per GPU, each holding a row slab ------------ */
 /* The only exchange in accel_update is one fp64 sum-allreduce of the
  * 2*(mvec+1) partial dot products (the reference's `dp` hook contract:
@@ -125,13 +147,15 @@ typedef struct nka_state_view {
 
 void nka_get_state (NKA, nka_state_view *out);
 
-/* Kernel launches issued by this handle so far (all of them ours). */
+/* Kernel launches issued by this handle so far (all of them ours); kernels
+ * captured into a CUDA graph are not launches and are not counted. */
 unsigned long long nka_launch_count (NKA);
 
 /* Per-kernel device timing with CUDA events on the handle's stream.
  * which: 0 = pass A, 1 = state, 2 = materialise, 3 = pass B, 4 = allreduce.
  * nka_timing_read synchronises the stream and returns accumulated ms and
- * launch counts since the last nka_timing_reset. */
+ * launch counts since the last nka_timing_reset (eager calls only: a graph
+ * replay records no events). */
 void nka_timing_enable (NKA, int on);
 void nka_timing_reset (NKA);
 void nka_timing_read (NKA, double ms[5], unsigned long long count[5]);

@@ -50,6 +50,7 @@ SYMBOLS = {
     "nka_set_stream": (None, [C.c_void_p, C.c_void_p]),
     "nka_get_stream": (C.c_void_p, [C.c_void_p]),
     "nka_synchronize": (None, [C.c_void_p]),
+    "nka_stream_capturing": (C.c_int, [C.c_void_p]),
     "nka_comm_unique_id": (C.c_int, [C.c_void_p]),
     "nka_comm_init": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "nka_comm_adopt": (None, [C.c_void_p, C.c_void_p, C.c_int, C.c_int]),

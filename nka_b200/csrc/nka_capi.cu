@@ -153,6 +153,10 @@ struct nka_state {
   // host-side knowledge of the device list: exact `pending`, upper bound on its length
   bool pending = false;
   int ub_len = 0;
+  // CUDA graphs: a replay runs on whatever the list holds by then, and the host never sees it.  Once a
+  // call has been captured the handle stops tracking the list and launches the capacity shape for good.
+  bool captured = false;        // some call on this handle has been captured
+  bool in_capture = false;      // the current call is being captured: no bookkeeping, spans or launch counts
   bool lazy = true;             // skip the doomed oldest column in pass A (single GPU only)
   bool poison = false;          // NKA_POISON_ALLOC=1 (tests): data buffers start as NaN bytes, see poison_fill
   // the reference's dp hook: global sum of each partial dot product through a host callback
@@ -204,7 +208,7 @@ static void fold_timing(NKA st)
 struct SpanScope {
   NKA st; int kind; cudaEvent_t beg = nullptr;
   SpanScope(NKA s, int k) : st(s), kind(k) {
-    if (st->timing) { beg = get_event(st); CUDA_CHECK(cudaEventRecord(beg, st->stream)); }
+    if (st->timing && !st->in_capture) { beg = get_event(st); CUDA_CHECK(cudaEventRecord(beg, st->stream)); }
   }
   ~SpanScope() {
     if (beg) {
@@ -214,6 +218,56 @@ struct SpanScope {
       if (st->spans.size() >= 8192) fold_timing(st);
     }
   }
+};
+
+// A captured node is not a launch: nka_launch_count counts what ran eagerly.
+static void count_launch(NKA st)
+{
+  if (!st->in_capture) st->launches += 1;
+}
+
+// ---------------------------------------------------------------------------
+// stream capture (CUDA graphs)
+// ---------------------------------------------------------------------------
+// 1: the handle's stream is capturing (an invalidated capture counts: it has not ended yet);
+// 0: it is not; -1: the handle is on the legacy default stream while a blocking stream captures,
+// so nothing can be queued on it.
+static int capture_status(NKA st)
+{
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  const cudaError_t e = cudaStreamIsCapturing(st->stream, &cs);
+  if (e == cudaErrorStreamCaptureImplicit) { cudaGetLastError(); return -1; }
+  CUDA_CHECK(e);
+  return cs == cudaStreamCaptureStatusNone ? 0 : 1;
+}
+
+[[noreturn]] static void capture_fail(const char* call, const char* why)
+{
+  char b[320];
+  snprintf(b, sizeof b, "%s cannot be captured in a CUDA graph: %s", call, why);
+  nka_fail(__FILE__, __LINE__, b);
+}
+
+// Calls that synchronise, read the device state back or stage through the host: refused while the
+// handle's stream captures, before anything reaches the stream (it would invalidate the capture).
+static void refuse_capture(NKA st, const char* call, const char* why)
+{
+  if (capture_status(st) != 0) capture_fail(call, why);
+}
+
+// Around a call that can be captured (update, relax, restart, set_vec_tol).  The first capture
+// marks the handle: from then on every call, captured or eager, uses the capacity shape.
+struct CaptureScope {
+  NKA st;
+  CaptureScope(NKA s, const char* call) : st(s) {
+    const int c = capture_status(st);
+    if (c < 0)
+      capture_fail(call, "the handle is on the legacy default stream while another stream captures; "
+                         "nka_set_stream to the capture stream before the capture begins");
+    st->in_capture = c > 0;
+    if (st->in_capture) st->captured = true;
+  }
+  ~CaptureScope() { st->in_capture = false; }
 };
 
 static int grid_for(NKA st, int per_sm, size_t n, int V, int threads = NKA_THREADS)
@@ -444,6 +498,13 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
     nka_fail(__FILE__, __LINE__, b);
   }
   st->max_grid = st->num_sms * 32;
+  // the occupancy of the capacity shape's kernels, queried now: never from inside a capture
+  // (tuning builds instantiate fewer sizes: those they lack fail later, on use, as before)
+  for (int V = 1; V <= 2; ++V) {
+    if (nka_get_pass_a(mvec, V)) resident_a(st, mvec, V);
+    if (nka_get_pass_a(mvec + 1, V)) resident_a(st, mvec + 1, V);
+    if (nka_get_pass_b(mvec, V)) resident_b(st, mvec, V);
+  }
   CUDA_CHECK(cudaMalloc(&st->S, sizeof(NkaDevState)));
   CUDA_CHECK(cudaMalloc(&st->dots, 2 * NKA_MAXSLOT * sizeof(double)));
   CUDA_CHECK(cudaMalloc(&st->partials, (size_t)st->max_grid * 2 * NKA_MAXSLOT * sizeof(double)));
@@ -456,7 +517,7 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
   poison_fill(st, st->dots, 2 * NKA_MAXSLOT * sizeof(double));
   nka_init_kernel<<<1, 32, 0, st->stream>>>(st->S, mvec, vtol, st->lazy ? 1 : 0);
   CUDA_CHECK(cudaGetLastError());
-  st->launches += 1;
+  count_launch(st);
   st->pending = false;
   st->ub_len = 0;
   return st;
@@ -467,7 +528,7 @@ static void set_lazy(NKA st, bool on)
   st->lazy = on;
   nka_set_lazy_kernel<<<1, 32, 0, st->stream>>>(st->S, on ? 1 : 0);
   CUDA_CHECK(cudaGetLastError());
-  st->launches += 1;
+  count_launch(st);
 }
 
 static void install_dp(NKA st, double (*dp)(int, double*, double*), double (*dp_ctx)(int, double*, double*, void*), void* user)
@@ -475,6 +536,7 @@ static void install_dp(NKA st, double (*dp)(int, double*, double*), double (*dp_
   NKA_REQUIRE(st->comm == nullptr || (!dp && !dp_ctx),
               "nka_set_dot_prod: the handle already sums over ranks through nka_comm_init; use one or the other");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_set_dot_prod", "it changes the launch shape the host chooses for later updates");
   st->dp = dp; st->dp_ctx = dp_ctx; st->dp_user = user;
   // the lazily skipped oldest column would need a second, conditional reduction: not with a host callback
   bool lazy = !(dp || dp_ctx);
@@ -543,10 +605,21 @@ static UpdateShape update_shape(NKA st, const double* f)
 {
   UpdateShape u;
   u.V = (((uintptr_t)f) % 16 == 0) ? 2 : 1;
-  u.L = st->ub_len;                               // upper bound on the list length at entry
   // fused = the dot products are complete when pass A's last CTA has them (single GPU, or
   // summed over the ranks through peer memory inside pass A): state step in place, lazy last column
   u.fused = ((st->comm == nullptr) || (st->peer != nullptr)) && !st->dp && !st->dp_ctx;
+  if (st->captured) {
+    // The capacity shape, valid for any list: pass A always runs (on an empty list the state step
+    // ignores the dots), wide enough for a full list, the fix-up is always queued where the lazy
+    // column applies (it exits at once unless needed), pass B takes up to mvec pairs.  With a full,
+    // pending list, which is the steady state, it is exactly the shape below.
+    u.L = st->mvec + 1;
+    u.may_skip = u.fused && st->lazy;
+    u.NC = u.may_skip ? st->mvec : st->mvec + 1;
+    u.nz = st->mvec;
+    return u;
+  }
+  u.L = st->ub_len;                               // upper bound on the list length at entry
   u.may_skip = u.fused && st->lazy && st->pending && u.L == st->mvec + 1;
   u.NC = u.may_skip ? st->mvec : u.L;             // columns pass A can be asked to stream
   u.nz = nz_expected(st);
@@ -566,7 +639,7 @@ static int launch_pass_a(NKA st, const UpdateShape& u, double* f, size_t off, si
   launch_chained(nka_get_pass_a(u.NC, u.V), grid, NKA_THREADS_A, st->stream,
                  f + off, st->W + off, st->ld, len, st->S, rows, st->ticket, st->dots, u.fused ? 1 : 0, st->peer,
                  st->partials, final ? (unsigned)(row0 + grid) : 0u);
-  st->launches += 1;
+  count_launch(st);
   return grid;
 }
 
@@ -596,7 +669,7 @@ static void launch_mid(NKA st, const UpdateShape& u, double* f)
       }
       SpanScope t(st, T_STATE);
       launch_chained(nka_state_kernel, 1, NKA_STATE_THREADS, st->stream, st->S, st->dots, 1);
-      st->launches += 1;
+      count_launch(st);
     } else if (!u.fused) {
       {
         SpanScope t(st, T_COMM);
@@ -605,19 +678,19 @@ static void launch_mid(NKA st, const UpdateShape& u, double* f)
       }
       SpanScope t(st, T_STATE);
       launch_chained(nka_state_kernel, 1, NKA_STATE_THREADS, st->stream, st->S, st->dots, 1);
-      st->launches += 1;
+      count_launch(st);
     } else if (u.may_skip) {
       // the oldest column was left out of pass A; this exits at once unless a vtol drop
       // (or the s == 0 guard) means it is needed after all
       SpanScope t(st, T_STATE);
       launch_chained(nka_fixup_kernel, grid_for(st, 4, n, 1), NKA_THREADS, st->stream, f, st->W, st->ld, n, st->S,
                      st->partials, st->ticket, st->dots, st->peer);
-      st->launches += 1;
+      count_launch(st);
     }
   } else {
     SpanScope t(st, T_STATE);
     launch_chained(nka_state_kernel, 1, NKA_STATE_THREADS, st->stream, st->S, st->dots, 1);
-    st->launches += 1;
+    count_launch(st);
   }
 }
 
@@ -631,18 +704,19 @@ static void launch_pass_b(NKA st, const UpdateShape& u, double* f, size_t off, s
       const size_t ntiles = (len + 511) / 512;
       const int grid = (int)(ntiles < (size_t)st->num_sms ? ntiles : (size_t)st->num_sms);
       launch_chained_smem(k, grid, threads, (size_t)smem, st->stream, f + off, st->W + off, st->Z + off, st->ld, len, st->S);
-      st->launches += 1;
+      count_launch(st);
       return;
     }
   }
   const int grid = grid_for(st, per_sm_b(st, u.nz, u.V, len), len, u.V, nka_threads_b(u.nz));
   launch_chained(nka_get_pass_b(u.nz, u.V), grid, nka_threads_b(u.nz), st->stream, f + off, st->W + off, st->Z + off,
                  st->ld, len, st->S);
-  st->launches += 1;
+  count_launch(st);
 }
 
 static void update_done(NKA st, const UpdateShape& u)
 {
+  if (st->captured) return;                       // the capacity shape needs no bookkeeping
   // list length: the pending slot (if any) became a pair, capacity mvec pairs, plus the new pending slot
   if (st->pending) st->ub_len = u.L + 1 < st->mvec + 1 ? u.L + 1 : st->mvec + 1;
   else st->ub_len = u.L + 1;
@@ -654,6 +728,9 @@ extern "C" void nka_accel_update_dev(NKA st, double* f)
   NKA_REQUIRE(st != NULL, "nka_accel_update: null handle");
   NKA_REQUIRE(f != NULL || st->vlen == 0, "nka_accel_update: null vector");
   DeviceGuard guard(st->device);
+  CaptureScope cap(st, "nka_accel_update");
+  if (st->in_capture && (st->dp || st->dp_ctx))
+    capture_fail("nka_accel_update", "the handle sums its dot products through a host callback (nka_set_dot_prod)");
   NkaRange nvtx("nka:accel_update");
   const UpdateShape u = update_shape(st, f);
   if (u.L > 0) launch_pass_a(st, u, f, 0, st->vlen, 0, 0, true);
@@ -702,6 +779,7 @@ extern "C" void nka_accel_update_host(NKA st, double* f)
   NKA_REQUIRE(st != NULL, "nka_accel_update: null handle");
   NKA_REQUIRE(f != NULL || st->vlen == 0, "nka_accel_update: null vector");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_accel_update_host", "a host f is staged through the device and the call synchronises");
   NkaRange nvtx("nka:accel_update(host f: h2d | sweeps | d2h, pipelined)");
   const size_t n = st->vlen;
   const size_t bytes = n * sizeof(double);
@@ -809,17 +887,23 @@ extern "C" void nka_accel_update(NKA st, double* f)
   cudaPointerAttributes attr;
   cudaError_t e = cudaPointerGetAttributes(&attr, f);
   if (e != cudaSuccess) { cudaGetLastError(); attr.type = cudaMemoryTypeUnregistered; }
-  if (attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged) nka_accel_update_dev(st, f);
-  else nka_accel_update_host(st, f);
+  if (attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged) { nka_accel_update_dev(st, f); return; }
+  {
+    DeviceGuard guard(st->device);
+    refuse_capture(st, "nka_accel_update with a host pointer", "a host f is staged through the device and the call synchronises");
+  }
+  nka_accel_update_host(st, f);
 }
 
 extern "C" void nka_restart(NKA st)
 {
   NKA_REQUIRE(st != NULL, "nka_restart: null handle");
   DeviceGuard guard(st->device);
+  CaptureScope cap(st, "nka_restart");
   nka_restart_kernel<<<1, NKA_STATE_THREADS, 0, st->stream>>>(st->S);
   CUDA_CHECK(cudaGetLastError());
-  st->launches += 1;
+  count_launch(st);
+  if (st->captured) return;
   st->pending = false;
   st->ub_len = 0;
 }
@@ -827,16 +911,20 @@ extern "C" void nka_restart(NKA st)
 extern "C" void nka_relax(NKA st)
 {
   NKA_REQUIRE(st != NULL, "nka_relax: null handle");
-  if (!st->pending) return;                       // src-C/...c:470: nothing pending, nothing to do
   DeviceGuard guard(st->device);
+  CaptureScope cap(st, "nka_relax");
+  // src-C/...c:470: nothing pending, nothing to do.  A captured handle does not know and queues both
+  // kernels: the relax kernel then changes nothing and leaves no conversion for nka_materialise.
+  if (!st->captured && !st->pending) return;
   nka_relax_kernel<<<1, NKA_STATE_THREADS, 0, st->stream>>>(st->S);
   CUDA_CHECK(cudaGetLastError());
-  st->launches += 1;
-  if (st->ub_len >= 2) {
+  count_launch(st);
+  if (st->captured || st->ub_len >= 2) {
     const int grid = grid_for(st, 4, st->vlen, 1);
     launch_chained(nka_materialise, grid, NKA_THREADS, st->stream, st->W, st->ld, st->vlen, st->S);
-    st->launches += 1;
+    count_launch(st);
   }
+  if (st->captured) return;
   st->pending = false;
   st->ub_len -= 1;
 }
@@ -844,9 +932,10 @@ extern "C" void nka_relax(NKA st)
 // ---------------------------------------------------------------------------
 // queries
 // ---------------------------------------------------------------------------
-static void fetch_state(NKA st, NkaDevState* h)
+static void fetch_state(NKA st, NkaDevState* h, const char* call)
 {
   DeviceGuard guard(st->device);
+  refuse_capture(st, call, "it copies the device state to the host and synchronises");
   CUDA_CHECK(cudaMemcpyAsync(h, st->S, sizeof(NkaDevState), cudaMemcpyDeviceToHost, st->stream));
   CUDA_CHECK(cudaStreamSynchronize(st->stream));
 }
@@ -855,7 +944,7 @@ extern "C" int nka_num_vec(NKA st)
 {
   NKA_REQUIRE(st != NULL, "nka_num_vec: null handle");
   static thread_local NkaDevState h;
-  fetch_state(st, &h);
+  fetch_state(st, &h, "nka_num_vec");
   int n = 0;
   for (int k = h.first; k != NKA_NIL; k = h.next[k]) ++n;
   return h.pending ? n - 1 : n;
@@ -871,17 +960,18 @@ extern "C" void nka_set_vec_tol(NKA st, double vtol)
   NKA_REQUIRE(st != NULL, "nka_set_vec_tol: null handle");
   NKA_REQUIRE(vtol > 0.0, "nka_set_vec_tol: vtol must be > 0");
   DeviceGuard guard(st->device);
-  st->vtol = vtol;
+  CaptureScope cap(st, "nka_set_vec_tol");
+  if (!st->in_capture) st->vtol = vtol;           // nka_vec_tol: the tolerance last set eagerly
   nka_set_vtol_kernel<<<1, 32, 0, st->stream>>>(st->S, vtol);
   CUDA_CHECK(cudaGetLastError());
-  st->launches += 1;
+  count_launch(st);
 }
 
 extern "C" int nka_defined(NKA st)
 {
   if (!st || !st->W || !st->Z || !st->S) return 0;
   static thread_local NkaDevState h;
-  fetch_state(st, &h);
+  fetch_state(st, &h, "nka_defined");
   if (h.mvec != st->mvec) return 0;
   return nka_state_defined(h);
 }
@@ -890,7 +980,7 @@ extern "C" void nka_get_state(NKA st, nka_state_view* out)
 {
   NKA_REQUIRE(st != NULL && out != NULL, "nka_get_state: null argument");
   static thread_local NkaDevState h;
-  fetch_state(st, &h);
+  fetch_state(st, &h, "nka_get_state");
   memset(out, 0, sizeof *out);
   const int n = h.mvec + 1;
   out->mvec = h.mvec; out->subspace = h.subspace; out->pending = h.pending;
@@ -909,6 +999,7 @@ extern "C" void nka_set_stream(NKA st, void* stream)
 {
   NKA_REQUIRE(st != NULL, "nka_set_stream: null handle");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_set_stream", "it synchronises the handle's stream; set the capture stream before the capture begins");
   fold_timing(st);
   CUDA_CHECK(cudaStreamSynchronize(st->stream));
   st->stream = (cudaStream_t)stream;
@@ -920,6 +1011,7 @@ extern "C" void nka_synchronize(NKA st)
 {
   NKA_REQUIRE(st != NULL, "nka_synchronize: null handle");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_synchronize", "it synchronises the handle's stream");
   CUDA_CHECK(cudaStreamSynchronize(st->stream));
 }
 
@@ -929,6 +1021,7 @@ extern "C" void nka_timing_enable(NKA st, int on)
 {
   NKA_REQUIRE(st != NULL, "nka_timing_enable: null handle");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_timing_enable", "switching the timing off synchronises the handle's stream");
   if (!on) fold_timing(st);
   st->timing = on != 0;
 }
@@ -937,6 +1030,7 @@ extern "C" void nka_timing_reset(NKA st)
 {
   NKA_REQUIRE(st != NULL, "nka_timing_reset: null handle");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_timing_reset", "it synchronises the handle's stream");
   fold_timing(st);
   for (int k = 0; k < T_NKIND; ++k) { st->t_ms[k] = 0.0; st->t_cnt[k] = 0; }
 }
@@ -945,6 +1039,7 @@ extern "C" void nka_timing_read(NKA st, double ms[5], unsigned long long count[5
 {
   NKA_REQUIRE(st != NULL, "nka_timing_read: null handle");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_timing_read", "it synchronises the handle's stream");
   fold_timing(st);
   for (int k = 0; k < T_NKIND; ++k) { ms[k] = st->t_ms[k]; count[k] = st->t_cnt[k]; }
 }
@@ -953,13 +1048,17 @@ extern "C" void nka_launch_geometry(NKA st, int* grid_a, int* grid_b, int* threa
 {
   NKA_REQUIRE(st != NULL, "nka_launch_geometry: null handle");
   DeviceGuard guard(st->device);
-  const int L = st->ub_len;
-  const bool may_skip = (st->comm == nullptr || st->peer != nullptr) && st->lazy && st->pending && L == st->mvec + 1;
-  const int NC = may_skip ? st->mvec : L;
-  if (grid_a) *grid_a = L > 0 ? grid_for(st, per_sm_a(st, NC, 2, st->vlen), st->vlen, 2, NKA_THREADS_A) : 0;
-  const int nz = nz_expected(st);
-  if (grid_b) *grid_b = grid_for(st, per_sm_b(st, nz, 2, st->vlen), st->vlen, 2, nka_threads_b(nz));
-  if (threads) *threads = NKA_THREADS_A * 10000 + nka_threads_b(nz);
+  const UpdateShape u = update_shape(st, nullptr);          // a 16-byte aligned f
+  if (grid_a) *grid_a = u.L > 0 ? grid_for(st, per_sm_a(st, u.NC, 2, st->vlen), st->vlen, 2, NKA_THREADS_A) : 0;
+  if (grid_b) *grid_b = grid_for(st, per_sm_b(st, u.nz, 2, st->vlen), st->vlen, 2, nka_threads_b(u.nz));
+  if (threads) *threads = NKA_THREADS_A * 10000 + nka_threads_b(u.nz);
+}
+
+extern "C" int nka_stream_capturing(NKA st)
+{
+  NKA_REQUIRE(st != NULL, "nka_stream_capturing: null handle");
+  DeviceGuard guard(st->device);
+  return capture_status(st);
 }
 
 extern "C" const char* nka_b200_version(void) { return NKA_VERSION; }
@@ -995,8 +1094,9 @@ extern "C" int nka_comm_init(NKA st, int nranks, int rank, const void* id128)
 {
   NKA_REQUIRE(st != NULL && id128 != NULL, "nka_comm_init: null argument");
   NKA_REQUIRE(nranks >= 1 && rank >= 0 && rank < nranks, "nka_comm_init: bad rank/nranks");
-  if (!nka_nccl_load()) return -1;
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_comm_init", "it is a collective that synchronises the handle's stream");
+  if (!nka_nccl_load()) return -1;
   NkaId128 id;
   memcpy(id.bytes, id128, sizeof id.bytes);
   void* comm = nullptr;
@@ -1011,8 +1111,9 @@ extern "C" int nka_comm_init(NKA st, int nranks, int rank, const void* id128)
 extern "C" void nka_comm_adopt(NKA st, void* nccl_comm, int nranks, int rank)
 {
   NKA_REQUIRE(st != NULL, "nka_comm_adopt: null handle");
-  NKA_REQUIRE(nka_nccl_load(), "nka_comm_adopt: libnccl.so.2 not found");
   DeviceGuard guard(st->device);
+  refuse_capture(st, "nka_comm_adopt", "it is a collective that synchronises the handle's stream");
+  NKA_REQUIRE(nka_nccl_load(), "nka_comm_adopt: libnccl.so.2 not found");
   NkaComm* c = new NkaComm();
   c->comm = nccl_comm; c->owned = false; c->nranks = nranks; c->rank = rank;
   attach_comm(st, c);

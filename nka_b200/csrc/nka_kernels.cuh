@@ -421,9 +421,12 @@ nka_pass_a(const double* __restrict__ f, const double* __restrict__ W, size_t ld
   NKA_STAMP_MIN(0);
   const int ncol = S->planA.ncol - S->planA.skip_last;      // columns actually streamed
   const unsigned long long submask = S->planA.submask;
+  // Columns j >= ncol are never loaded.  Their address is column 0 rather than planA.col[0]: with
+  // an empty list (the capacity shape of a captured handle runs pass A on the first call) that
+  // entry has never been written.
   const double* wcol[NC];
 #pragma unroll
-  for (int j = 0; j < NC; ++j) wcol[j] = W + (size_t)S->planA.col[j < ncol ? j : 0] * ld;
+  for (int j = 0; j < NC; ++j) wcol[j] = W + (size_t)(j < ncol ? S->planA.col[j] : 0) * ld;
 
   double acc[2 * NC];
 #pragma unroll

@@ -74,23 +74,36 @@ class NKA:
             raise NKAError("accelerator is not initialised")
         return self._h
 
+    def _uncaptured(self, call: str, why: str):
+        """The handle, or NKAError while its stream is capturing: `call` cannot be part of a CUDA
+        graph, and the library would abort on it."""
+        h = self._handle()
+        if self._lib.nka_stream_capturing(h) != 0:
+            raise NKAError("%s cannot be captured in a CUDA graph: %s" % (call, why))
+        return h
+
     # -- the hot path -----------------------------------------------------
     def accel_update(self, f) -> None:
         """accel_update(f): f is overwritten with the accelerated correction
-        (src-F08/nka_type.F90:249-419)."""
+        (src-F08/nka_type.F90:249-419).  A CUDA tensor f can be captured in a CUDA graph
+        (INTEGRATION.md, "CUDA graphs"); a host f cannot."""
         h = self._handle()
         if _is_torch(f):
             import torch
             if f.dtype != torch.float64 or not f.is_contiguous() or f.numel() != self._vlen:
                 raise ValueError("f must be a contiguous float64 tensor of length vlen")   # ASSERT(size(f) == vlen) :258
             if f.is_cuda:
+                if getattr(self, "_dp_keepalive", None) is not None:
+                    self._uncaptured("accel_update", "the handle sums its dot products through a host callback")
                 self._lib.nka_accel_update_dev(h, f.data_ptr())
             else:
+                self._uncaptured("accel_update of a host f", "it is staged through the device and synchronises")
                 self._lib.nka_accel_update_host(h, f.data_ptr())
         else:
             if not isinstance(f, np.ndarray) or f.dtype != np.float64 or not f.flags["C_CONTIGUOUS"] \
                     or f.size != self._vlen:
                 raise ValueError("f must be a contiguous float64 array of length vlen")
+            self._uncaptured("accel_update of a host f", "it is staged through the device and synchronises")
             self._lib.nka_accel_update_host(h, f.ctypes.data)
 
     def relax(self): self._lib.nka_relax(self._handle())
@@ -100,8 +113,9 @@ class NKA:
         """set_dot_prod(dot_prod): src-F08/nka_type.F90:209-219.  dp(n, x, y) is a ctypes callback of the
         C header's type (double (*)(int, double*, double*)) or None; the library calls it with n = 1 to
         make each of this process's partial dot products global (include/nonlinear_krylov_accelerator.h)."""
+        h = self._uncaptured("set_dot_prod", "it changes the launch shape of later updates")
         self._dp_keepalive = dp
-        self._lib.nka_set_dot_prod(self._handle(), C.cast(dp, C.c_void_p) if dp is not None else None)
+        self._lib.nka_set_dot_prod(h, C.cast(dp, C.c_void_p) if dp is not None else None)
 
     def set_vec_tol(self, vtol: float):
         if not vtol > 0.0:
@@ -109,19 +123,30 @@ class NKA:
         self._lib.nka_set_vec_tol(self._handle(), vtol)
 
     # -- queries ----------------------------------------------------------
-    def num_vec(self) -> int: return self._lib.nka_num_vec(self._handle())
+    def num_vec(self) -> int: return self._lib.nka_num_vec(self._uncaptured("num_vec", "it copies the device state to the host and synchronises"))
     def max_vec(self) -> int: return self._lib.nka_max_vec(self._handle())
     def vec_len(self) -> int: return self._lib.nka_vec_len64(self._handle())
     def vec_tol(self) -> float: return self._lib.nka_vec_tol(self._handle())
-    def defined(self) -> bool: return bool(self._h) and bool(self._lib.nka_defined(self._h))
+    def defined(self) -> bool:
+        return bool(self._h) and bool(self._lib.nka_defined(self._uncaptured("defined", "it copies the device state to the host and synchronises")))
 
     # -- additive: streams, distributed, introspection --------------------
-    def set_stream(self, stream: int | None): self._lib.nka_set_stream(self._handle(), stream)
-    def synchronize(self): self._lib.nka_synchronize(self._handle())
+    def set_stream(self, stream: int | None):
+        """The stream every later call is queued on.  To capture calls in a CUDA graph, set the capture
+        stream here before the capture begins."""
+        self._lib.nka_set_stream(self._uncaptured("set_stream", "it synchronises the handle's stream"), stream)
+
+    def synchronize(self): self._lib.nka_synchronize(self._uncaptured("synchronize", "it synchronises the handle's stream"))
+
+    def stream_capturing(self) -> int:
+        """1 while the handle's stream is capturing a CUDA graph, 0 when not, -1 when the handle is on
+        the legacy default stream while a blocking stream captures (include/nka_b200.h)."""
+        return self._lib.nka_stream_capturing(self._handle())
 
     def comm_init(self, nranks: int, rank: int, unique_id: bytes):
         buf = C.create_string_buffer(unique_id, 128)
-        rc = self._lib.nka_comm_init(self._handle(), nranks, rank, buf)
+        rc = self._lib.nka_comm_init(self._uncaptured("comm_init", "it is a collective that synchronises"),
+                                     nranks, rank, buf)
         if rc != 0:
             raise NKAError("nka_comm_init failed with NCCL code %d" % rc)
 
@@ -131,7 +156,7 @@ class NKA:
 
     def state(self) -> dict:
         v = _lib.StateView()
-        self._lib.nka_get_state(self._handle(), C.byref(v))
+        self._lib.nka_get_state(self._uncaptured("state", "it copies the device state to the host and synchronises"), C.byref(v))
         n = v.mvec + 1
         return {
             "subspace": v.subspace, "pending": v.pending, "first": v.first, "last": v.last,
@@ -143,13 +168,15 @@ class NKA:
         }
 
     def launch_count(self) -> int: return self._lib.nka_launch_count(self._handle())
-    def timing_enable(self, on: bool = True): self._lib.nka_timing_enable(self._handle(), int(on))
-    def timing_reset(self): self._lib.nka_timing_reset(self._handle())
+    def timing_enable(self, on: bool = True):
+        self._lib.nka_timing_enable(self._uncaptured("timing_enable", "it synchronises the handle's stream"), int(on))
+
+    def timing_reset(self): self._lib.nka_timing_reset(self._uncaptured("timing_reset", "it synchronises the handle's stream"))
 
     def timing_read(self) -> dict:
         ms = (C.c_double * 5)()
         cnt = (C.c_ulonglong * 5)()
-        self._lib.nka_timing_read(self._handle(), ms, cnt)
+        self._lib.nka_timing_read(self._uncaptured("timing_read", "it synchronises the handle's stream"), ms, cnt)
         names = ("pass_a", "state", "materialise", "pass_b", "allreduce")
         return {k: {"ms": ms[i], "count": cnt[i]} for i, k in enumerate(names)}
 

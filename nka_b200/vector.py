@@ -122,6 +122,7 @@ class VectorNKA:
         return self
 
     def accel_update(self, f: GpuVector):
+        """Can be captured in a CUDA graph on the vectors' stream (INTEGRATION.md, "CUDA graphs")."""
         if not isinstance(f, GpuVector):
             raise TypeError("incompatible arguments to NKA%ACCEL_UPDATE")
         self._lib.nka_accel_update_vec(self._h, f._h)
@@ -133,10 +134,17 @@ class VectorNKA:
 
     def relax(self): self._lib.nka_relax(self._h)
     def restart(self): self._lib.nka_restart(self._h)
-    def num_vec(self): return self._lib.nka_num_vec(self._h)
     def max_vec(self): return self._lib.nka_max_vec(self._h)
     def vec_tol(self): return self._lib.nka_vec_tol(self._h)
-    def defined(self): return bool(self._h) and bool(self._lib.nka_defined(self._h))
+
+    def _uncaptured(self, call: str):
+        if self._lib.nka_stream_capturing(self._h) != 0:
+            raise NKAError("%s cannot be captured in a CUDA graph: it copies the device state to the host "
+                           "and synchronises" % call)
+        return self._h
+
+    def num_vec(self): return self._lib.nka_num_vec(self._uncaptured("num_vec"))
+    def defined(self): return bool(self._h) and bool(self._lib.nka_defined(self._uncaptured("defined")))
 
     def delete(self):
         if self._h:
