@@ -166,6 +166,43 @@ void nka_launch_geometry (NKA, int *grid_a, int *grid_b, int *threads);
 
 const char *nka_b200_version (void);
 
+/* ---- batched accelerators: many independent same-length instances ------- */
+/* One handle holds nbatch (1..65535) independent accelerators that share vlen,
+ * mvec and vtol.  Each member has its own subspace, list, Gram factor, vtol
+ * decisions, relax and restart, and gives bit for bit what a single handle in
+ * the capacity shape (see "CUDA graphs" above) gives when fed that member's
+ * calls, whatever nbatch, the member's index and the other members hold.
+ * Device-only and single-GPU.  One update is four kernel launches whatever
+ * nbatch is (three with NKA_LAZY_LAST=0).
+ *
+ * f_dev holds nbatch rows of vlen doubles, row b at f_dev + b*ldf (ldf >= vlen).
+ * active_dev / mask_dev: NULL (every member) or nbatch device bytes, nonzero =
+ * selected, read by the kernels on the device.  An unselected member's update
+ * is exactly no call: its row of f is neither read nor written and its state is
+ * untouched.  Update, relax, restart and set_vec_tol can be captured in a CUDA
+ * graph (the handle keeps no host-side shape state); the queries, set_stream
+ * and synchronize abort while the handle's stream captures.
+ *
+ * The prototypes spell the handle as `struct nka_batch *`, which NKABATCH is. */
+typedef struct nka_batch *NKABATCH;
+struct nka_batch *nka_batch_init (int nbatch, size_t vlen, int mvec, double vtol, int device, void *stream);
+void nka_batch_delete (struct nka_batch *b);
+void nka_batch_accel_update (struct nka_batch *b, double *f_dev, size_t ldf, const unsigned char *active_dev);
+void nka_batch_relax (struct nka_batch *b, const unsigned char *mask_dev);
+void nka_batch_restart (struct nka_batch *b, const unsigned char *mask_dev);
+void nka_batch_set_vec_tol (struct nka_batch *b, double vtol);
+/* nbatch ints on the host; synchronises */
+void nka_batch_num_vec (struct nka_batch *b, int *out);
+/* 1 if every member passes the invariant check of nka_defined; synchronises */
+int nka_batch_defined (struct nka_batch *b);
+void nka_batch_get_state (struct nka_batch *b, int member, nka_state_view *out);
+void nka_batch_set_stream (struct nka_batch *b, void *stream);
+void nka_batch_synchronize (struct nka_batch *b);
+/* as nka_stream_capturing */
+int nka_batch_stream_capturing (struct nka_batch *b);
+/* kernel launches run eagerly so far; captured kernels are not counted */
+unsigned long long nka_batch_launch_count (struct nka_batch *b);
+
 #ifdef __cplusplus
 }
 #endif

@@ -81,6 +81,20 @@ SYMBOLS = {
     "nka_timing_read": (None, [C.c_void_p, _dp, C.POINTER(C.c_ulonglong)]),
     "nka_launch_geometry": (None, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "nka_b200_version": (C.c_char_p, []),
+    # include/nka_b200.h: batched accelerators
+    "nka_batch_init": (C.c_void_p, [C.c_int, C.c_size_t, C.c_int, C.c_double, C.c_int, C.c_void_p]),
+    "nka_batch_delete": (None, [C.c_void_p]),
+    "nka_batch_accel_update": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "nka_batch_relax": (None, [C.c_void_p, C.c_void_p]),
+    "nka_batch_restart": (None, [C.c_void_p, C.c_void_p]),
+    "nka_batch_set_vec_tol": (None, [C.c_void_p, C.c_double]),
+    "nka_batch_num_vec": (None, [C.c_void_p, C.POINTER(C.c_int)]),
+    "nka_batch_defined": (C.c_int, [C.c_void_p]),
+    "nka_batch_get_state": (None, [C.c_void_p, C.c_int, C.POINTER(StateView)]),
+    "nka_batch_set_stream": (None, [C.c_void_p, C.c_void_p]),
+    "nka_batch_synchronize": (None, [C.c_void_p]),
+    "nka_batch_stream_capturing": (C.c_int, [C.c_void_p]),
+    "nka_batch_launch_count": (C.c_ulonglong, [C.c_void_p]),
     # include/nka_example.h
     "nka_system_init": (C.c_void_p, [C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),
     "nka_system_init_slab": (C.c_void_p, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),

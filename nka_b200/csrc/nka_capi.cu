@@ -131,7 +131,7 @@ struct nka_state {
   int mvec = 0;
   double vtol = 0.01;
   int device = 0;
-  int num_sms = 0;
+  NkaSweepGeom geom;            // CTA counts of the sweeps on this device
   cudaStream_t stream = nullptr;
   bool own_stream = false;
   double* W = nullptr;          // (mvec+1) columns of ld doubles: raw cached inputs / differences
@@ -149,7 +149,6 @@ struct nka_state {
   double* hslot[3] = {nullptr, nullptr, nullptr};
   size_t hslot_bytes = 0;
   cudaEvent_t hslot_ev[3] = {};
-  int max_grid = 0;
   // host-side knowledge of the device list: exact `pending`, upper bound on its length
   bool pending = false;
   int ub_len = 0;
@@ -178,8 +177,6 @@ struct nka_state {
   std::vector<cudaEvent_t> free_events;
   double t_ms[T_NKIND] = {0, 0, 0, 0, 0};
   unsigned long long t_cnt[T_NKIND] = {0, 0, 0, 0, 0};
-  int occ_a[NKA_MAXSLOT + 1][3];
-  int occ_b[NKA_MAXSLOT + 1][3];
 };
 
 static cudaEvent_t get_event(NKA st)
@@ -232,16 +229,16 @@ static void count_launch(NKA st)
 // 1: the handle's stream is capturing (an invalidated capture counts: it has not ended yet);
 // 0: it is not; -1: the handle is on the legacy default stream while a blocking stream captures,
 // so nothing can be queued on it.
-static int capture_status(NKA st)
+int nka_capture_status(cudaStream_t stream)
 {
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-  const cudaError_t e = cudaStreamIsCapturing(st->stream, &cs);
+  const cudaError_t e = cudaStreamIsCapturing(stream, &cs);
   if (e == cudaErrorStreamCaptureImplicit) { cudaGetLastError(); return -1; }
   CUDA_CHECK(e);
   return cs == cudaStreamCaptureStatusNone ? 0 : 1;
 }
 
-[[noreturn]] static void capture_fail(const char* call, const char* why)
+[[noreturn]] void nka_capture_fail(const char* call, const char* why)
 {
   char b[320];
   snprintf(b, sizeof b, "%s cannot be captured in a CUDA graph: %s", call, why);
@@ -249,11 +246,15 @@ static int capture_status(NKA st)
 }
 
 // Calls that synchronise, read the device state back or stage through the host: refused while the
-// handle's stream captures, before anything reaches the stream (it would invalidate the capture).
-static void refuse_capture(NKA st, const char* call, const char* why)
+// stream captures, before anything reaches the stream (it would invalidate the capture).
+void nka_refuse_capture(cudaStream_t stream, const char* call, const char* why)
 {
-  if (capture_status(st) != 0) capture_fail(call, why);
+  if (nka_capture_status(stream) != 0) nka_capture_fail(call, why);
 }
+
+static int capture_status(NKA st) { return nka_capture_status(st->stream); }
+[[noreturn]] static void capture_fail(const char* call, const char* why) { nka_capture_fail(call, why); }
+static void refuse_capture(NKA st, const char* call, const char* why) { nka_refuse_capture(st->stream, call, why); }
 
 // Around a call that can be captured (update, relax, restart, set_vec_tol).  The first capture
 // marks the handle: from then on every call, captured or eager, uses the capacity shape.
@@ -270,15 +271,15 @@ struct CaptureScope {
   ~CaptureScope() { st->in_capture = false; }
 };
 
-static int grid_for(NKA st, int per_sm, size_t n, int V, int threads = NKA_THREADS)
+int nka_grid_for(const NkaSweepGeom& g, int per_sm, size_t n, int V, int threads)
 {
   const size_t nv = n / V;
   size_t need = (nv + threads - 1) / threads;
   if (need < 1) need = 1;
-  size_t full = (size_t)st->num_sms * (per_sm > 0 ? per_sm : 1);
-  size_t g = need < full ? need : full;
-  if (g > (size_t)st->max_grid) g = st->max_grid;
-  return (int)g;
+  size_t full = (size_t)g.num_sms * (per_sm > 0 ? per_sm : 1);
+  size_t grid = need < full ? need : full;
+  if (grid > (size_t)g.max_grid) grid = g.max_grid;
+  return (int)grid;
 }
 
 // CTAs per SM for a sweep over n elements = resident CTAs x waves.  Several waves even out the
@@ -286,46 +287,70 @@ static int grid_for(NKA st, int per_sm, size_t n, int V, int threads = NKA_THREA
 // more prologue / reduction epilogue and the last CTA one more partial row to fold: at n = 2^25
 // one wave is 2.6 % faster than eight, at 2^24 5.5 % (profiles/r1i_waves_sweep.txt).  So: one
 // wave per ~2^17 double2 per SM.
-static int waves_for(NKA st, size_t n, int V)
+static int waves_for(const NkaSweepGeom& g, size_t n, int V)
 {
-  const size_t per_wave = (size_t)st->num_sms * 113000u;
+  const size_t per_wave = (size_t)g.num_sms * 113000u;
   size_t w = (n / V) / per_wave;
   if (w < 1) w = 1;
   if (w > NKA_WAVES) w = NKA_WAVES;
   return (int)w;
 }
 
-static int resident_a(NKA st, int nc, int V)
+static int resident_a(NkaSweepGeom& g, int nc, int V)
 {
-  if (st->occ_a[nc][V] < 0) {
+  if (g.occ_a[nc][V] < 0) {
     int nb = 0;
     NKA_REQUIRE(nka_get_pass_a(nc, V) != nullptr, "pass A is not instantiated for this subspace size in this build");
     CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, nka_get_pass_a(nc, V), NKA_THREADS_A, 0));
-    st->occ_a[nc][V] = nb > 0 ? nb : 1;
+    g.occ_a[nc][V] = nb > 0 ? nb : 1;
   }
-  return st->occ_a[nc][V];
+  return g.occ_a[nc][V];
 }
 
-static int resident_b(NKA st, int nz, int V)
+static int resident_b(NkaSweepGeom& g, int nz, int V)
 {
-  if (st->occ_b[nz][V] < 0) {
+  if (g.occ_b[nz][V] < 0) {
     int nb = 0;
     NKA_REQUIRE(nka_get_pass_b(nz, V) != nullptr, "pass B is not instantiated for this subspace size in this build");
     CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, nka_get_pass_b(nz, V), nka_threads_b(nz), 0));
-    st->occ_b[nz][V] = nb > 0 ? nb : 1;
+    g.occ_b[nz][V] = nb > 0 ? nb : 1;
   }
-  return st->occ_b[nz][V];
+  return g.occ_b[nz][V];
 }
 
-static int per_sm_a(NKA st, int nc, int V, size_t len)
+int nka_per_sm_a(NkaSweepGeom& g, int nc, int V, size_t len)
 {
-  return g_grid_per_sm_a > 0 ? g_grid_per_sm_a : resident_a(st, nc, V) * waves_for(st, len, V);
+  return g_grid_per_sm_a > 0 ? g_grid_per_sm_a : resident_a(g, nc, V) * waves_for(g, len, V);
 }
 
-static int per_sm_b(NKA st, int nz, int V, size_t len)
+int nka_per_sm_b(NkaSweepGeom& g, int nz, int V, size_t len)
 {
-  return g_grid_per_sm_b > 0 ? g_grid_per_sm_b : resident_b(st, nz, V) * waves_for(st, len, V);
+  return g_grid_per_sm_b > 0 ? g_grid_per_sm_b : resident_b(g, nz, V) * waves_for(g, len, V);
 }
+
+void nka_geom_init(NkaSweepGeom& g, int device, int mvec)
+{
+  ensure_tables();
+  CUDA_CHECK(cudaDeviceGetAttribute(&g.num_sms, cudaDevAttrMultiProcessorCount, device));
+  g.max_grid = g.num_sms * 32;
+  for (int i = 0; i <= NKA_MAXSLOT; ++i)
+    for (int v = 0; v < 3; ++v) { g.occ_a[i][v] = -1; g.occ_b[i][v] = -1; }
+  // the occupancy of the capacity shape's kernels, queried now: never from inside a capture
+  // (tuning builds instantiate fewer sizes: those they lack fail later, on use, as before)
+  for (int V = 1; V <= 2; ++V) {
+    if (nka_get_pass_a(mvec, V)) resident_a(g, mvec, V);
+    if (nka_get_pass_a(mvec + 1, V)) resident_a(g, mvec + 1, V);
+    if (nka_get_pass_b(mvec, V)) resident_b(g, mvec, V);
+  }
+}
+
+static int grid_for(NKA st, int per_sm, size_t n, int V, int threads = NKA_THREADS)
+{
+  return nka_grid_for(st->geom, per_sm, n, V, threads);
+}
+
+static int per_sm_a(NKA st, int nc, int V, size_t len) { return nka_per_sm_a(st->geom, nc, V, len); }
+static int per_sm_b(NKA st, int nz, int V, size_t len) { return nka_per_sm_b(st->geom, nz, V, len); }
 
 // How many pairs are expected on the list at entry (pass B streams their Z columns): exact
 // unless a vtol drop fired earlier on the device (pass B copes with any actual count).
@@ -472,7 +497,6 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
   if (device < 0) CUDA_CHECK(cudaGetDevice(&device));
   st->device = device;
   DeviceGuard guard(device);
-  CUDA_CHECK(cudaDeviceGetAttribute(&st->num_sms, cudaDevAttrMultiProcessorCount, device));
   st->vlen = vlen;
   st->mvec = mvec;
   st->vtol = vtol;
@@ -482,8 +506,6 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
   // (and on other blocking streams), like the synchronous CPU interface it replaces
   st->stream = (cudaStream_t)stream;
   st->own_stream = false;
-  for (int i = 0; i <= NKA_MAXSLOT; ++i)
-    for (int v = 0; v < 3; ++v) { st->occ_a[i][v] = -1; st->occ_b[i][v] = -1; }
   if (const char* e = getenv("NKA_LAZY_LAST")) st->lazy = atoi(e) != 0;      // ablation switch
   if (const char* e = getenv("NKA_POISON_ALLOC")) st->poison = atoi(e) != 0;
 
@@ -497,23 +519,16 @@ extern "C" NKA nka_init_ex(size_t vlen, int mvec, double vtol, int device, void*
              poolbytes, cudaGetErrorString(e));
     nka_fail(__FILE__, __LINE__, b);
   }
-  st->max_grid = st->num_sms * 32;
-  // the occupancy of the capacity shape's kernels, queried now: never from inside a capture
-  // (tuning builds instantiate fewer sizes: those they lack fail later, on use, as before)
-  for (int V = 1; V <= 2; ++V) {
-    if (nka_get_pass_a(mvec, V)) resident_a(st, mvec, V);
-    if (nka_get_pass_a(mvec + 1, V)) resident_a(st, mvec + 1, V);
-    if (nka_get_pass_b(mvec, V)) resident_b(st, mvec, V);
-  }
+  nka_geom_init(st->geom, device, mvec);
   CUDA_CHECK(cudaMalloc(&st->S, sizeof(NkaDevState)));
   CUDA_CHECK(cudaMalloc(&st->dots, 2 * NKA_MAXSLOT * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&st->partials, (size_t)st->max_grid * 2 * NKA_MAXSLOT * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&st->partials, (size_t)st->geom.max_grid * 2 * NKA_MAXSLOT * sizeof(double)));
   CUDA_CHECK(cudaMalloc(&st->ticket, sizeof(unsigned)));
   CUDA_CHECK(cudaMemsetAsync(st->ticket, 0, sizeof(unsigned), st->stream));
   CUDA_CHECK(cudaMemsetAsync(st->dots, 0, 2 * NKA_MAXSLOT * sizeof(double), st->stream));
   poison_fill(st, st->W, poolbytes);
   poison_fill(st, st->Z, poolbytes);
-  poison_fill(st, st->partials, (size_t)st->max_grid * 2 * NKA_MAXSLOT * sizeof(double));
+  poison_fill(st, st->partials, (size_t)st->geom.max_grid * 2 * NKA_MAXSLOT * sizeof(double));
   poison_fill(st, st->dots, 2 * NKA_MAXSLOT * sizeof(double));
   nka_init_kernel<<<1, 32, 0, st->stream>>>(st->S, mvec, vtol, st->lazy ? 1 : 0);
   CUDA_CHECK(cudaGetLastError());
@@ -632,7 +647,7 @@ static int launch_pass_a(NKA st, const UpdateShape& u, double* f, size_t off, si
 {
   int grid = grid_for(st, per_sm_a(st, u.NC, u.V, len), len, u.V, NKA_THREADS_A);
   if (grid_cap > 0 && grid > grid_cap) grid = grid_cap;
-  NKA_REQUIRE(row0 + grid <= st->max_grid, "pass A: too many partial rows");
+  NKA_REQUIRE(row0 + grid <= st->geom.max_grid, "pass A: too many partial rows");
   double* rows = st->partials + (size_t)row0 * 2 * u.NC;
   NkaRange nvtx("nka:pass_a");
   SpanScope t(st, T_PASS_A);
@@ -702,7 +717,7 @@ static void launch_pass_b(NKA st, const UpdateShape& u, double* f, size_t off, s
     int threads = 0, smem = 0;
     if (PassBFn k = nka_get_pass_b_tma(u.nz, &threads, &smem)) {
       const size_t ntiles = (len + 511) / 512;
-      const int grid = (int)(ntiles < (size_t)st->num_sms ? ntiles : (size_t)st->num_sms);
+      const int grid = (int)(ntiles < (size_t)st->geom.num_sms ? ntiles : (size_t)st->geom.num_sms);
       launch_chained_smem(k, grid, threads, (size_t)smem, st->stream, f + off, st->W + off, st->Z + off, st->ld, len, st->S);
       count_launch(st);
       return;
@@ -837,7 +852,7 @@ extern "C" void nka_accel_update_host(NKA st, double* f)
   // the staging buffer is free once everything queued on the handle's stream has run
   CUDA_CHECK(cudaEventRecord(st->order_ev, st->stream));
   CUDA_CHECK(cudaStreamWaitEvent(st->copy_in, st->order_ev, 0));
-  const int grid_cap = st->max_grid / nc;
+  const int grid_cap = st->geom.max_grid / nc;
   int row0 = 0;
   for (int c = 0; c < nc; ++c) {
     const size_t len = off[c + 1] - off[c];
@@ -981,6 +996,11 @@ extern "C" void nka_get_state(NKA st, nka_state_view* out)
   NKA_REQUIRE(st != NULL && out != NULL, "nka_get_state: null argument");
   static thread_local NkaDevState h;
   fetch_state(st, &h, "nka_get_state");
+  nka_state_view_from(h, out);
+}
+
+void nka_state_view_from(const NkaDevState& h, nka_state_view* out)
+{
   memset(out, 0, sizeof *out);
   const int n = h.mvec + 1;
   out->mvec = h.mvec; out->subspace = h.subspace; out->pending = h.pending;

@@ -22,6 +22,18 @@ struct NkaRange {
     char b_[256]; snprintf(b_, sizeof b_, "%s failed: %s", #call, cudaGetErrorString(e_));      \
     nka_fail(__FILE__, __LINE__, b_); } } while (0)
 
+// CUDA graphs (nka_capi.cu).  nka_capture_status: 1 while `stream` captures (an invalidated capture
+// counts: it has not ended yet), 0 when not, -1 when `stream` is the legacy default stream while a
+// blocking stream captures.  nka_refuse_capture aborts with a message naming `call` unless it is 0.
+int nka_capture_status(cudaStream_t stream);
+[[noreturn]] void nka_capture_fail(const char* call, const char* why);
+void nka_refuse_capture(cudaStream_t stream, const char* call, const char* why);
+
+// The device state as include/nka_b200.h shows it (nka_get_state, nka_batch_get_state).
+struct NkaDevState;
+struct nka_state_view;
+void nka_state_view_from(const NkaDevState& h, nka_state_view* out);
+
 struct DeviceGuard {
   int prev = -1;
   explicit DeviceGuard(int dev) {
