@@ -203,6 +203,46 @@ int nka_batch_stream_capturing (struct nka_batch *b);
 /* kernel launches run eagerly so far; captured kernels are not counted */
 unsigned long long nka_batch_launch_count (struct nka_batch *b);
 
+/* ---- device-side fixed-point loops over a batched accelerator ----------- */
+/* One graph launch runs a whole solve of x_b = G(x_b) for every member b: a
+ * WHILE graph node repeats { residual graph; record r = ||F_b||_2 of each
+ * running member and stop it when r is not finite (NONFINITE), when
+ * r < max(atol, rtol * r0_b) (CONVERGED, r0_b = its norm at the launch's first
+ * check) or after maxit steps (MAXIT); nka_batch_accel_update(F, ldf, running);
+ * X_b += F_b for the running members } until no member runs.
+ *
+ * residual_graph is a cudaGraph_t that reads X and writes F = G(X) - X for
+ * every row.  It is cloned: the caller may destroy it, but keeps alive the
+ * memory it addresses.  It may hold only node types a conditional body can
+ * (kernels, memsets, memcopies, child graphs): a graph CUDA refuses, or a
+ * driver older than 12.4, makes create print CUDA's reason and return NULL.
+ * x_dev, f_dev: nbatch rows of vlen doubles at row strides ldx, ldf >= vlen.
+ *
+ * Each member's X, F, step count, status, history and state are bit for bit
+ * those of a host-driven loop making the same residual, accel_update (same
+ * masks) and X_b += F_b calls.  The accelerator is not restarted by a launch.
+ * launch is queued on the batch's stream and aborts while that stream
+ * captures; results and history synchronise (refused while it captures).
+ * A launch is not counted by nka_batch_launch_count.
+ *
+ * The prototypes spell the handle as `struct nka_batch_loop *`, which
+ * NKABATCHLOOP is. */
+typedef struct nka_batch_loop *NKABATCHLOOP;
+#define NKA_LOOP_RUNNING   0     /* never launched, or the launch has not finished */
+#define NKA_LOOP_CONVERGED 1
+#define NKA_LOOP_MAXIT     2
+#define NKA_LOOP_NONFINITE 3
+struct nka_batch_loop *nka_batch_loop_create (struct nka_batch *b, void *residual_graph /* cudaGraph_t */,
+                                              double *x_dev, size_t ldx, double *f_dev, size_t ldf,
+                                              double atol, double rtol, int maxit);
+/* async on the batch's stream */
+void nka_batch_loop_launch (struct nka_batch_loop *L);
+/* nbatch each: steps taken, NKA_LOOP_* status, latest norm; synchronises */
+void nka_batch_loop_results (struct nka_batch_loop *L, int *iters, int *status, double *norm);
+/* (maxit+1) x nbatch, row k = check k, NaN where a member made no check k; synchronises */
+void nka_batch_loop_history (struct nka_batch_loop *L, double *norms);
+void nka_batch_loop_destroy (struct nka_batch_loop *L);
+
 #ifdef __cplusplus
 }
 #endif

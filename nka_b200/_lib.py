@@ -95,6 +95,13 @@ SYMBOLS = {
     "nka_batch_synchronize": (None, [C.c_void_p]),
     "nka_batch_stream_capturing": (C.c_int, [C.c_void_p]),
     "nka_batch_launch_count": (C.c_ulonglong, [C.c_void_p]),
+    # include/nka_b200.h: device-side fixed-point loops
+    "nka_batch_loop_create": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                           C.c_double, C.c_double, C.c_int]),
+    "nka_batch_loop_launch": (None, [C.c_void_p]),
+    "nka_batch_loop_results": (None, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), _dp]),
+    "nka_batch_loop_history": (None, [C.c_void_p, _dp]),
+    "nka_batch_loop_destroy": (None, [C.c_void_p]),
     # include/nka_example.h
     "nka_system_init": (C.c_void_p, [C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),
     "nka_system_init_slab": (C.c_void_p, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),

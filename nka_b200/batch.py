@@ -8,6 +8,7 @@ Device-only and single-GPU: rows of f are CUDA float64 tensor rows (INTEGRATION.
 from __future__ import annotations
 
 import ctypes as C
+import weakref
 
 import numpy as np
 
@@ -23,6 +24,7 @@ class BatchNKA:
     def __init__(self, nbatch: int | None = None, vlen: int | None = None, mvec: int | None = None,
                  vtol: float = 0.01, device: int = -1, stream: int | None = None):
         self._h = None
+        self._loops = weakref.WeakSet()
         self._lib = _lib.load()
         if nbatch is not None:
             self.init(nbatch, vlen, mvec, vtol=vtol, device=device, stream=stream)
@@ -49,6 +51,8 @@ class BatchNKA:
         return self
 
     def delete(self):
+        for loop in list(self._loops):
+            loop.destroy()
         if self._h:
             self._lib.nka_batch_delete(self._h)
             self._h = None
@@ -82,26 +86,31 @@ class BatchNKA:
             raise ValueError("%s must be a contiguous CUDA bool or uint8 tensor of length nbatch" % what)
         return mask.data_ptr()
 
+    def _rows(self, T, name: str) -> int:
+        """The row stride of T, a CUDA float64 tensor [nbatch, vlen] with unit column stride."""
+        if not _is_torch(T):
+            raise ValueError("%s must be a CUDA float64 tensor of shape [nbatch, vlen]" % name)
+        import torch
+        if T.dtype != torch.float64 or T.dim() != 2 or tuple(T.shape) != (self.nbatch, self.vlen):
+            raise ValueError("%s must be a CUDA float64 tensor of shape [nbatch, vlen] = [%d, %d]"
+                             % (name, self.nbatch, self.vlen))
+        if T.stride(1) != 1 and self.vlen > 1:
+            raise ValueError("%s must have unit column stride (%s.stride(1) == 1)" % (name, name))
+        ld = T.stride(0)
+        if ld < self.vlen:
+            if self.nbatch > 1:
+                raise ValueError("%s's row stride must be >= vlen" % name)
+            ld = self.vlen                      # one row: its stride is never used to address anything
+        if not T.is_cuda:
+            raise ValueError("%s must be a CUDA tensor: the batched accelerator is device-only" % name)
+        return ld
+
     # -- the hot path -----------------------------------------------------
     def accel_update(self, F, active=None) -> None:
         """F: CUDA float64 tensor [nbatch, vlen] with unit column stride; row b is member b's f and is
         overwritten with its accelerated correction.  active: optional length-nbatch CUDA bool / uint8
         tensor; an inactive member's row and state are left exactly as they are.  Capturable."""
-        if not _is_torch(F):
-            raise ValueError("F must be a CUDA float64 tensor of shape [nbatch, vlen]")
-        import torch
-        if F.dtype != torch.float64 or F.dim() != 2 or tuple(F.shape) != (self.nbatch, self.vlen):
-            raise ValueError("F must be a CUDA float64 tensor of shape [nbatch, vlen] = [%d, %d]"
-                             % (self.nbatch, self.vlen))
-        if F.stride(1) != 1 and self.vlen > 1:
-            raise ValueError("F must have unit column stride (F.stride(1) == 1)")
-        ldf = F.stride(0)
-        if ldf < self.vlen:
-            if self.nbatch > 1:
-                raise ValueError("F's row stride must be >= vlen")
-            ldf = self.vlen                     # one row: its stride is never used to address anything
-        if not F.is_cuda:
-            raise ValueError("F must be a CUDA tensor: the batched accelerator is device-only")
+        ldf = self._rows(F, "F")
         a = self._mask(active, "active")
         self._lib.nka_batch_accel_update(self._handle(), F.data_ptr(), ldf, a)
 
@@ -158,3 +167,96 @@ class BatchNKA:
 
     def launch_count(self) -> int:
         return self._lib.nka_batch_launch_count(self._handle())
+
+    # -- device-side fixed-point loops --------------------------------------
+    def fixed_point_loop(self, residual, X, F, atol: float = 0.0, rtol: float = 1e-8,
+                         maxit: int = 100) -> "FixedPointLoop":
+        """A solve of x_b = G(x_b) for every member that runs to its end in one graph launch
+        (INTEGRATION.md section 8).  residual: a zero-argument callable writing F = G(X) - X in place with
+        torch ops; it is run once to warm up, then captured.  X, F: CUDA float64 tensors [nbatch, vlen]
+        with unit column stride.  A member stops when ||F_b|| is not finite, when ||F_b|| <
+        max(atol, rtol * (its norm at the launch's first check)), or after maxit steps."""
+        if isinstance(atol, bool) or not isinstance(atol, (int, float)) or not atol >= 0.0:
+            raise ValueError("atol must be a number >= 0")
+        if isinstance(rtol, bool) or not isinstance(rtol, (int, float)) or not rtol >= 0.0:
+            raise ValueError("rtol must be a number >= 0")
+        if isinstance(maxit, bool) or not isinstance(maxit, (int, np.integer)) or maxit < 0 or maxit > 2**31 - 2:
+            raise ValueError("maxit must be an integer >= 0")
+        ldx = self._rows(X, "X")
+        ldf = self._rows(F, "F")
+        h = self._uncaptured("fixed_point_loop", "it captures the residual and synchronises")
+        import torch
+        side = torch.cuda.Stream(device=F.device)
+        side.wait_stream(torch.cuda.current_stream(F.device))
+        with torch.cuda.stream(side):
+            residual()
+        torch.cuda.current_stream(F.device).wait_stream(side)
+        graph = torch.cuda.CUDAGraph(keep_graph=True)
+        with torch.cuda.graph(graph):
+            residual()
+        torch.cuda.synchronize(F.device)
+        loop = FixedPointLoop(self, graph, X, F, int(maxit))
+        loop._h = self._lib.nka_batch_loop_create(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
+                                                  float(atol), float(rtol), int(maxit))
+        if not loop._h:
+            raise NKAError("nka_batch_loop_create returned NULL: CUDA refused the residual graph or the driver "
+                           "has no conditional graph nodes (the reason is printed on stderr)")
+        self._loops.add(loop)
+        return loop
+
+
+class FixedPointLoop:
+    """A device-side fixed-point loop over a BatchNKA (BatchNKA.fixed_point_loop).  Keeps the captured
+    residual graph (and its memory pool), X, F and the batch alive."""
+
+    def __init__(self, batch: BatchNKA, graph, X, F, maxit: int):
+        self._h = None
+        self._batch, self._graph, self._X, self._F = batch, graph, X, F
+        self._lib = batch._lib
+        self.maxit = maxit
+
+    def _handle(self, call: str, why: str | None = None):
+        if not self._h:
+            raise NKAError("fixed-point loop is destroyed")
+        if why is not None:
+            self._batch._uncaptured(call, why)
+        return self._h
+
+    def run(self) -> None:
+        """One graph launch on the batch's stream: the whole solve.  Returns at once."""
+        self._lib.nka_batch_loop_launch(self._handle(
+            "run", "a graph with conditional nodes cannot become a child of another graph"))
+
+    def results(self):
+        """(steps, status, norm) per member as numpy arrays; status is one of RUNNING, CONVERGED, MAXIT,
+        NONFINITE.  Synchronises."""
+        h = self._handle("results", "it copies the loop's results to the host and synchronises")
+        nb = self._batch.nbatch
+        it = np.zeros(nb, dtype=np.int32)
+        st = np.zeros(nb, dtype=np.int32)
+        norm = np.zeros(nb, dtype=np.float64)
+        self._lib.nka_batch_loop_results(h, it.ctypes.data_as(C.POINTER(C.c_int)), st.ctypes.data_as(C.POINTER(C.c_int)),
+                                         norm.ctypes.data_as(C.POINTER(C.c_double)))
+        return it, st, norm
+
+    def history(self) -> np.ndarray:
+        """[(maxit+1), nbatch]: row k holds each member's norm at check k, NaN where it made none.  Synchronises."""
+        h = self._handle("history", "it copies the loop's history to the host and synchronises")
+        out = np.zeros((self.maxit + 1, self._batch.nbatch), dtype=np.float64)
+        self._lib.nka_batch_loop_history(h, out.ctypes.data_as(C.POINTER(C.c_double)))
+        return out
+
+    def destroy(self) -> None:
+        if self._h:
+            self._lib.nka_batch_loop_destroy(self._h)
+            self._h = None
+        self._batch._loops.discard(self)
+
+    def __del__(self):
+        try:
+            self.destroy()
+        except Exception:
+            pass
+
+
+RUNNING, CONVERGED, MAXIT, NONFINITE = 0, 1, 2, 3

@@ -188,27 +188,6 @@ __global__ void nka_batch_query_kernel(const NkaDevState* Sall, int nbatch, int 
 // ---------------------------------------------------------------------------
 // the handle
 // ---------------------------------------------------------------------------
-struct nka_batch {
-  int nbatch = 0, mvec = 0;
-  size_t vlen = 0, ld = 0, wstride = 0;   // wstride = (mvec+1)*ld: one member's W (or Z) block
-  double vtol = 0.01;
-  int device = 0;
-  cudaStream_t stream = nullptr;
-  NkaSweepGeom geom;
-  bool lazy = true;                       // NKA_LAZY_LAST, as nka_init_ex reads it
-  bool poison = false;                    // NKA_POISON_ALLOC
-  int nc = 0;                             // pass A's columns: mvec (lazy) or mvec + 1
-  double* W = nullptr;
-  double* Z = nullptr;
-  NkaDevState* S = nullptr;
-  double* dots = nullptr;                 // nbatch x 2*NKA_MAXSLOT
-  double* partials = nullptr;             // nbatch x prow
-  size_t prow = 0;                        // doubles of partial rows per member
-  unsigned* tickets = nullptr;            // nbatch
-  int* query = nullptr;                   // device, 2*nbatch ints (nka_batch_query_kernel)
-  unsigned long long launches = 0;
-};
-
 static void batch_poison(NKABATCH bt, void* p, size_t bytes)
 {
   if (bt->poison) CUDA_CHECK(cudaMemsetAsync(p, 0xFF, bytes, bt->stream));
@@ -318,7 +297,31 @@ extern "C" void nka_batch_delete(NKABATCH bt)
   delete bt;
 }
 
-// One batched update: pass A, state step, [fix-up], pass B, each one launch over every member.
+// One batched update: pass A, state step, [fix-up], pass B, each one launch over every member, queued
+// on `stream`; a captured update (cap) counts no launches.
+static void batch_update(NKABATCH bt, double* f, size_t ldf, const unsigned char* active, cudaStream_t stream, bool cap)
+{
+  // the 16-byte path needs every row 16-byte aligned: f itself and an even row stride
+  const int V = ((uintptr_t)f % 16 == 0 && ldf % 2 == 0) ? 2 : 1;
+  const unsigned nb = (unsigned)bt->nbatch;
+  const size_t n = bt->vlen;
+  nka_get_batch_pass_a(bt->nc, V)<<<dim3((unsigned)batch_grid_a(bt, V), nb), NKA_THREADS_A, 0, stream>>>(
+      f, ldf, bt->W, bt->wstride, bt->ld, n, bt->S, bt->partials, bt->prow, bt->tickets, bt->dots, active);
+  batch_launched(bt, cap, 1);
+  const unsigned nstate = (nb + NKA_BATCH_STATE_MEMBERS - 1) / NKA_BATCH_STATE_MEMBERS;
+  nka_batch_state_kernel<<<nstate, 32 * NKA_BATCH_STATE_MEMBERS, 0, stream>>>(bt->S, bt->dots, bt->nbatch, active);
+  batch_launched(bt, cap, 1);
+  if (bt->lazy) {
+    // exits at once for every member whose step did not ask for the skipped column
+    nka_batch_fixup_kernel<<<dim3((unsigned)batch_grid_fixup(bt), nb), NKA_THREADS, 0, stream>>>(
+        f, ldf, bt->W, bt->wstride, bt->ld, n, bt->S, bt->partials, bt->prow, bt->tickets, bt->dots, active);
+    batch_launched(bt, cap, 1);
+  }
+  nka_get_batch_pass_b(bt->mvec, V)<<<dim3((unsigned)batch_grid_b(bt, V), nb), nka_threads_b(bt->mvec), 0, stream>>>(
+      f, ldf, bt->W, bt->Z, bt->wstride, bt->ld, n, bt->S, active);
+  batch_launched(bt, cap, 1);
+}
+
 extern "C" void nka_batch_accel_update(NKABATCH bt, double* f, size_t ldf, const unsigned char* active)
 {
   NKA_REQUIRE(bt != NULL, "nka_batch_accel_update: null handle");
@@ -327,25 +330,12 @@ extern "C" void nka_batch_accel_update(NKABATCH bt, double* f, size_t ldf, const
   DeviceGuard guard(bt->device);
   const bool cap = batch_capturing(bt, "nka_batch_accel_update");
   NkaRange nvtx("nka:batch_accel_update");
-  // the 16-byte path needs every row 16-byte aligned: f itself and an even row stride
-  const int V = ((uintptr_t)f % 16 == 0 && ldf % 2 == 0) ? 2 : 1;
-  const unsigned nb = (unsigned)bt->nbatch;
-  const size_t n = bt->vlen;
-  nka_get_batch_pass_a(bt->nc, V)<<<dim3((unsigned)batch_grid_a(bt, V), nb), NKA_THREADS_A, 0, bt->stream>>>(
-      f, ldf, bt->W, bt->wstride, bt->ld, n, bt->S, bt->partials, bt->prow, bt->tickets, bt->dots, active);
-  batch_launched(bt, cap, 1);
-  const unsigned nstate = (nb + NKA_BATCH_STATE_MEMBERS - 1) / NKA_BATCH_STATE_MEMBERS;
-  nka_batch_state_kernel<<<nstate, 32 * NKA_BATCH_STATE_MEMBERS, 0, bt->stream>>>(bt->S, bt->dots, bt->nbatch, active);
-  batch_launched(bt, cap, 1);
-  if (bt->lazy) {
-    // exits at once for every member whose step did not ask for the skipped column
-    nka_batch_fixup_kernel<<<dim3((unsigned)batch_grid_fixup(bt), nb), NKA_THREADS, 0, bt->stream>>>(
-        f, ldf, bt->W, bt->wstride, bt->ld, n, bt->S, bt->partials, bt->prow, bt->tickets, bt->dots, active);
-    batch_launched(bt, cap, 1);
-  }
-  nka_get_batch_pass_b(bt->mvec, V)<<<dim3((unsigned)batch_grid_b(bt, V), nb), nka_threads_b(bt->mvec), 0, bt->stream>>>(
-      f, ldf, bt->W, bt->Z, bt->wstride, bt->ld, n, bt->S, active);
-  batch_launched(bt, cap, 1);
+  batch_update(bt, f, ldf, active, bt->stream, cap);
+}
+
+void nka_batch_update_captured(NKABATCH bt, double* f, size_t ldf, const unsigned char* active, cudaStream_t stream)
+{
+  batch_update(bt, f, ldf, active, stream, true);
 }
 
 extern "C" void nka_batch_relax(NKABATCH bt, const unsigned char* mask)

@@ -1,7 +1,33 @@
-// nka_batch.h -- kernel tables of the batched accelerator (nka_batch.cu, nka_batch_pass_a.cu,
-// nka_batch_pass_b.cu).
+// nka_batch.h -- the batched accelerator's handle and kernel tables (nka_batch.cu, nka_batch_pass_a.cu,
+// nka_batch_pass_b.cu), shared with its device-side fixed-point loops (nka_batch_loop.cu).
 #pragma once
+#include <cuda_runtime.h>
 #include "nka_dispatch.h"
+
+struct nka_batch {
+  int nbatch = 0, mvec = 0;
+  size_t vlen = 0, ld = 0, wstride = 0;   // wstride = (mvec+1)*ld: one member's W (or Z) block
+  double vtol = 0.01;
+  int device = 0;
+  cudaStream_t stream = nullptr;
+  NkaSweepGeom geom;
+  bool lazy = true;                       // NKA_LAZY_LAST, as nka_init_ex reads it
+  bool poison = false;                    // NKA_POISON_ALLOC
+  int nc = 0;                             // pass A's columns: mvec (lazy) or mvec + 1
+  double* W = nullptr;
+  double* Z = nullptr;
+  NkaDevState* S = nullptr;
+  double* dots = nullptr;                 // nbatch x 2*NKA_MAXSLOT
+  double* partials = nullptr;             // nbatch x prow
+  size_t prow = 0;                        // doubles of partial rows per member
+  unsigned* tickets = nullptr;            // nbatch
+  int* query = nullptr;                   // device, 2*nbatch ints (nka_batch_query_kernel)
+  unsigned long long launches = 0;
+};
+
+// One batched update queued on `stream` while that stream captures (a loop's body graph): the update
+// nka_batch_accel_update queues, counted as no launch, whatever stream the handle itself uses.
+void nka_batch_update_captured(nka_batch* bt, double* f, size_t ldf, const unsigned char* active, cudaStream_t stream);
 
 // (F, ldf, W, wstride, ld, n, S, partials, prow, tickets, dots, active)
 typedef void (*NkaBatchPassAFn)(const double*, size_t, const double*, size_t, size_t, size_t, const NkaDevState*, double*,

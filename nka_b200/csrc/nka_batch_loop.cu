@@ -1,0 +1,303 @@
+// nka_batch_loop.cu -- device-side fixed-point loops over a batched accelerator (include/nka_b200.h,
+// INTEGRATION.md section 8, DESIGN.md section 13).  One graph launch runs a whole solve:
+//
+//   reset -> WHILE (any member running) { residual graph -> check -> decide -> batched update -> step }
+//
+// check reduces each running member's ||F_b||_2 with the batch's fixed-order grid reduction, records it
+// and decides the member's status; decide sets the WHILE node's condition; the update and step touch
+// only members still running.  A member's bits are those of a host-driven loop making the same calls:
+//   - check's CTA count per member follows vlen only (nka_grid_for, as the batch's fix-up), and
+//     nka_grid_reduce folds its partial rows in a fixed order, so a norm depends on the row alone;
+//   - the update is nka_batch_accel_update's own launch sequence, with check's mask;
+//   - step is X_b + F_b element by element, as X[b] += F[b] computes it.
+#include <cuda_runtime.h>
+#include <math.h>
+#include <stdint.h>
+#include <stdio.h>
+
+#include "../../include/nka_b200.h"
+#include "nka_internal.h"
+#include "nka_batch.h"
+#include "nka_kernels.cuh"
+
+// ---------------------------------------------------------------------------
+// kernels
+// ---------------------------------------------------------------------------
+// Every member running at step 0, the history NaN.  (r0 needs no reset: check 0 writes it.)
+__global__ void __launch_bounds__(NKA_THREADS)
+nka_loop_reset(int* __restrict__ iters, int* __restrict__ status, unsigned char* __restrict__ active,
+               double* __restrict__ rlast, double* __restrict__ hist, size_t nhist, int nbatch)
+{
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nhist; i += stride) {
+    hist[i] = nan;
+    if (i < (size_t)nbatch) {
+      iters[i] = 0;
+      status[i] = NKA_LOOP_RUNNING;
+      active[i] = 1;
+      rlast[i] = nan;
+    }
+  }
+}
+
+// ||F_b|| of every running member (blockIdx.y), recorded as check k = iters[b], and its status.
+template <int V>
+__global__ void __launch_bounds__(NKA_THREADS)
+nka_loop_check(const double* __restrict__ F, size_t ldf, size_t n, int nbatch, const int* __restrict__ iters,
+               int* __restrict__ status, unsigned char* __restrict__ active, double* __restrict__ r0,
+               double* __restrict__ rlast, double* __restrict__ hist, double* __restrict__ partials_all, size_t prow,
+               unsigned* __restrict__ tickets, double atol, double rtol, int maxit)
+{
+  const size_t b = blockIdx.y;
+  // every CTA of a member sees the same status: only the member's last CTA writes it, after all took tickets
+  if (status[b] != NKA_LOOP_RUNNING) return;
+  const double* f = F + b * ldf;
+  double acc[1] = {0.0};
+  const size_t nv = n / V;
+  const size_t stride = (size_t)gridDim.x * NKA_THREADS;
+  const size_t start = (size_t)blockIdx.x * NKA_THREADS + threadIdx.x;
+  for (size_t i = start; i < nv; i += stride) {
+    const Vec<V> x = Vec<V>::ld(f, i);
+    x.dot_into(x, acc[0]);
+  }
+  if (V == 2 && (n & 1) && start == 0) acc[0] = fma(f[n - 1], f[n - 1], acc[0]);
+  __shared__ double ss;
+  double* partials = partials_all + b * prow;
+  const bool last = nka_grid_reduce<1, NKA_THREADS>(acc, partials, tickets + b, partials, gridDim.x,
+                                                    [&](int, double v) { ss = v; });
+  if (last && threadIdx.x == 0) {
+    const double r = sqrt(ss);
+    const int k = iters[b];
+    hist[(size_t)k * nbatch + b] = r;
+    rlast[b] = r;
+    if (k == 0) r0[b] = r;
+    int st = NKA_LOOP_RUNNING;
+    if (!isfinite(r)) st = NKA_LOOP_NONFINITE;
+    else if (r < fmax(atol, rtol * r0[b])) st = NKA_LOOP_CONVERGED;
+    else if (k >= maxit) st = NKA_LOOP_MAXIT;
+    status[b] = st;
+    active[b] = st == NKA_LOOP_RUNNING;
+  }
+}
+
+// The WHILE node's condition: whether any member is still running.
+__global__ void __launch_bounds__(1024)
+nka_loop_decide(const unsigned char* __restrict__ active, int nbatch, cudaGraphConditionalHandle cond)
+{
+  int any = 0;
+  for (int b = threadIdx.x; b < nbatch; b += blockDim.x) any |= active[b];
+  any = __syncthreads_or(any);
+  if (threadIdx.x == 0) cudaGraphSetConditional(cond, any ? 1u : 0u);
+}
+
+// X_b += F_b and one more step for every running member (blockIdx.y).
+template <int V>
+__global__ void __launch_bounds__(NKA_THREADS)
+nka_loop_step(double* __restrict__ X, size_t ldx, const double* __restrict__ F, size_t ldf, size_t n,
+              const unsigned char* __restrict__ active, int* __restrict__ iters)
+{
+  const size_t b = blockIdx.y;
+  if (!active[b]) return;
+  double* x = X + b * ldx;
+  const double* f = F + b * ldf;
+  const size_t nv = n / V;
+  const size_t stride = (size_t)gridDim.x * NKA_THREADS;
+  const size_t start = (size_t)blockIdx.x * NKA_THREADS + threadIdx.x;
+  for (size_t i = start; i < nv; i += stride) (Vec<V>::ld_plain(x, i) + Vec<V>::ld(f, i)).st(x, i);
+  if (V == 2 && (n & 1) && start == 0) x[n - 1] = x[n - 1] + f[n - 1];
+  if (start == 0) iters[b] += 1;
+}
+
+// ---------------------------------------------------------------------------
+// the handle
+// ---------------------------------------------------------------------------
+struct nka_batch_loop {
+  NKABATCH bt = nullptr;
+  int maxit = 0;
+  cudaGraphExec_t exec = nullptr;
+  int* iters = nullptr;                   // device, nbatch
+  int* status = nullptr;                  // device, nbatch
+  unsigned char* active = nullptr;        // device, nbatch: status == RUNNING, the update's mask
+  double* r0 = nullptr;                   // device, nbatch: each member's norm at check 0
+  double* rlast = nullptr;                // device, nbatch: each member's latest norm
+  double* hist = nullptr;                 // device, (maxit+1) x nbatch
+  double* partials = nullptr;             // device, nbatch x prow
+  unsigned* tickets = nullptr;            // device, nbatch
+};
+
+static void loop_free(NKABATCHLOOP L)
+{
+  if (L->exec) cudaGraphExecDestroy(L->exec);
+  cudaFree(L->iters); cudaFree(L->status); cudaFree(L->active); cudaFree(L->r0); cudaFree(L->rlast);
+  cudaFree(L->hist); cudaFree(L->partials); cudaFree(L->tickets);
+  delete L;
+}
+
+// CUDA refused the graph: the caller's residual graph or the driver.  Not a library fault: print CUDA's
+// reason, clear the (non-sticky) error and let the caller decide.
+static NKABATCHLOOP loop_refused(NKABATCHLOOP L, cudaGraph_t g, cudaStream_t s, const char* what, cudaError_t e)
+{
+  fprintf(stderr, "nka_b200: nka_batch_loop_create: %s: %s\n", what, cudaGetErrorString(e));
+  fflush(stderr);
+  cudaGetLastError();
+  if (g) cudaGraphDestroy(g);
+  cudaStreamDestroy(s);
+  loop_free(L);
+  return nullptr;
+}
+
+// CTAs per member of check and step: the batch's rule for a one-accumulator sweep of vlen (its fix-up's)
+static int loop_grid(NKABATCH bt, int V) { return nka_grid_for(bt->geom, 4, bt->vlen, V, NKA_THREADS); }
+
+extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
+                                             size_t ldf, double atol, double rtol, int maxit)
+{
+  NKA_REQUIRE(bt != NULL, "nka_batch_loop_create: null handle");
+  NKA_REQUIRE(residual_graph != NULL, "nka_batch_loop_create: null residual graph");
+  NKA_REQUIRE(x != NULL && f != NULL, "nka_batch_loop_create: null x or f");
+  NKA_REQUIRE(ldx >= bt->vlen && ldf >= bt->vlen, "nka_batch_loop_create: ldx and ldf must be >= vlen");
+  NKA_REQUIRE(atol >= 0.0 && rtol >= 0.0, "nka_batch_loop_create: atol and rtol must be >= 0");
+  NKA_REQUIRE(maxit >= 0, "nka_batch_loop_create: maxit must be >= 0");
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, "nka_batch_loop_create", "it builds and uploads a graph and synchronises");
+  int driver = 0;
+  CUDA_CHECK(cudaDriverGetVersion(&driver));
+  if (driver < 12040) {
+    fprintf(stderr, "nka_b200: nka_batch_loop_create: conditional graph nodes need a CUDA 12.4 driver, this one is "
+                    "%d.%d: %s\n", driver / 1000, (driver % 1000) / 10, cudaGetErrorString(cudaErrorInsufficientDriver));
+    fflush(stderr);
+    return nullptr;
+  }
+
+  NKABATCHLOOP L = new nka_batch_loop();
+  L->bt = bt;
+  L->maxit = maxit;
+  const size_t nb = (size_t)bt->nbatch;
+  const size_t nhist = (size_t)(maxit + 1) * nb;
+  // the 16-byte paths need every row 16-byte aligned: the base address and an even row stride
+  const int Vc = ((uintptr_t)f % 16 == 0 && ldf % 2 == 0) ? 2 : 1;
+  const int Vs = Vc == 2 && (uintptr_t)x % 16 == 0 && ldx % 2 == 0 ? 2 : 1;
+  const unsigned gc = (unsigned)loop_grid(bt, Vc), gs = (unsigned)loop_grid(bt, Vs);
+  const size_t prow = gc;
+  CUDA_CHECK(cudaMalloc(&L->iters, nb * sizeof(int)));
+  CUDA_CHECK(cudaMalloc(&L->status, nb * sizeof(int)));
+  CUDA_CHECK(cudaMalloc(&L->active, nb));
+  CUDA_CHECK(cudaMalloc(&L->r0, nb * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&L->rlast, nb * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&L->hist, nhist * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&L->partials, nb * prow * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&L->tickets, nb * sizeof(unsigned)));
+
+  cudaStream_t s = nullptr;               // private: the batch's own stream may be the legacy default
+  CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+  CUDA_CHECK(cudaMemsetAsync(L->tickets, 0, nb * sizeof(unsigned), s));
+  if (bt->poison) {
+    CUDA_CHECK(cudaMemsetAsync(L->partials, 0xFF, nb * prow * sizeof(double), s));
+    CUDA_CHECK(cudaMemsetAsync(L->r0, 0xFF, nb * sizeof(double), s));
+  }
+  const unsigned greset = (unsigned)((nhist + NKA_THREADS - 1) / NKA_THREADS < 1024 ? (nhist + NKA_THREADS - 1) / NKA_THREADS : 1024);
+  // before any launch: every member RUNNING at 0 steps, as the results of a loop never launched read
+  nka_loop_reset<<<greset, NKA_THREADS, 0, s>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
+  CUDA_CHECK(cudaGetLastError());
+
+  // reset, then the WHILE node
+  cudaGraph_t g = nullptr;
+  CUDA_CHECK(cudaGraphCreate(&g, 0));
+  cudaGraphConditionalHandle cond;
+  cudaError_t e = cudaGraphConditionalHandleCreate(&cond, g, 1, cudaGraphCondAssignDefault);
+  if (e != cudaSuccess) return loop_refused(L, g, s, "cudaGraphConditionalHandleCreate", e);
+  CUDA_CHECK(cudaStreamBeginCaptureToGraph(s, g, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
+  nka_loop_reset<<<greset, NKA_THREADS, 0, s>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
+  CUDA_CHECK(cudaGetLastError());
+  CUDA_CHECK(cudaStreamEndCapture(s, &g));
+  cudaGraphNode_t reset = nullptr;
+  size_t nnodes = 1;
+  CUDA_CHECK(cudaGraphGetNodes(g, &reset, &nnodes));
+  cudaGraphNodeParams cp = {};
+  cp.type = cudaGraphNodeTypeConditional;
+  cp.conditional.handle = cond;
+  cp.conditional.type = cudaGraphCondTypeWhile;
+  cp.conditional.size = 1;
+  cudaGraphNode_t wnode = nullptr;
+  e = cudaGraphAddNode(&wnode, g, &reset, 1, &cp);
+  if (e != cudaSuccess) return loop_refused(L, g, s, "cudaGraphAddNode (WHILE)", e);
+  cudaGraph_t body = cp.conditional.phGraph_out[0];
+
+  // the body: the caller's residual (cloned), then check, decide, update and step, captured after it
+  cudaGraphNode_t child = nullptr;
+  e = cudaGraphAddChildGraphNode(&child, body, nullptr, 0, (cudaGraph_t)residual_graph);
+  if (e != cudaSuccess) return loop_refused(L, g, s, "the residual graph cannot be a conditional body's child graph", e);
+  CUDA_CHECK(cudaStreamBeginCaptureToGraph(s, body, &child, nullptr, 1, cudaStreamCaptureModeThreadLocal));
+  const unsigned nbu = (unsigned)nb;
+  if (Vc == 2)
+    nka_loop_check<2><<<dim3(gc, nbu), NKA_THREADS, 0, s>>>(f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active,
+                                                           L->r0, L->rlast, L->hist, L->partials, prow, L->tickets,
+                                                           atol, rtol, maxit);
+  else
+    nka_loop_check<1><<<dim3(gc, nbu), NKA_THREADS, 0, s>>>(f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active,
+                                                           L->r0, L->rlast, L->hist, L->partials, prow, L->tickets,
+                                                           atol, rtol, maxit);
+  CUDA_CHECK(cudaGetLastError());
+  nka_loop_decide<<<1, 1024, 0, s>>>(L->active, bt->nbatch, cond);
+  CUDA_CHECK(cudaGetLastError());
+  nka_batch_update_captured(bt, f, ldf, L->active, s);
+  if (Vs == 2)
+    nka_loop_step<2><<<dim3(gs, nbu), NKA_THREADS, 0, s>>>(x, ldx, f, ldf, bt->vlen, L->active, L->iters);
+  else
+    nka_loop_step<1><<<dim3(gs, nbu), NKA_THREADS, 0, s>>>(x, ldx, f, ldf, bt->vlen, L->active, L->iters);
+  CUDA_CHECK(cudaGetLastError());
+  CUDA_CHECK(cudaStreamEndCapture(s, &body));
+
+  e = cudaGraphInstantiate(&L->exec, g, 0);
+  if (e != cudaSuccess) {
+    L->exec = nullptr;
+    return loop_refused(L, g, s, "cudaGraphInstantiate", e);
+  }
+  CUDA_CHECK(cudaGraphUpload(L->exec, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  CUDA_CHECK(cudaGraphDestroy(g));
+  CUDA_CHECK(cudaStreamDestroy(s));
+  return L;
+}
+
+extern "C" void nka_batch_loop_launch(NKABATCHLOOP L)
+{
+  NKA_REQUIRE(L != NULL, "nka_batch_loop_launch: null loop");
+  DeviceGuard guard(L->bt->device);
+  if (nka_capture_status(L->bt->stream) != 0)
+    nka_capture_fail("nka_batch_loop_launch", "a graph with conditional nodes cannot become a child of another graph");
+  CUDA_CHECK(cudaGraphLaunch(L->exec, L->bt->stream));
+}
+
+extern "C" void nka_batch_loop_results(NKABATCHLOOP L, int* iters, int* status, double* norm)
+{
+  NKA_REQUIRE(L != NULL && iters != NULL && status != NULL && norm != NULL, "nka_batch_loop_results: null argument");
+  NKABATCH bt = L->bt;
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, "nka_batch_loop_results", "it copies the loop's results to the host and synchronises");
+  const size_t nb = (size_t)bt->nbatch;
+  CUDA_CHECK(cudaMemcpyAsync(iters, L->iters, nb * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
+  CUDA_CHECK(cudaMemcpyAsync(status, L->status, nb * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
+  CUDA_CHECK(cudaMemcpyAsync(norm, L->rlast, nb * sizeof(double), cudaMemcpyDeviceToHost, bt->stream));
+  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+}
+
+extern "C" void nka_batch_loop_history(NKABATCHLOOP L, double* norms)
+{
+  NKA_REQUIRE(L != NULL && norms != NULL, "nka_batch_loop_history: null argument");
+  NKABATCH bt = L->bt;
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, "nka_batch_loop_history", "it copies the loop's history to the host and synchronises");
+  const size_t bytes = (size_t)(L->maxit + 1) * (size_t)bt->nbatch * sizeof(double);
+  CUDA_CHECK(cudaMemcpyAsync(norms, L->hist, bytes, cudaMemcpyDeviceToHost, bt->stream));
+  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+}
+
+extern "C" void nka_batch_loop_destroy(NKABATCHLOOP L)
+{
+  if (!L) return;
+  DeviceGuard guard(L->bt->device);
+  cudaStreamSynchronize(L->bt->stream);
+  loop_free(L);
+}

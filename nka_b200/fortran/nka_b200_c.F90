@@ -350,6 +350,49 @@ module nka_b200_c
       integer(c_long_long) :: n
     end function
 
+    !! ---- device-side fixed-point loops (include/nka_b200.h): the handle is a struct nka_batch_loop *
+
+    !! NKABATCHLOOP nka_batch_loop_create (NKABATCH, void *residual_graph, double *x_dev, size_t ldx,
+    !!                                     double *f_dev, size_t ldf, double atol, double rtol, int maxit)
+    !! residual_graph: a cudaGraph_t; x_dev, f_dev: device arrays of nbatch rows, passed as
+    !! nka_batch_accel_update's f_dev is.  c_null_ptr if CUDA refuses the graph.
+    function nka_batch_loop_create(batch, residual_graph, x_dev, ldx, f_dev, ldf, atol, rtol, maxit) &
+        bind(C, name='nka_batch_loop_create') result(handle)
+      import :: c_ptr, c_double, c_size_t, c_int
+      type(c_ptr), value :: batch, residual_graph
+      real(c_double), intent(inout) :: x_dev(*)
+      integer(c_size_t), value :: ldx
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      real(c_double), value :: atol, rtol
+      integer(c_int), value :: maxit
+      type(c_ptr) :: handle
+    end function
+
+    subroutine nka_batch_loop_launch(handle) bind(C, name='nka_batch_loop_launch')
+      import :: c_ptr
+      type(c_ptr), value :: handle
+    end subroutine
+
+    !! iters, status: c_loc of integer(c_int) arrays of nbatch elements on the host; norm: nbatch reals
+    subroutine nka_batch_loop_results(handle, iters, status, norm) bind(C, name='nka_batch_loop_results')
+      import :: c_ptr, c_double
+      type(c_ptr), value :: handle, iters, status
+      real(c_double), intent(out) :: norm(*)
+    end subroutine
+
+    !! norms: (maxit+1) x nbatch reals on the host, member index fastest
+    subroutine nka_batch_loop_history(handle, norms) bind(C, name='nka_batch_loop_history')
+      import :: c_ptr, c_double
+      type(c_ptr), value :: handle
+      real(c_double), intent(out) :: norms(*)
+    end subroutine
+
+    subroutine nka_batch_loop_destroy(handle) bind(C, name='nka_batch_loop_destroy')
+      import :: c_ptr
+      type(c_ptr), value :: handle
+    end subroutine
+
   end interface
 
 end module nka_b200_c
