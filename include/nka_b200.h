@@ -243,6 +243,49 @@ void nka_batch_loop_results (struct nka_batch_loop *L, int *iters, int *status, 
 void nka_batch_loop_history (struct nka_batch_loop *L, double *norms);
 void nka_batch_loop_destroy (struct nka_batch_loop *L);
 
+/* ---- device-side work queues: more fixed-point problems than members ---- */
+/* One graph launch solves nproblems independent problems x_p = G_p(x_p) on the
+ * batch's nbatch members, used as slots: when a slot's problem stops, the same
+ * launch writes that problem's final iterate out, loads the next problem into
+ * the slot and restarts the slot's accelerator, with no host round trip.
+ *
+ * x0_dev holds nproblems rows of vlen doubles (row stride ldx0): each problem's
+ * initial guess, read when the problem is claimed.  xout_dev receives each
+ * problem's final iterate (row stride ldxout) when it retires; xout_dev ==
+ * x0_dev solves in place.  x_dev, f_dev are the slots' rows (nbatch rows, as
+ * for nka_batch_loop_create).  slot_problem_dev is nbatch device ints the
+ * queue keeps: the problem slot b solves, or -1 while it is idle.  The
+ * residual graph reads it to find each row's parameters; it runs over every
+ * row, idle ones included, so it must accept -1 (its output there is ignored).
+ *
+ * Each problem stops by fixed_point_loop's rule: NONFINITE, CONVERGED when
+ * r < max(atol, rtol * r0_p), MAXIT after maxit steps.  Its final iterate,
+ * steps, status and norm are bit for bit what nka_batch_loop_create's loop
+ * gives it on a member just restarted with X row = its x0 row, whichever slot
+ * it lands in, whatever nbatch, that slot's earlier problems and the other
+ * slots hold.  Free slots take the next problem ids in slot order, so two
+ * launches on the same inputs assign slots alike.  A launch starts from
+ * problem 0 and the current x0 rows, and leaves every slot idle (-1).
+ *
+ * launch is queued on the batch's stream, aborts while that stream captures
+ * and is not counted by nka_batch_launch_count; results synchronise (refused
+ * while it captures).  create returns NULL, after printing CUDA's reason, on a
+ * residual graph CUDA refuses or a driver older than 12.4.
+ *
+ * The prototypes spell the handle as `struct nka_batch_queue *`, which
+ * NKABATCHQUEUE is. */
+typedef struct nka_batch_queue *NKABATCHQUEUE;
+struct nka_batch_queue *nka_batch_queue_create (struct nka_batch *b, void *residual_graph /* cudaGraph_t */,
+                                                double *x_dev, size_t ldx, double *f_dev, size_t ldf,
+                                                int *slot_problem_dev, const double *x0_dev, size_t ldx0,
+                                                double *xout_dev, size_t ldxout, size_t nproblems,
+                                                double atol, double rtol, int maxit);
+/* async on the batch's stream */
+void nka_batch_queue_launch (struct nka_batch_queue *Q);
+/* nproblems each: steps taken, NKA_LOOP_* status, final norm; synchronises */
+void nka_batch_queue_results (struct nka_batch_queue *Q, int *iters, int *status, double *norm);
+void nka_batch_queue_destroy (struct nka_batch_queue *Q);
+
 #ifdef __cplusplus
 }
 #endif

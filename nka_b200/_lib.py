@@ -102,6 +102,13 @@ SYMBOLS = {
     "nka_batch_loop_results": (None, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), _dp]),
     "nka_batch_loop_history": (None, [C.c_void_p, _dp]),
     "nka_batch_loop_destroy": (None, [C.c_void_p]),
+    # include/nka_b200.h: device-side work queues
+    "nka_batch_queue_create": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                            C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t,
+                                            C.c_double, C.c_double, C.c_int]),
+    "nka_batch_queue_launch": (None, [C.c_void_p]),
+    "nka_batch_queue_results": (None, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), _dp]),
+    "nka_batch_queue_destroy": (None, [C.c_void_p]),
     # include/nka_example.h
     "nka_system_init": (C.c_void_p, [C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),
     "nka_system_init_slab": (C.c_void_p, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),

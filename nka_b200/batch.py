@@ -24,7 +24,7 @@ class BatchNKA:
     def __init__(self, nbatch: int | None = None, vlen: int | None = None, mvec: int | None = None,
                  vtol: float = 0.01, device: int = -1, stream: int | None = None):
         self._h = None
-        self._loops = weakref.WeakSet()
+        self._loops = weakref.WeakSet()          # its device-side loops and queues
         self._lib = _lib.load()
         if nbatch is not None:
             self.init(nbatch, vlen, mvec, vtol=vtol, device=device, stream=stream)
@@ -176,25 +176,11 @@ class BatchNKA:
         torch ops; it is run once to warm up, then captured.  X, F: CUDA float64 tensors [nbatch, vlen]
         with unit column stride.  A member stops when ||F_b|| is not finite, when ||F_b|| <
         max(atol, rtol * (its norm at the launch's first check)), or after maxit steps."""
-        if isinstance(atol, bool) or not isinstance(atol, (int, float)) or not atol >= 0.0:
-            raise ValueError("atol must be a number >= 0")
-        if isinstance(rtol, bool) or not isinstance(rtol, (int, float)) or not rtol >= 0.0:
-            raise ValueError("rtol must be a number >= 0")
-        if isinstance(maxit, bool) or not isinstance(maxit, (int, np.integer)) or maxit < 0 or maxit > 2**31 - 2:
-            raise ValueError("maxit must be an integer >= 0")
+        _check_stopping(atol, rtol, maxit)
         ldx = self._rows(X, "X")
         ldf = self._rows(F, "F")
         h = self._uncaptured("fixed_point_loop", "it captures the residual and synchronises")
-        import torch
-        side = torch.cuda.Stream(device=F.device)
-        side.wait_stream(torch.cuda.current_stream(F.device))
-        with torch.cuda.stream(side):
-            residual()
-        torch.cuda.current_stream(F.device).wait_stream(side)
-        graph = torch.cuda.CUDAGraph(keep_graph=True)
-        with torch.cuda.graph(graph):
-            residual()
-        torch.cuda.synchronize(F.device)
+        graph = _capture(residual, F.device)
         loop = FixedPointLoop(self, graph, X, F, int(maxit))
         loop._h = self._lib.nka_batch_loop_create(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
                                                   float(atol), float(rtol), int(maxit))
@@ -203,6 +189,93 @@ class BatchNKA:
                            "has no conditional graph nodes (the reason is printed on stderr)")
         self._loops.add(loop)
         return loop
+
+    def _problem_rows(self, T, name: str, nproblems: int) -> int:
+        """The row stride of T, a float64 tensor [nproblems, vlen] with unit column stride (its device is
+        checked by the caller)."""
+        if not _is_torch(T):
+            raise ValueError("%s must be a CUDA float64 tensor of shape [nproblems, vlen]" % name)
+        import torch
+        if T.dtype != torch.float64 or T.dim() != 2 or tuple(T.shape) != (nproblems, self.vlen):
+            raise ValueError("%s must be a CUDA float64 tensor of shape [nproblems, vlen] = [%s, %d]"
+                             % (name, "nproblems" if nproblems is None else nproblems, self.vlen))
+        if T.stride(1) != 1 and self.vlen > 1:
+            raise ValueError("%s must have unit column stride (%s.stride(1) == 1)" % (name, name))
+        ld = T.stride(0)
+        if ld < self.vlen:
+            if nproblems > 1:
+                raise ValueError("%s's row stride must be >= vlen" % name)
+            ld = self.vlen                      # one row: its stride is never used to address anything
+        return ld
+
+    def fixed_point_queue(self, residual, X, F, slot_problem, X0, Xout=None, atol: float = 0.0, rtol: float = 1e-8,
+                          maxit: int = 100) -> "FixedPointQueue":
+        """Solve nproblems = X0.shape[0] problems x_p = G_p(x_p) on the members as slots, in one graph launch
+        (INTEGRATION.md section 9).  When a slot's problem stops, the launch writes its final iterate to
+        Xout[p], loads the next problem's X0 row into the slot and restarts the slot's accelerator.
+        residual: a zero-argument callable writing F = G(X) - X for every row with torch ops, reading
+        slot_problem (the problem of each row, -1 for an idle row, whose F is ignored) to find each row's
+        parameters; it is run once to warm up, then captured.  X, F: CUDA float64 [nbatch, vlen], the slots'
+        rows.  slot_problem: contiguous CUDA int32 [nbatch], set here to the launch's first assignment
+        (slot b solves problem b) and kept by the queue.  X0, Xout: CUDA float64 [nproblems, vlen] with unit
+        column stride; Xout=None solves in place (Xout is X0).  The stopping rule is fixed_point_loop's."""
+        _check_stopping(atol, rtol, maxit)
+        sp_bad = "slot_problem must be a contiguous CUDA int32 tensor of length nbatch = %d" % self.nbatch
+        if not _is_torch(slot_problem):
+            raise ValueError(sp_bad)
+        import torch
+        if slot_problem.dtype != torch.int32 or slot_problem.dim() != 1 or slot_problem.numel() != self.nbatch \
+                or (self.nbatch > 1 and slot_problem.stride(0) != 1):
+            raise ValueError(sp_bad)
+        nproblems = X0.shape[0] if _is_torch(X0) and X0.dim() == 2 else None
+        if nproblems is not None and not 1 <= nproblems <= 2**31 - 1:
+            raise ValueError("X0 must hold 1 to 2**31 - 1 problems (rows)")
+        ldx0 = self._problem_rows(X0, "X0", nproblems)
+        if Xout is None:
+            Xout = X0
+        ldxout = self._problem_rows(Xout, "Xout", nproblems)
+        for T, name in ((slot_problem, "slot_problem"), (X0, "X0"), (Xout, "Xout")):
+            if not T.is_cuda:
+                raise ValueError("%s must be a CUDA tensor: the batched accelerator is device-only" % name)
+        ldx = self._rows(X, "X")
+        ldf = self._rows(F, "F")
+        h = self._uncaptured("fixed_point_queue", "it captures the residual and synchronises")
+        ids = torch.arange(self.nbatch, dtype=torch.int32, device=slot_problem.device)
+        slot_problem.copy_(torch.where(ids < nproblems, ids, torch.full_like(ids, -1)))
+        graph = _capture(residual, F.device)
+        queue = FixedPointQueue(self, graph, X, F, slot_problem, X0, Xout, nproblems)
+        queue._h = self._lib.nka_batch_queue_create(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
+                                                    slot_problem.data_ptr(), X0.data_ptr(), ldx0, Xout.data_ptr(),
+                                                    ldxout, nproblems, float(atol), float(rtol), int(maxit))
+        if not queue._h:
+            raise NKAError("nka_batch_queue_create returned NULL: CUDA refused the residual graph or the driver "
+                           "has no conditional graph nodes (the reason is printed on stderr)")
+        self._loops.add(queue)
+        return queue
+
+
+def _check_stopping(atol, rtol, maxit):
+    if isinstance(atol, bool) or not isinstance(atol, (int, float)) or not atol >= 0.0:
+        raise ValueError("atol must be a number >= 0")
+    if isinstance(rtol, bool) or not isinstance(rtol, (int, float)) or not rtol >= 0.0:
+        raise ValueError("rtol must be a number >= 0")
+    if isinstance(maxit, bool) or not isinstance(maxit, (int, np.integer)) or maxit < 0 or maxit > 2**31 - 2:
+        raise ValueError("maxit must be an integer >= 0")
+
+
+def _capture(residual, device):
+    """residual() run once on a side stream to warm up, then captured into a kept torch CUDA graph."""
+    import torch
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    with torch.cuda.stream(side):
+        residual()
+    torch.cuda.current_stream(device).wait_stream(side)
+    graph = torch.cuda.CUDAGraph(keep_graph=True)
+    with torch.cuda.graph(graph):
+        residual()
+    torch.cuda.synchronize(device)
+    return graph
 
 
 class FixedPointLoop:
@@ -249,6 +322,54 @@ class FixedPointLoop:
     def destroy(self) -> None:
         if self._h:
             self._lib.nka_batch_loop_destroy(self._h)
+            self._h = None
+        self._batch._loops.discard(self)
+
+    def __del__(self):
+        try:
+            self.destroy()
+        except Exception:
+            pass
+
+
+class FixedPointQueue:
+    """A device-side work queue over a BatchNKA (BatchNKA.fixed_point_queue).  Keeps the captured residual
+    graph (and its memory pool), X, F, slot_problem, X0, Xout and the batch alive."""
+
+    def __init__(self, batch: BatchNKA, graph, X, F, slot_problem, X0, Xout, nproblems: int):
+        self._h = None
+        self._batch, self._graph, self._X, self._F = batch, graph, X, F
+        self._slot_problem, self.X0, self.Xout = slot_problem, X0, Xout
+        self._lib = batch._lib
+        self.nproblems = nproblems
+
+    def _handle(self, call: str, why: str):
+        if not self._h:
+            raise NKAError("fixed-point queue is destroyed")
+        self._batch._uncaptured(call, why)
+        return self._h
+
+    def run(self) -> None:
+        """One graph launch on the batch's stream: every problem from problem 0 and the current X0 rows to its
+        end, results in Xout.  Returns at once."""
+        self._lib.nka_batch_queue_launch(self._handle(
+            "run", "a graph with conditional nodes cannot become a child of another graph"))
+
+    def results(self):
+        """(steps, status, norm) per problem as numpy arrays; status is one of RUNNING, CONVERGED, MAXIT,
+        NONFINITE.  Synchronises."""
+        h = self._handle("results", "it copies the queue's results to the host and synchronises")
+        n = self.nproblems
+        it = np.zeros(n, dtype=np.int32)
+        st = np.zeros(n, dtype=np.int32)
+        norm = np.zeros(n, dtype=np.float64)
+        self._lib.nka_batch_queue_results(h, it.ctypes.data_as(C.POINTER(C.c_int)), st.ctypes.data_as(C.POINTER(C.c_int)),
+                                          norm.ctypes.data_as(C.POINTER(C.c_double)))
+        return it, st, norm
+
+    def destroy(self) -> None:
+        if self._h:
+            self._lib.nka_batch_queue_destroy(self._h)
             self._h = None
         self._batch._loops.discard(self)
 

@@ -360,6 +360,12 @@ extern "C" void nka_batch_restart(NKABATCH bt, const unsigned char* mask)
   batch_launched(bt, cap, 1);
 }
 
+void nka_batch_restart_captured(NKABATCH bt, const unsigned char* mask, cudaStream_t stream)
+{
+  nka_batch_restart_kernel<<<bt->nbatch, NKA_STATE_THREADS, 0, stream>>>(bt->S, mask);
+  batch_launched(bt, true, 1);
+}
+
 extern "C" void nka_batch_set_vec_tol(NKABATCH bt, double vtol)
 {
   NKA_REQUIRE(bt != NULL, "nka_batch_set_vec_tol: null handle");

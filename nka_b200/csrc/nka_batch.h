@@ -1,7 +1,9 @@
 // nka_batch.h -- the batched accelerator's handle and kernel tables (nka_batch.cu, nka_batch_pass_a.cu,
-// nka_batch_pass_b.cu), shared with its device-side fixed-point loops (nka_batch_loop.cu).
+// nka_batch_pass_b.cu), shared with its device-side fixed-point loops (nka_batch_loop.cu) and work
+// queues (nka_batch_queue.cu).
 #pragma once
 #include <cuda_runtime.h>
+#include <functional>
 #include "nka_dispatch.h"
 
 struct nka_batch {
@@ -28,6 +30,28 @@ struct nka_batch {
 // One batched update queued on `stream` while that stream captures (a loop's body graph): the update
 // nka_batch_accel_update queues, counted as no launch, whatever stream the handle itself uses.
 void nka_batch_update_captured(nka_batch* bt, double* f, size_t ldf, const unsigned char* active, cudaStream_t stream);
+// nka_batch_restart of the masked members, queued on a capturing `stream` likewise.
+void nka_batch_restart_captured(nka_batch* bt, const unsigned char* mask, cudaStream_t stream);
+
+// ---- shared by the device-side loops and queues (nka_batch_loop.cu) ----
+// 0 if the driver has conditional graph nodes (12.4); otherwise prints why `call` cannot build its graph.
+int nka_loop_driver_refused(const char* call);
+// CTAs per member of the loop's check and step kernels at access width V (vlen only, as the batch's fix-up)
+int nka_loop_grid(nka_batch* bt, int V);
+// nka_loop_check<V> / nka_loop_step<V> queued on `s` over dim3(grid, nbatch) (nka_batch_loop.cu documents
+// them); check k of member b is recorded at hist[k * hstride + b]
+void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, const double* F, size_t ldf, size_t n,
+                          int hstride, const int* iters, int* status, unsigned char* active, double* r0, double* rlast,
+                          double* hist, double* partials, size_t prow, unsigned* tickets, double atol, double rtol,
+                          int maxit);
+void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
+                         size_t n, int nbatch, const unsigned char* active, int* iters);
+// The graph  prologue -> WHILE (cond) { residual graph, cloned as a child -> body }, instantiated and
+// uploaded on `s`.  prologue and body queue their kernels on `s` while it captures.  A graph CUDA
+// refuses gives nullptr, after printing CUDA's reason under `call`, with no error left behind.
+typedef std::function<void(cudaStream_t, cudaGraphConditionalHandle)> NkaCaptureFn;
+cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t residual, const NkaCaptureFn& prologue,
+                                const NkaCaptureFn& body);
 
 // (F, ldf, W, wstride, ld, n, S, partials, prow, tickets, dots, active)
 typedef void (*NkaBatchPassAFn)(const double*, size_t, const double*, size_t, size_t, size_t, const NkaDevState*, double*,

@@ -15,6 +15,9 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <algorithm>
+#include <vector>
+
 #include "../../include/nka_b200.h"
 #include "nka_internal.h"
 #include "nka_batch.h"
@@ -134,22 +137,115 @@ static void loop_free(NKABATCHLOOP L)
   delete L;
 }
 
-// CUDA refused the graph: the caller's residual graph or the driver.  Not a library fault: print CUDA's
-// reason, clear the (non-sticky) error and let the caller decide.
-static NKABATCHLOOP loop_refused(NKABATCHLOOP L, cudaGraph_t g, cudaStream_t s, const char* what, cudaError_t e)
+// ---------------------------------------------------------------------------
+// shared with the work queues (nka_batch_queue.cu)
+// ---------------------------------------------------------------------------
+int nka_loop_driver_refused(const char* call)
 {
-  fprintf(stderr, "nka_b200: nka_batch_loop_create: %s: %s\n", what, cudaGetErrorString(e));
+  int driver = 0;
+  CUDA_CHECK(cudaDriverGetVersion(&driver));
+  if (driver >= 12040) return 0;
+  fprintf(stderr, "nka_b200: %s: conditional graph nodes need a CUDA 12.4 driver, this one is %d.%d: %s\n", call,
+          driver / 1000, (driver % 1000) / 10, cudaGetErrorString(cudaErrorInsufficientDriver));
   fflush(stderr);
-  cudaGetLastError();
-  if (g) cudaGraphDestroy(g);
-  cudaStreamDestroy(s);
-  loop_free(L);
-  return nullptr;
+  return 1;
 }
 
 // CTAs per member of check and step: the batch's rule for a one-accumulator sweep of vlen (its fix-up's)
-static int loop_grid(NKABATCH bt, int V) { return nka_grid_for(bt->geom, 4, bt->vlen, V, NKA_THREADS); }
+int nka_loop_grid(NKABATCH bt, int V) { return nka_grid_for(bt->geom, 4, bt->vlen, V, NKA_THREADS); }
 
+void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, const double* F, size_t ldf, size_t n,
+                          int hstride, const int* iters, int* status, unsigned char* active, double* r0, double* rlast,
+                          double* hist, double* partials, size_t prow, unsigned* tickets, double atol, double rtol,
+                          int maxit)
+{
+  const dim3 g(grid, (unsigned)nbatch);
+  if (V == 2)
+    nka_loop_check<2><<<g, NKA_THREADS, 0, s>>>(F, ldf, n, hstride, iters, status, active, r0, rlast, hist, partials, prow,
+                                                tickets, atol, rtol, maxit);
+  else
+    nka_loop_check<1><<<g, NKA_THREADS, 0, s>>>(F, ldf, n, hstride, iters, status, active, r0, rlast, hist, partials, prow,
+                                                tickets, atol, rtol, maxit);
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
+                         size_t n, int nbatch, const unsigned char* active, int* iters)
+{
+  const dim3 g(grid, (unsigned)nbatch);
+  if (V == 2)
+    nka_loop_step<2><<<g, NKA_THREADS, 0, s>>>(X, ldx, F, ldf, n, active, iters);
+  else
+    nka_loop_step<1><<<g, NKA_THREADS, 0, s>>>(X, ldx, F, ldf, n, active, iters);
+  CUDA_CHECK(cudaGetLastError());
+}
+
+// CUDA refused the graph: the caller's residual graph or the driver.  Not a library fault: print CUDA's
+// reason, clear the (non-sticky) error and let the caller decide.
+static cudaGraphExec_t graph_refused(const char* call, cudaGraph_t g, const char* what, cudaError_t e)
+{
+  fprintf(stderr, "nka_b200: %s: %s: %s\n", call, what, cudaGetErrorString(e));
+  fflush(stderr);
+  cudaGetLastError();
+  if (g) cudaGraphDestroy(g);
+  return nullptr;
+}
+
+cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t residual, const NkaCaptureFn& prologue,
+                                const NkaCaptureFn& body_fn)
+{
+  cudaGraph_t g = nullptr;
+  CUDA_CHECK(cudaGraphCreate(&g, 0));
+  cudaGraphConditionalHandle cond;
+  cudaError_t e = cudaGraphConditionalHandleCreate(&cond, g, 1, cudaGraphCondAssignDefault);
+  if (e != cudaSuccess) return graph_refused(call, g, "cudaGraphConditionalHandleCreate", e);
+  CUDA_CHECK(cudaStreamBeginCaptureToGraph(s, g, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
+  prologue(s, cond);
+  CUDA_CHECK(cudaStreamEndCapture(s, &g));
+  // the prologue is a chain: the WHILE node follows its one node without a dependent
+  size_t nnodes = 0, nedges = 0;
+  CUDA_CHECK(cudaGraphGetNodes(g, nullptr, &nnodes));
+  CUDA_CHECK(cudaGraphGetEdges(g, nullptr, nullptr, &nedges));
+  std::vector<cudaGraphNode_t> nodes(nnodes), from(nedges), to(nedges);
+  CUDA_CHECK(cudaGraphGetNodes(g, nodes.data(), &nnodes));
+  if (nedges) CUDA_CHECK(cudaGraphGetEdges(g, from.data(), to.data(), &nedges));
+  cudaGraphNode_t tail = nullptr;
+  int ntails = 0;
+  for (cudaGraphNode_t nd : nodes)
+    if (std::find(from.begin(), from.end(), nd) == from.end()) {
+      tail = nd;
+      ++ntails;
+    }
+  NKA_REQUIRE(ntails == 1, "nka_while_graph: the prologue must end in exactly one node (a chain)");
+  cudaGraphNodeParams cp = {};
+  cp.type = cudaGraphNodeTypeConditional;
+  cp.conditional.handle = cond;
+  cp.conditional.type = cudaGraphCondTypeWhile;
+  cp.conditional.size = 1;
+  cudaGraphNode_t wnode = nullptr;
+  e = cudaGraphAddNode(&wnode, g, &tail, 1, &cp);
+  if (e != cudaSuccess) return graph_refused(call, g, "cudaGraphAddNode (WHILE)", e);
+  cudaGraph_t body = cp.conditional.phGraph_out[0];
+
+  // the body: the caller's residual (cloned), then the body's kernels, captured after it
+  cudaGraphNode_t child = nullptr;
+  e = cudaGraphAddChildGraphNode(&child, body, nullptr, 0, residual);
+  if (e != cudaSuccess) return graph_refused(call, g, "the residual graph cannot be a conditional body's child graph", e);
+  CUDA_CHECK(cudaStreamBeginCaptureToGraph(s, body, &child, nullptr, 1, cudaStreamCaptureModeThreadLocal));
+  body_fn(s, cond);
+  CUDA_CHECK(cudaStreamEndCapture(s, &body));
+
+  cudaGraphExec_t exec = nullptr;
+  e = cudaGraphInstantiate(&exec, g, 0);
+  if (e != cudaSuccess) return graph_refused(call, g, "cudaGraphInstantiate", e);
+  CUDA_CHECK(cudaGraphUpload(exec, s));
+  CUDA_CHECK(cudaGraphDestroy(g));
+  return exec;
+}
+
+// ---------------------------------------------------------------------------
+// the handle's entry points
+// ---------------------------------------------------------------------------
 extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
                                              size_t ldf, double atol, double rtol, int maxit)
 {
@@ -161,14 +257,7 @@ extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph,
   NKA_REQUIRE(maxit >= 0, "nka_batch_loop_create: maxit must be >= 0");
   DeviceGuard guard(bt->device);
   nka_refuse_capture(bt->stream, "nka_batch_loop_create", "it builds and uploads a graph and synchronises");
-  int driver = 0;
-  CUDA_CHECK(cudaDriverGetVersion(&driver));
-  if (driver < 12040) {
-    fprintf(stderr, "nka_b200: nka_batch_loop_create: conditional graph nodes need a CUDA 12.4 driver, this one is "
-                    "%d.%d: %s\n", driver / 1000, (driver % 1000) / 10, cudaGetErrorString(cudaErrorInsufficientDriver));
-    fflush(stderr);
-    return nullptr;
-  }
+  if (nka_loop_driver_refused("nka_batch_loop_create")) return nullptr;
 
   NKABATCHLOOP L = new nka_batch_loop();
   L->bt = bt;
@@ -178,7 +267,7 @@ extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph,
   // the 16-byte paths need every row 16-byte aligned: the base address and an even row stride
   const int Vc = ((uintptr_t)f % 16 == 0 && ldf % 2 == 0) ? 2 : 1;
   const int Vs = Vc == 2 && (uintptr_t)x % 16 == 0 && ldx % 2 == 0 ? 2 : 1;
-  const unsigned gc = (unsigned)loop_grid(bt, Vc), gs = (unsigned)loop_grid(bt, Vs);
+  const unsigned gc = (unsigned)nka_loop_grid(bt, Vc), gs = (unsigned)nka_loop_grid(bt, Vs);
   const size_t prow = gc;
   CUDA_CHECK(cudaMalloc(&L->iters, nb * sizeof(int)));
   CUDA_CHECK(cudaMalloc(&L->status, nb * sizeof(int)));
@@ -201,62 +290,26 @@ extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph,
   nka_loop_reset<<<greset, NKA_THREADS, 0, s>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
   CUDA_CHECK(cudaGetLastError());
 
-  // reset, then the WHILE node
-  cudaGraph_t g = nullptr;
-  CUDA_CHECK(cudaGraphCreate(&g, 0));
-  cudaGraphConditionalHandle cond;
-  cudaError_t e = cudaGraphConditionalHandleCreate(&cond, g, 1, cudaGraphCondAssignDefault);
-  if (e != cudaSuccess) return loop_refused(L, g, s, "cudaGraphConditionalHandleCreate", e);
-  CUDA_CHECK(cudaStreamBeginCaptureToGraph(s, g, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
-  nka_loop_reset<<<greset, NKA_THREADS, 0, s>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
-  CUDA_CHECK(cudaGetLastError());
-  CUDA_CHECK(cudaStreamEndCapture(s, &g));
-  cudaGraphNode_t reset = nullptr;
-  size_t nnodes = 1;
-  CUDA_CHECK(cudaGraphGetNodes(g, &reset, &nnodes));
-  cudaGraphNodeParams cp = {};
-  cp.type = cudaGraphNodeTypeConditional;
-  cp.conditional.handle = cond;
-  cp.conditional.type = cudaGraphCondTypeWhile;
-  cp.conditional.size = 1;
-  cudaGraphNode_t wnode = nullptr;
-  e = cudaGraphAddNode(&wnode, g, &reset, 1, &cp);
-  if (e != cudaSuccess) return loop_refused(L, g, s, "cudaGraphAddNode (WHILE)", e);
-  cudaGraph_t body = cp.conditional.phGraph_out[0];
-
-  // the body: the caller's residual (cloned), then check, decide, update and step, captured after it
-  cudaGraphNode_t child = nullptr;
-  e = cudaGraphAddChildGraphNode(&child, body, nullptr, 0, (cudaGraph_t)residual_graph);
-  if (e != cudaSuccess) return loop_refused(L, g, s, "the residual graph cannot be a conditional body's child graph", e);
-  CUDA_CHECK(cudaStreamBeginCaptureToGraph(s, body, &child, nullptr, 1, cudaStreamCaptureModeThreadLocal));
-  const unsigned nbu = (unsigned)nb;
-  if (Vc == 2)
-    nka_loop_check<2><<<dim3(gc, nbu), NKA_THREADS, 0, s>>>(f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active,
-                                                           L->r0, L->rlast, L->hist, L->partials, prow, L->tickets,
-                                                           atol, rtol, maxit);
-  else
-    nka_loop_check<1><<<dim3(gc, nbu), NKA_THREADS, 0, s>>>(f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active,
-                                                           L->r0, L->rlast, L->hist, L->partials, prow, L->tickets,
-                                                           atol, rtol, maxit);
-  CUDA_CHECK(cudaGetLastError());
-  nka_loop_decide<<<1, 1024, 0, s>>>(L->active, bt->nbatch, cond);
-  CUDA_CHECK(cudaGetLastError());
-  nka_batch_update_captured(bt, f, ldf, L->active, s);
-  if (Vs == 2)
-    nka_loop_step<2><<<dim3(gs, nbu), NKA_THREADS, 0, s>>>(x, ldx, f, ldf, bt->vlen, L->active, L->iters);
-  else
-    nka_loop_step<1><<<dim3(gs, nbu), NKA_THREADS, 0, s>>>(x, ldx, f, ldf, bt->vlen, L->active, L->iters);
-  CUDA_CHECK(cudaGetLastError());
-  CUDA_CHECK(cudaStreamEndCapture(s, &body));
-
-  e = cudaGraphInstantiate(&L->exec, g, 0);
-  if (e != cudaSuccess) {
-    L->exec = nullptr;
-    return loop_refused(L, g, s, "cudaGraphInstantiate", e);
+  // reset, then the WHILE node: { residual, check, decide, update, step }
+  auto prologue = [&](cudaStream_t cs, cudaGraphConditionalHandle) {
+    nka_loop_reset<<<greset, NKA_THREADS, 0, cs>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
+    CUDA_CHECK(cudaGetLastError());
+  };
+  auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
+    nka_loop_queue_check(Vc, gc, bt->nbatch, cs, f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active, L->r0, L->rlast,
+                         L->hist, L->partials, prow, L->tickets, atol, rtol, maxit);
+    nka_loop_decide<<<1, 1024, 0, cs>>>(L->active, bt->nbatch, cond);
+    CUDA_CHECK(cudaGetLastError());
+    nka_batch_update_captured(bt, f, ldf, L->active, cs);
+    nka_loop_queue_step(Vs, gs, cs, x, ldx, f, ldf, bt->vlen, bt->nbatch, L->active, L->iters);
+  };
+  L->exec = nka_while_graph("nka_batch_loop_create", s, (cudaGraph_t)residual_graph, prologue, body);
+  if (!L->exec) {
+    cudaStreamDestroy(s);
+    loop_free(L);
+    return nullptr;
   }
-  CUDA_CHECK(cudaGraphUpload(L->exec, s));
   CUDA_CHECK(cudaStreamSynchronize(s));
-  CUDA_CHECK(cudaGraphDestroy(g));
   CUDA_CHECK(cudaStreamDestroy(s));
   return L;
 }

@@ -393,6 +393,50 @@ module nka_b200_c
       type(c_ptr), value :: handle
     end subroutine
 
+    !! ---- device-side work queues (include/nka_b200.h): the handle is a struct nka_batch_queue *
+
+    !! NKABATCHQUEUE nka_batch_queue_create (NKABATCH, void *residual_graph, double *x_dev, size_t ldx,
+    !!     double *f_dev, size_t ldf, int *slot_problem_dev, const double *x0_dev, size_t ldx0,
+    !!     double *xout_dev, size_t ldxout, size_t nproblems, double atol, double rtol, int maxit)
+    !! x_dev, f_dev: nbatch rows; x0_dev, xout_dev: nproblems rows, passed as nka_batch_accel_update's
+    !! f_dev is; slot_problem_dev: the device address of nbatch integer(c_int).  c_null_ptr if CUDA
+    !! refuses the graph.
+    function nka_batch_queue_create(batch, residual_graph, x_dev, ldx, f_dev, ldf, slot_problem_dev, x0_dev, ldx0, &
+                                    xout_dev, ldxout, nproblems, atol, rtol, maxit) &
+        bind(C, name='nka_batch_queue_create') result(handle)
+      import :: c_ptr, c_double, c_size_t, c_int
+      type(c_ptr), value :: batch, residual_graph
+      real(c_double), intent(inout) :: x_dev(*)
+      integer(c_size_t), value :: ldx
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      type(c_ptr), value :: slot_problem_dev
+      real(c_double), intent(in) :: x0_dev(*)
+      integer(c_size_t), value :: ldx0
+      real(c_double), intent(inout) :: xout_dev(*)
+      integer(c_size_t), value :: ldxout, nproblems
+      real(c_double), value :: atol, rtol
+      integer(c_int), value :: maxit
+      type(c_ptr) :: handle
+    end function
+
+    subroutine nka_batch_queue_launch(handle) bind(C, name='nka_batch_queue_launch')
+      import :: c_ptr
+      type(c_ptr), value :: handle
+    end subroutine
+
+    !! iters, status: c_loc of integer(c_int) arrays of nproblems elements on the host; norm: nproblems reals
+    subroutine nka_batch_queue_results(handle, iters, status, norm) bind(C, name='nka_batch_queue_results')
+      import :: c_ptr, c_double
+      type(c_ptr), value :: handle, iters, status
+      real(c_double), intent(out) :: norm(*)
+    end subroutine
+
+    subroutine nka_batch_queue_destroy(handle) bind(C, name='nka_batch_queue_destroy')
+      import :: c_ptr
+      type(c_ptr), value :: handle
+    end subroutine
+
   end interface
 
 end module nka_b200_c
