@@ -286,6 +286,53 @@ void nka_batch_queue_launch (struct nka_batch_queue *Q);
 void nka_batch_queue_results (struct nka_batch_queue *Q, int *iters, int *status, double *norm);
 void nka_batch_queue_destroy (struct nka_batch_queue *Q);
 
+/* ---- per-problem stopping tests for device-side loops and queues -------- */
+/* The _stop creates take the stopping rule as a struct.  For member p of a loop,
+ * or problem p of a queue, at check k, with r0_p its norm at check 0:
+ *
+ *   r = || s_b . F_b ||_2      (s_b = row b of scale_dev; no scale: ||F_b||_2)
+ *   NONFINITE  if r is not finite
+ *   CONVERGED  else if r < fmax(atol_p, rtol_p * r0_p)
+ *   DIVERGED   else if dtol > 0 and r > dtol * r0_p
+ *   MAXIT      else if k >= maxit_p,  maxit_p = min(max(maxit_dev[p], 0), maxit)
+ *
+ * evaluated as written, in IEEE double (fmax included: a NaN atol_p or rtol_p
+ * term drops out of it).  atol_p is atol_dev[p] when atol_dev is given, else
+ * atol; rtol_p and maxit_p likewise.  In a loop p = b; in a queue p =
+ * slot_problem[b], the problem slot b holds.  The arrays are device memory,
+ * read at every launch (the caller may change them between launches).
+ *
+ * scale_dev: NULL, or nbatch rows (slots, shaped like f_dev) of vlen doubles at
+ * row stride ldscale >= vlen, read after the residual graph in every
+ * iteration: the residual graph may write it, e.g. weights 1/(atol_i +
+ * rtol*|x_i|) from X.  Per element t = s_i * f_i; r^2 accumulates fma(t, t, .)
+ * in the order and on the CTAs of the unscaled norm, so a scale of 1.0 gives
+ * the unscaled bits, and the bits never depend on where the scale rows sit.
+ * The iteration itself (the accelerator, X_b += F_b) always uses F unscaled.
+ *
+ * create aborts (file:line) on a NULL stop, atol or rtol < 0 (or NaN),
+ * maxit < 0, dtol neither 0 nor >= 1, or a scale with ldscale < vlen.  The
+ * scalar maxit also sizes a loop's history: (maxit+1) x nbatch.
+ * nka_batch_loop_create / nka_batch_queue_create are the _stop creates with
+ * {atol, rtol, 0, maxit, NULL, NULL, NULL, NULL, 0}. */
+#define NKA_LOOP_DIVERGED  4     /* r > dtol * r0: its X row keeps its last finite iterate */
+typedef struct nka_stop_test {
+  double atol, rtol, dtol;           /* dtol = 0: off; else >= 1 */
+  int maxit;                         /* >= 0; bounds maxit_dev entries and the loop's history */
+  const double *atol_dev, *rtol_dev; /* NULL, or one per member (loop) / per problem (queue), device */
+  const int *maxit_dev;              /* likewise */
+  const double *scale_dev;           /* NULL, or nbatch rows of vlen doubles at stride ldscale, device */
+  size_t ldscale;
+} nka_stop_test;
+struct nka_batch_loop *nka_batch_loop_create_stop (struct nka_batch *b, void *residual_graph /* cudaGraph_t */,
+                                                   double *x_dev, size_t ldx, double *f_dev, size_t ldf,
+                                                   const nka_stop_test *stop);
+struct nka_batch_queue *nka_batch_queue_create_stop (struct nka_batch *b, void *residual_graph /* cudaGraph_t */,
+                                                     double *x_dev, size_t ldx, double *f_dev, size_t ldf,
+                                                     int *slot_problem_dev, const double *x0_dev, size_t ldx0,
+                                                     double *xout_dev, size_t ldxout, size_t nproblems,
+                                                     const nka_stop_test *stop);
+
 #ifdef __cplusplus
 }
 #endif

@@ -25,6 +25,15 @@ class StateView(C.Structure):
     ]
 
 
+class StopTest(C.Structure):
+    """include/nka_b200.h: nka_stop_test"""
+    _fields_ = [
+        ("atol", C.c_double), ("rtol", C.c_double), ("dtol", C.c_double), ("maxit", C.c_int),
+        ("atol_dev", C.c_void_p), ("rtol_dev", C.c_void_p), ("maxit_dev", C.c_void_p),
+        ("scale_dev", C.c_void_p), ("ldscale", C.c_size_t),
+    ]
+
+
 # every symbol include/*.h declares: name -> (restype, argtypes)
 _dp = C.POINTER(C.c_double)
 SYMBOLS = {
@@ -109,6 +118,12 @@ SYMBOLS = {
     "nka_batch_queue_launch": (None, [C.c_void_p]),
     "nka_batch_queue_results": (None, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), _dp]),
     "nka_batch_queue_destroy": (None, [C.c_void_p]),
+    # include/nka_b200.h: per-problem stopping tests
+    "nka_batch_loop_create_stop": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                                C.POINTER(StopTest)]),
+    "nka_batch_queue_create_stop": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                                 C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t,
+                                                 C.POINTER(StopTest)]),
     # include/nka_example.h
     "nka_system_init": (C.c_void_p, [C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),
     "nka_system_init_slab": (C.c_void_p, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),

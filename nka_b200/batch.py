@@ -169,21 +169,31 @@ class BatchNKA:
         return self._lib.nka_batch_launch_count(self._handle())
 
     # -- device-side fixed-point loops --------------------------------------
-    def fixed_point_loop(self, residual, X, F, atol: float = 0.0, rtol: float = 1e-8,
-                         maxit: int = 100) -> "FixedPointLoop":
+    def fixed_point_loop(self, residual, X, F, atol=0.0, rtol=1e-8, maxit=100, dtol: float = 0.0,
+                         scale=None) -> "FixedPointLoop":
         """A solve of x_b = G(x_b) for every member that runs to its end in one graph launch
         (INTEGRATION.md section 8).  residual: a zero-argument callable writing F = G(X) - X in place with
         torch ops; it is run once to warm up, then captured.  X, F: CUDA float64 tensors [nbatch, vlen]
-        with unit column stride.  A member stops when ||F_b|| is not finite, when ||F_b|| <
-        max(atol, rtol * (its norm at the launch's first check)), or after maxit steps."""
-        _check_stopping(atol, rtol, maxit)
+        with unit column stride.  With r = ||F_b|| (or ||scale_b * F_b||), a member stops when r is not
+        finite (NONFINITE), when r < max(atol_b, rtol_b * r0_b) (CONVERGED, r0_b = its r at the launch's
+        first check), when dtol > 0 and r > dtol * r0_b (DIVERGED), or after maxit_b steps (MAXIT).
+        atol, rtol: a number >= 0 or a contiguous CUDA float64 tensor of nbatch entries; maxit: an int >= 0
+        or a contiguous CUDA int32 tensor of nbatch entries (the loop's history then has max(maxit) + 1
+        rows); dtol: 0 (off) or >= 1; scale: None or a CUDA float64 tensor [nbatch, vlen] with unit column
+        stride, read after the residual in every iteration, so the residual may rewrite it
+        (INTEGRATION.md section 9a)."""
+        _check_stopping(atol, rtol, maxit, dtol)
+        _check_lengths(self.nbatch, "nbatch", atol, rtol, maxit)
+        ldscale = self._rows(scale, "scale") if scale is not None else 0
         ldx = self._rows(X, "X")
         ldf = self._rows(F, "F")
         h = self._uncaptured("fixed_point_loop", "it captures the residual and synchronises")
+        stop = _stop_test(atol, rtol, maxit, dtol, scale, ldscale)
         graph = _capture(residual, F.device)
-        loop = FixedPointLoop(self, graph, X, F, int(maxit))
-        loop._h = self._lib.nka_batch_loop_create(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
-                                                  float(atol), float(rtol), int(maxit))
+        loop = FixedPointLoop(self, graph, X, F, stop.maxit)
+        loop._stop = (atol, rtol, maxit, scale)
+        loop._h = self._lib.nka_batch_loop_create_stop(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
+                                                       C.byref(stop))
         if not loop._h:
             raise NKAError("nka_batch_loop_create returned NULL: CUDA refused the residual graph or the driver "
                            "has no conditional graph nodes (the reason is printed on stderr)")
@@ -208,8 +218,8 @@ class BatchNKA:
             ld = self.vlen                      # one row: its stride is never used to address anything
         return ld
 
-    def fixed_point_queue(self, residual, X, F, slot_problem, X0, Xout=None, atol: float = 0.0, rtol: float = 1e-8,
-                          maxit: int = 100) -> "FixedPointQueue":
+    def fixed_point_queue(self, residual, X, F, slot_problem, X0, Xout=None, atol=0.0, rtol=1e-8,
+                          maxit=100, dtol: float = 0.0, scale=None) -> "FixedPointQueue":
         """Solve nproblems = X0.shape[0] problems x_p = G_p(x_p) on the members as slots, in one graph launch
         (INTEGRATION.md section 9).  When a slot's problem stops, the launch writes its final iterate to
         Xout[p], loads the next problem's X0 row into the slot and restarts the slot's accelerator.
@@ -218,8 +228,10 @@ class BatchNKA:
         parameters; it is run once to warm up, then captured.  X, F: CUDA float64 [nbatch, vlen], the slots'
         rows.  slot_problem: contiguous CUDA int32 [nbatch], set here to the launch's first assignment
         (slot b solves problem b) and kept by the queue.  X0, Xout: CUDA float64 [nproblems, vlen] with unit
-        column stride; Xout=None solves in place (Xout is X0).  The stopping rule is fixed_point_loop's."""
-        _check_stopping(atol, rtol, maxit)
+        column stride; Xout=None solves in place (Xout is X0).  The stopping rule is fixed_point_loop's,
+        with tensor atol, rtol and maxit holding one entry per problem (nproblems), found through
+        slot_problem; scale is per slot, [nbatch, vlen], like F."""
+        _check_stopping(atol, rtol, maxit, dtol)
         sp_bad = "slot_problem must be a contiguous CUDA int32 tensor of length nbatch = %d" % self.nbatch
         if not _is_torch(slot_problem):
             raise ValueError(sp_bad)
@@ -237,16 +249,20 @@ class BatchNKA:
         for T, name in ((slot_problem, "slot_problem"), (X0, "X0"), (Xout, "Xout")):
             if not T.is_cuda:
                 raise ValueError("%s must be a CUDA tensor: the batched accelerator is device-only" % name)
+        _check_lengths(nproblems, "nproblems", atol, rtol, maxit)
+        ldscale = self._rows(scale, "scale") if scale is not None else 0
         ldx = self._rows(X, "X")
         ldf = self._rows(F, "F")
         h = self._uncaptured("fixed_point_queue", "it captures the residual and synchronises")
+        stop = _stop_test(atol, rtol, maxit, dtol, scale, ldscale)
         ids = torch.arange(self.nbatch, dtype=torch.int32, device=slot_problem.device)
         slot_problem.copy_(torch.where(ids < nproblems, ids, torch.full_like(ids, -1)))
         graph = _capture(residual, F.device)
         queue = FixedPointQueue(self, graph, X, F, slot_problem, X0, Xout, nproblems)
-        queue._h = self._lib.nka_batch_queue_create(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
-                                                    slot_problem.data_ptr(), X0.data_ptr(), ldx0, Xout.data_ptr(),
-                                                    ldxout, nproblems, float(atol), float(rtol), int(maxit))
+        queue._stop = (atol, rtol, maxit, scale)
+        queue._h = self._lib.nka_batch_queue_create_stop(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
+                                                         slot_problem.data_ptr(), X0.data_ptr(), ldx0, Xout.data_ptr(),
+                                                         ldxout, nproblems, C.byref(stop))
         if not queue._h:
             raise NKAError("nka_batch_queue_create returned NULL: CUDA refused the residual graph or the driver "
                            "has no conditional graph nodes (the reason is printed on stderr)")
@@ -254,13 +270,54 @@ class BatchNKA:
         return queue
 
 
-def _check_stopping(atol, rtol, maxit):
-    if isinstance(atol, bool) or not isinstance(atol, (int, float)) or not atol >= 0.0:
-        raise ValueError("atol must be a number >= 0")
-    if isinstance(rtol, bool) or not isinstance(rtol, (int, float)) or not rtol >= 0.0:
-        raise ValueError("rtol must be a number >= 0")
-    if isinstance(maxit, bool) or not isinstance(maxit, (int, np.integer)) or maxit < 0 or maxit > 2**31 - 2:
+def _check_stopping(atol, rtol, maxit, dtol):
+    """Numbers, or tensors of the right kind (their length is _check_lengths', their entries _stop_test's)."""
+    for v, name in ((atol, "atol"), (rtol, "rtol")):
+        if _is_torch(v):
+            import torch
+            if v.dtype != torch.float64 or v.dim() != 1 or not v.is_cuda or (v.numel() > 1 and v.stride(0) != 1):
+                raise ValueError("%s must be a number >= 0 or a contiguous 1-D CUDA float64 tensor" % name)
+        elif isinstance(v, bool) or not isinstance(v, (int, float)) or not v >= 0.0:
+            raise ValueError("%s must be a number >= 0" % name)
+    if _is_torch(maxit):
+        import torch
+        if maxit.dtype != torch.int32 or maxit.dim() != 1 or not maxit.is_cuda or (maxit.numel() > 1 and maxit.stride(0) != 1):
+            raise ValueError("maxit must be an integer >= 0 or a contiguous 1-D CUDA int32 tensor")
+    elif isinstance(maxit, bool) or not isinstance(maxit, (int, np.integer)) or maxit < 0 or maxit > 2**31 - 2:
         raise ValueError("maxit must be an integer >= 0")
+    if isinstance(dtol, bool) or not isinstance(dtol, (int, float)) or not (dtol == 0.0 or dtol >= 1.0):
+        raise ValueError("dtol must be 0 (off) or a number >= 1")
+
+
+def _check_lengths(count: int, what: str, *values):
+    for v, name in zip(values, ("atol", "rtol", "maxit")):
+        if _is_torch(v) and v.numel() != count:
+            raise ValueError("%s must hold one entry per %s: %d, not %d"
+                             % (name, "member" if what == "nbatch" else "problem", count, v.numel()))
+
+
+def _stop_test(atol, rtol, maxit, dtol, scale, ldscale) -> _lib.StopTest:
+    """The nka_stop_test of validated arguments.  Tensor entries are checked here (this synchronises): a
+    tolerance entry must be >= 0 (not NaN), a maxit entry in 0..2**31 - 2, whose maximum bounds the loop."""
+    stop = _lib.StopTest()
+    for v, name in ((atol, "atol"), (rtol, "rtol")):
+        if _is_torch(v):
+            if not bool((v >= 0.0).all()):
+                raise ValueError("%s entries must be >= 0 (and not NaN)" % name)
+            setattr(stop, name + "_dev", v.data_ptr())
+        else:
+            setattr(stop, name, float(v))
+    if _is_torch(maxit):
+        lo, hi = int(maxit.min()), int(maxit.max())
+        if lo < 0 or hi > 2**31 - 2:
+            raise ValueError("maxit entries must be integers in 0..2**31 - 2")
+        stop.maxit, stop.maxit_dev = hi, maxit.data_ptr()
+    else:
+        stop.maxit = int(maxit)
+    stop.dtol = float(dtol)
+    if scale is not None:
+        stop.scale_dev, stop.ldscale = scale.data_ptr(), ldscale
+    return stop
 
 
 def _capture(residual, device):
@@ -280,10 +337,11 @@ def _capture(residual, device):
 
 class FixedPointLoop:
     """A device-side fixed-point loop over a BatchNKA (BatchNKA.fixed_point_loop).  Keeps the captured
-    residual graph (and its memory pool), X, F and the batch alive."""
+    residual graph (and its memory pool), X, F, the stop test's tensors and the batch alive."""
 
     def __init__(self, batch: BatchNKA, graph, X, F, maxit: int):
         self._h = None
+        self._stop = None
         self._batch, self._graph, self._X, self._F = batch, graph, X, F
         self._lib = batch._lib
         self.maxit = maxit
@@ -302,7 +360,7 @@ class FixedPointLoop:
 
     def results(self):
         """(steps, status, norm) per member as numpy arrays; status is one of RUNNING, CONVERGED, MAXIT,
-        NONFINITE.  Synchronises."""
+        NONFINITE, DIVERGED.  Synchronises."""
         h = self._handle("results", "it copies the loop's results to the host and synchronises")
         nb = self._batch.nbatch
         it = np.zeros(nb, dtype=np.int32)
@@ -334,10 +392,11 @@ class FixedPointLoop:
 
 class FixedPointQueue:
     """A device-side work queue over a BatchNKA (BatchNKA.fixed_point_queue).  Keeps the captured residual
-    graph (and its memory pool), X, F, slot_problem, X0, Xout and the batch alive."""
+    graph (and its memory pool), X, F, slot_problem, X0, Xout, the stop test's tensors and the batch alive."""
 
     def __init__(self, batch: BatchNKA, graph, X, F, slot_problem, X0, Xout, nproblems: int):
         self._h = None
+        self._stop = None
         self._batch, self._graph, self._X, self._F = batch, graph, X, F
         self._slot_problem, self.X0, self.Xout = slot_problem, X0, Xout
         self._lib = batch._lib
@@ -357,7 +416,7 @@ class FixedPointQueue:
 
     def results(self):
         """(steps, status, norm) per problem as numpy arrays; status is one of RUNNING, CONVERGED, MAXIT,
-        NONFINITE.  Synchronises."""
+        NONFINITE, DIVERGED.  Synchronises."""
         h = self._handle("results", "it copies the queue's results to the host and synchronises")
         n = self.nproblems
         it = np.zeros(n, dtype=np.int32)
@@ -380,4 +439,4 @@ class FixedPointQueue:
             pass
 
 
-RUNNING, CONVERGED, MAXIT, NONFINITE = 0, 1, 2, 3
+RUNNING, CONVERGED, MAXIT, NONFINITE, DIVERGED = 0, 1, 2, 3, 4

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <functional>
 #include "nka_dispatch.h"
+#include "../../include/nka_b200.h"
 
 struct nka_batch {
   int nbatch = 0, mvec = 0;
@@ -39,11 +40,14 @@ int nka_loop_driver_refused(const char* call);
 // CTAs per member of the loop's check and step kernels at access width V (vlen only, as the batch's fix-up)
 int nka_loop_grid(nka_batch* bt, int V);
 // nka_loop_check<V> / nka_loop_step<V> queued on `s` over dim3(grid, nbatch) (nka_batch_loop.cu documents
-// them); check k of member b is recorded at hist[k * hstride + b]
+// them); check k of member b is recorded at hist[k * hstride + b].  check applies `stop` with the per-problem
+// entries of row b at index[b] (index NULL: at b).
 void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, const double* F, size_t ldf, size_t n,
                           int hstride, const int* iters, int* status, unsigned char* active, double* r0, double* rlast,
-                          double* hist, double* partials, size_t prow, unsigned* tickets, double atol, double rtol,
-                          int maxit);
+                          double* hist, double* partials, size_t prow, unsigned* tickets, const nka_stop_test& stop,
+                          const int* index);
+// Aborts (file:line, under `call`) unless `stop` is a valid nka_stop_test for members of length vlen.
+void nka_stop_test_require(const char* call, const nka_stop_test* stop, size_t vlen);
 void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
                          size_t n, int nbatch, const unsigned char* active, int* iters);
 // The graph  prologue -> WHILE (cond) { residual graph, cloned as a child -> body }, instantiated and

@@ -3,9 +3,9 @@
 //
 //   reset -> WHILE (any member running) { residual graph -> check -> decide -> batched update -> step }
 //
-// check reduces each running member's ||F_b||_2 with the batch's fixed-order grid reduction, records it
-// and decides the member's status; decide sets the WHILE node's condition; the update and step touch
-// only members still running.  A member's bits are those of a host-driven loop making the same calls:
+// check reduces each running member's ||F_b||_2 (or a scaled ||s_b . F_b||_2) with the batch's
+// fixed-order grid reduction, records it and decides the member's status by its stop test; decide sets
+// the WHILE node's condition; the update and step touch only members still running.  A member's bits are those of a host-driven loop making the same calls:
 //   - check's CTA count per member follows vlen only (nka_grid_for, as the batch's fix-up), and
 //     nka_grid_reduce folds its partial rows in a fixed order, so a norm depends on the row alone;
 //   - the update is nka_batch_accel_update's own launch sequence, with check's mask;
@@ -44,13 +44,16 @@ nka_loop_reset(int* __restrict__ iters, int* __restrict__ status, unsigned char*
   }
 }
 
-// ||F_b|| of every running member (blockIdx.y), recorded as check k = iters[b], and its status.
+// ||s_b . F_b|| of every running member (blockIdx.y), recorded as check k = iters[b], and its status by
+// member (or, with `index`, problem) p = index[b]'s rule in `stop` (include/nka_b200.h: nka_stop_test).
+// Without a scale the sweep is ||F_b||'s; with one, t = s_i * f_i enters the same fma in the same order
+// on the same CTAs, F at width V as without, the scale 16 bytes at a time when scale16 (V = 2 only).
 template <int V>
 __global__ void __launch_bounds__(NKA_THREADS)
 nka_loop_check(const double* __restrict__ F, size_t ldf, size_t n, int nbatch, const int* __restrict__ iters,
                int* __restrict__ status, unsigned char* __restrict__ active, double* __restrict__ r0,
                double* __restrict__ rlast, double* __restrict__ hist, double* __restrict__ partials_all, size_t prow,
-               unsigned* __restrict__ tickets, double atol, double rtol, int maxit)
+               unsigned* __restrict__ tickets, const nka_stop_test stop, const int* __restrict__ index, int scale16)
 {
   const size_t b = blockIdx.y;
   // every CTA of a member sees the same status: only the member's last CTA writes it, after all took tickets
@@ -60,11 +63,40 @@ nka_loop_check(const double* __restrict__ F, size_t ldf, size_t n, int nbatch, c
   const size_t nv = n / V;
   const size_t stride = (size_t)gridDim.x * NKA_THREADS;
   const size_t start = (size_t)blockIdx.x * NKA_THREADS + threadIdx.x;
-  for (size_t i = start; i < nv; i += stride) {
-    const Vec<V> x = Vec<V>::ld(f, i);
-    x.dot_into(x, acc[0]);
+  const double* sc = stop.scale_dev;
+  if (!sc) {
+    for (size_t i = start; i < nv; i += stride) {
+      const Vec<V> x = Vec<V>::ld(f, i);
+      x.dot_into(x, acc[0]);
+    }
+    if (V == 2 && (n & 1) && start == 0) acc[0] = fma(f[n - 1], f[n - 1], acc[0]);
+  } else {
+    sc += b * stop.ldscale;
+    if constexpr (V == 2) {
+      if (scale16) {
+        for (size_t i = start; i < nv; i += stride) {
+          const Vec<2> x = Vec<2>::ld(f, i), s = Vec<2>::ld(sc, i);
+          const Vec<2> t = {s.x * x.x, s.y * x.y};
+          t.dot_into(t, acc[0]);
+        }
+      } else {
+        for (size_t i = start; i < nv; i += stride) {
+          const Vec<2> x = Vec<2>::ld(f, i);
+          const Vec<2> t = {__ldg(sc + 2 * i) * x.x, __ldg(sc + 2 * i + 1) * x.y};
+          t.dot_into(t, acc[0]);
+        }
+      }
+    } else {
+      for (size_t i = start; i < nv; i += stride) {
+        const double t = __ldg(sc + i) * Vec<1>::ld(f, i).x;
+        acc[0] = fma(t, t, acc[0]);
+      }
+    }
+    if (V == 2 && (n & 1) && start == 0) {
+      const double t = __ldg(sc + n - 1) * f[n - 1];
+      acc[0] = fma(t, t, acc[0]);
+    }
   }
-  if (V == 2 && (n & 1) && start == 0) acc[0] = fma(f[n - 1], f[n - 1], acc[0]);
   __shared__ double ss;
   double* partials = partials_all + b * prow;
   const bool last = nka_grid_reduce<1, NKA_THREADS>(acc, partials, tickets + b, partials, gridDim.x,
@@ -75,9 +107,14 @@ nka_loop_check(const double* __restrict__ F, size_t ldf, size_t n, int nbatch, c
     hist[(size_t)k * nbatch + b] = r;
     rlast[b] = r;
     if (k == 0) r0[b] = r;
+    const size_t p = index ? (size_t)index[b] : b;
+    const double atol = stop.atol_dev ? stop.atol_dev[p] : stop.atol;
+    const double rtol = stop.rtol_dev ? stop.rtol_dev[p] : stop.rtol;
+    const int maxit = stop.maxit_dev ? min(max(stop.maxit_dev[p], 0), stop.maxit) : stop.maxit;
     int st = NKA_LOOP_RUNNING;
     if (!isfinite(r)) st = NKA_LOOP_NONFINITE;
     else if (r < fmax(atol, rtol * r0[b])) st = NKA_LOOP_CONVERGED;
+    else if (stop.dtol > 0.0 && r > stop.dtol * r0[b]) st = NKA_LOOP_DIVERGED;
     else if (k >= maxit) st = NKA_LOOP_MAXIT;
     status[b] = st;
     active[b] = st == NKA_LOOP_RUNNING;
@@ -156,17 +193,34 @@ int nka_loop_grid(NKABATCH bt, int V) { return nka_grid_for(bt->geom, 4, bt->vle
 
 void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, const double* F, size_t ldf, size_t n,
                           int hstride, const int* iters, int* status, unsigned char* active, double* r0, double* rlast,
-                          double* hist, double* partials, size_t prow, unsigned* tickets, double atol, double rtol,
-                          int maxit)
+                          double* hist, double* partials, size_t prow, unsigned* tickets, const nka_stop_test& stop,
+                          const int* index)
 {
   const dim3 g(grid, (unsigned)nbatch);
+  // the scale's load width follows its own rows' alignment; V and grid follow F's alone
+  const int scale16 = stop.scale_dev && (uintptr_t)stop.scale_dev % 16 == 0 && stop.ldscale % 2 == 0;
   if (V == 2)
     nka_loop_check<2><<<g, NKA_THREADS, 0, s>>>(F, ldf, n, hstride, iters, status, active, r0, rlast, hist, partials, prow,
-                                                tickets, atol, rtol, maxit);
+                                                tickets, stop, index, scale16);
   else
     nka_loop_check<1><<<g, NKA_THREADS, 0, s>>>(F, ldf, n, hstride, iters, status, active, r0, rlast, hist, partials, prow,
-                                                tickets, atol, rtol, maxit);
+                                                tickets, stop, index, scale16);
   CUDA_CHECK(cudaGetLastError());
+}
+
+void nka_stop_test_require(const char* call, const nka_stop_test* stop, size_t vlen)
+{
+  char msg[160];
+  const auto require = [&](bool ok, const char* what) {
+    if (ok) return;
+    snprintf(msg, sizeof msg, "%s: %s", call, what);
+    nka_fail(__FILE__, __LINE__, msg);
+  };
+  require(stop != NULL, "null stop test");
+  require(stop->atol >= 0.0 && stop->rtol >= 0.0, "atol and rtol must be >= 0");
+  require(stop->maxit >= 0, "maxit must be >= 0");
+  require(stop->dtol == 0.0 || stop->dtol >= 1.0, "dtol must be 0 (off) or >= 1");
+  require(!stop->scale_dev || stop->ldscale >= vlen, "ldscale must be >= vlen");
 }
 
 void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
@@ -249,12 +303,20 @@ cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t re
 extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
                                              size_t ldf, double atol, double rtol, int maxit)
 {
+  const nka_stop_test stop = {atol, rtol, 0.0, maxit, NULL, NULL, NULL, NULL, 0};
+  return nka_batch_loop_create_stop(bt, residual_graph, x, ldx, f, ldf, &stop);
+}
+
+extern "C" NKABATCHLOOP nka_batch_loop_create_stop(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
+                                                  size_t ldf, const nka_stop_test* stop_in)
+{
   NKA_REQUIRE(bt != NULL, "nka_batch_loop_create: null handle");
   NKA_REQUIRE(residual_graph != NULL, "nka_batch_loop_create: null residual graph");
   NKA_REQUIRE(x != NULL && f != NULL, "nka_batch_loop_create: null x or f");
   NKA_REQUIRE(ldx >= bt->vlen && ldf >= bt->vlen, "nka_batch_loop_create: ldx and ldf must be >= vlen");
-  NKA_REQUIRE(atol >= 0.0 && rtol >= 0.0, "nka_batch_loop_create: atol and rtol must be >= 0");
-  NKA_REQUIRE(maxit >= 0, "nka_batch_loop_create: maxit must be >= 0");
+  nka_stop_test_require("nka_batch_loop_create", stop_in, bt->vlen);
+  const nka_stop_test stop = *stop_in;
+  const int maxit = stop.maxit;
   DeviceGuard guard(bt->device);
   nka_refuse_capture(bt->stream, "nka_batch_loop_create", "it builds and uploads a graph and synchronises");
   if (nka_loop_driver_refused("nka_batch_loop_create")) return nullptr;
@@ -297,7 +359,7 @@ extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph,
   };
   auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
     nka_loop_queue_check(Vc, gc, bt->nbatch, cs, f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active, L->r0, L->rlast,
-                         L->hist, L->partials, prow, L->tickets, atol, rtol, maxit);
+                         L->hist, L->partials, prow, L->tickets, stop, /*index=*/nullptr);
     nka_loop_decide<<<1, 1024, 0, cs>>>(L->active, bt->nbatch, cond);
     CUDA_CHECK(cudaGetLastError());
     nka_batch_update_captured(bt, f, ldf, L->active, cs);

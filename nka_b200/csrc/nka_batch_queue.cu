@@ -5,7 +5,8 @@
 //   reset -> claim -> rows -> restart
 //   WHILE (any slot holds a problem) { residual graph -> check -> claim -> rows -> restart -> update -> step }
 //
-// check and step are the loop's kernels (nka_batch_loop.cu), unchanged.  claim (one CTA) retires every
+// check and step are the loop's kernels (nka_batch_loop.cu); check reads each slot's problem from
+// slot_problem for the per-problem parts of the stop test.  claim (one CTA) retires every
 // slot whose problem stopped, writing that problem's steps, status and norm, and hands the free slots
 // the next problem ids in slot order; rows copies a retired slot's X row out and a claimed problem's
 // initial guess in; restart restarts the claimed slots' accelerators.  A claimed slot is not checked
@@ -197,6 +198,16 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create(NKABATCH bt, void* residual_grap
                                                double* xout, size_t ldxout, size_t nproblems, double atol, double rtol,
                                                int maxit)
 {
+  const nka_stop_test stop = {atol, rtol, 0.0, maxit, NULL, NULL, NULL, NULL, 0};
+  return nka_batch_queue_create_stop(bt, residual_graph, x, ldx, f, ldf, slot_problem, x0, ldx0, xout, ldxout, nproblems,
+                                     &stop);
+}
+
+extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
+                                                    size_t ldf, int* slot_problem, const double* x0, size_t ldx0,
+                                                    double* xout, size_t ldxout, size_t nproblems,
+                                                    const nka_stop_test* stop_in)
+{
   NKA_REQUIRE(bt != NULL, "nka_batch_queue_create: null handle");
   NKA_REQUIRE(residual_graph != NULL, "nka_batch_queue_create: null residual graph");
   NKA_REQUIRE(x != NULL && f != NULL && slot_problem != NULL && x0 != NULL && xout != NULL,
@@ -204,8 +215,8 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create(NKABATCH bt, void* residual_grap
   NKA_REQUIRE(ldx >= bt->vlen && ldf >= bt->vlen && ldx0 >= bt->vlen && ldxout >= bt->vlen,
               "nka_batch_queue_create: ldx, ldf, ldx0 and ldxout must be >= vlen");
   NKA_REQUIRE(nproblems >= 1 && nproblems <= (size_t)INT_MAX, "nka_batch_queue_create: nproblems must be in 1..INT_MAX");
-  NKA_REQUIRE(atol >= 0.0 && rtol >= 0.0, "nka_batch_queue_create: atol and rtol must be >= 0");
-  NKA_REQUIRE(maxit >= 0, "nka_batch_queue_create: maxit must be >= 0");
+  nka_stop_test_require("nka_batch_queue_create", stop_in, bt->vlen);
+  const nka_stop_test stop = *stop_in;
   DeviceGuard guard(bt->device);
   nka_refuse_capture(bt->stream, "nka_batch_queue_create", "it builds and uploads a graph and synchronises");
   if (nka_loop_driver_refused("nka_batch_queue_create")) return nullptr;
@@ -274,9 +285,10 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create(NKABATCH bt, void* residual_grap
     claim_rows_restart(cs, cond);
   };
   auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
-    // check's history stride is 0: every check of slot b writes hist[b], which nothing reads
+    // check's history stride is 0: every check of slot b writes hist[b], which nothing reads.  It runs after
+    // the residual and before claim, so slot_problem[b] is still the problem whose F it checks.
     nka_loop_queue_check(Vc, gc, bt->nbatch, cs, f, ldf, bt->vlen, /*hstride=*/0, Q->iters, Q->status, Q->active, Q->r0, Q->rlast,
-                         Q->hist, Q->partials, prow, Q->tickets, atol, rtol, maxit);
+                         Q->hist, Q->partials, prow, Q->tickets, stop, /*index=*/slot_problem);
     claim_rows_restart(cs, cond);
     nka_batch_update_captured(bt, f, ldf, Q->active, cs);
     nka_loop_queue_step(Vs, gs, cs, x, ldx, f, ldf, bt->vlen, bt->nbatch, Q->active, Q->iters);

@@ -16,6 +16,16 @@ module nka_b200_c
   implicit none
   public
 
+  !! include/nka_b200.h: nka_stop_test, the stopping rule of nka_batch_loop_create_stop and
+  !! nka_batch_queue_create_stop.  The *_dev components are device addresses (c_null_ptr: the scalar
+  !! applies; scale_dev c_null_ptr: no scale).  Declare it with the target attribute and pass c_loc of it.
+  type, bind(C) :: nka_stop_test
+    real(c_double) :: atol, rtol, dtol
+    integer(c_int) :: maxit
+    type(c_ptr) :: atol_dev, rtol_dev, maxit_dev, scale_dev
+    integer(c_size_t) :: ldscale
+  end type nka_stop_test
+
   interface
 
     !! NKA nka_init_ex (size_t vlen, int mvec, double vtol, int device, void *stream)
@@ -436,6 +446,45 @@ module nka_b200_c
       import :: c_ptr
       type(c_ptr), value :: handle
     end subroutine
+
+    !! ---- per-problem stopping tests (include/nka_b200.h): the creates above with an nka_stop_test
+
+    !! NKABATCHLOOP nka_batch_loop_create_stop (NKABATCH, void *residual_graph, double *x_dev, size_t ldx,
+    !!                                          double *f_dev, size_t ldf, const nka_stop_test *stop)
+    !! stop: c_loc of a type(nka_stop_test), target.  c_null_ptr if CUDA refuses the graph.
+    function nka_batch_loop_create_stop(batch, residual_graph, x_dev, ldx, f_dev, ldf, stop) &
+        bind(C, name='nka_batch_loop_create_stop') result(handle)
+      import :: c_ptr, c_double, c_size_t
+      type(c_ptr), value :: batch, residual_graph
+      real(c_double), intent(inout) :: x_dev(*)
+      integer(c_size_t), value :: ldx
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      type(c_ptr), value :: stop
+      type(c_ptr) :: handle
+    end function
+
+    !! NKABATCHQUEUE nka_batch_queue_create_stop (NKABATCH, void *residual_graph, double *x_dev, size_t ldx,
+    !!     double *f_dev, size_t ldf, int *slot_problem_dev, const double *x0_dev, size_t ldx0,
+    !!     double *xout_dev, size_t ldxout, size_t nproblems, const nka_stop_test *stop)
+    !! stop: c_loc of a type(nka_stop_test), target; its arrays hold one entry per problem.
+    function nka_batch_queue_create_stop(batch, residual_graph, x_dev, ldx, f_dev, ldf, slot_problem_dev, x0_dev, ldx0, &
+                                         xout_dev, ldxout, nproblems, stop) &
+        bind(C, name='nka_batch_queue_create_stop') result(handle)
+      import :: c_ptr, c_double, c_size_t
+      type(c_ptr), value :: batch, residual_graph
+      real(c_double), intent(inout) :: x_dev(*)
+      integer(c_size_t), value :: ldx
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      type(c_ptr), value :: slot_problem_dev
+      real(c_double), intent(in) :: x0_dev(*)
+      integer(c_size_t), value :: ldx0
+      real(c_double), intent(inout) :: xout_dev(*)
+      integer(c_size_t), value :: ldxout, nproblems
+      type(c_ptr), value :: stop
+      type(c_ptr) :: handle
+    end function
 
   end interface
 
