@@ -333,6 +333,50 @@ struct nka_batch_queue *nka_batch_queue_create_stop (struct nka_batch *b, void *
                                                      double *xout_dev, size_t ldxout, size_t nproblems,
                                                      const nka_stop_test *stop);
 
+/* ---- residual-growth restarts in device-side loops and queues ----------- */
+/* The _restart creates are the _stop creates with one more rule,
+ * restart_growth = gamma (0: off; else finite and > 0).  For member b of a
+ * loop, or the problem in slot b of a queue: when check k >= 1 leaves it
+ * RUNNING and r_k > gamma * r_{k-1} (the norms that check recorded: scaled when
+ * the stop test has a scale), its accelerator is restarted before this
+ * iteration's update, as nka_batch_restart with only b in the mask does.  That
+ * update then returns F_b unchanged and starts a new subspace from it, and
+ * X_b += F_b is a plain step.  gamma >= 1 restarts on growth, gamma < 1 when
+ * the decrease is too small.  A member that check stops (DIVERGED included) is
+ * never restarted; r0, the stop test and the step are unchanged; a loop launch
+ * still does not restart members at its start.  r_{k-1} is always the same
+ * launch's (loop) or the same problem's (queue), never a slot's previous
+ * problem's.
+ *
+ * Each member's bits are those of a host-driven loop that, after each
+ * residual, calls nka_batch_restart with the members the rule picks, then the
+ * masked accel_update and X_b += F_b; each queue problem's are those of the
+ * loop with the same gamma on a just-restarted member, whatever its slot.  A
+ * rule that never fires gives the _stop creates' bits.  Memory: per slot one
+ * double, one int and one byte; in a queue 4 bytes per problem more.
+ *
+ * create aborts (file:line) when restart_growth is negative or not finite, as
+ * it does on a bad stop test.  The _stop creates are these with gamma = 0,
+ * which build exactly the graphs they built before.
+ *
+ * _restarts copy the restarts the rule made: per member in the last launch
+ * (loop, nbatch ints), or per problem (queue, nproblems ints; the restart a
+ * queue makes when a slot takes a problem is not counted).  Zeros when
+ * restart_growth was 0.  They synchronise and abort while the batch's stream
+ * captures. */
+struct nka_batch_loop *nka_batch_loop_create_restart (struct nka_batch *b, void *residual_graph /* cudaGraph_t */,
+                                                      double *x_dev, size_t ldx, double *f_dev, size_t ldf,
+                                                      const nka_stop_test *stop, double restart_growth);
+struct nka_batch_queue *nka_batch_queue_create_restart (struct nka_batch *b, void *residual_graph /* cudaGraph_t */,
+                                                        double *x_dev, size_t ldx, double *f_dev, size_t ldf,
+                                                        int *slot_problem_dev, const double *x0_dev, size_t ldx0,
+                                                        double *xout_dev, size_t ldxout, size_t nproblems,
+                                                        const nka_stop_test *stop, double restart_growth);
+/* nbatch ints on the host; synchronises */
+void nka_batch_loop_restarts (struct nka_batch_loop *L, int *restarts);
+/* nproblems ints on the host; synchronises */
+void nka_batch_queue_restarts (struct nka_batch_queue *Q, int *restarts);
+
 #ifdef __cplusplus
 }
 #endif

@@ -124,6 +124,14 @@ SYMBOLS = {
     "nka_batch_queue_create_stop": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
                                                  C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t,
                                                  C.POINTER(StopTest)]),
+    # include/nka_b200.h: residual-growth restarts
+    "nka_batch_loop_create_restart": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                                   C.POINTER(StopTest), C.c_double]),
+    "nka_batch_queue_create_restart": (C.c_void_p, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t,
+                                                    C.POINTER(StopTest), C.c_double]),
+    "nka_batch_loop_restarts": (None, [C.c_void_p, C.POINTER(C.c_int)]),
+    "nka_batch_queue_restarts": (None, [C.c_void_p, C.POINTER(C.c_int)]),
     # include/nka_example.h
     "nka_system_init": (C.c_void_p, [C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),
     "nka_system_init_slab": (C.c_void_p, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),

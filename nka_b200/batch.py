@@ -170,7 +170,7 @@ class BatchNKA:
 
     # -- device-side fixed-point loops --------------------------------------
     def fixed_point_loop(self, residual, X, F, atol=0.0, rtol=1e-8, maxit=100, dtol: float = 0.0,
-                         scale=None) -> "FixedPointLoop":
+                         scale=None, restart_growth: float = 0.0) -> "FixedPointLoop":
         """A solve of x_b = G(x_b) for every member that runs to its end in one graph launch
         (INTEGRATION.md section 8).  residual: a zero-argument callable writing F = G(X) - X in place with
         torch ops; it is run once to warm up, then captured.  X, F: CUDA float64 tensors [nbatch, vlen]
@@ -181,8 +181,11 @@ class BatchNKA:
         or a contiguous CUDA int32 tensor of nbatch entries (the loop's history then has max(maxit) + 1
         rows); dtol: 0 (off) or >= 1; scale: None or a CUDA float64 tensor [nbatch, vlen] with unit column
         stride, read after the residual in every iteration, so the residual may rewrite it
-        (INTEGRATION.md section 9a)."""
+        (INTEGRATION.md section 9a).  restart_growth: 0 (off) or a finite number > 0; when check k >= 1
+        leaves a member running with r_k > restart_growth * r_{k-1}, its accelerator is restarted before
+        that iteration's update (INTEGRATION.md section 9b)."""
         _check_stopping(atol, rtol, maxit, dtol)
+        _check_restart_growth(restart_growth)
         _check_lengths(self.nbatch, "nbatch", atol, rtol, maxit)
         ldscale = self._rows(scale, "scale") if scale is not None else 0
         ldx = self._rows(X, "X")
@@ -192,8 +195,8 @@ class BatchNKA:
         graph = _capture(residual, F.device)
         loop = FixedPointLoop(self, graph, X, F, stop.maxit)
         loop._stop = (atol, rtol, maxit, scale)
-        loop._h = self._lib.nka_batch_loop_create_stop(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
-                                                       C.byref(stop))
+        loop._h = self._lib.nka_batch_loop_create_restart(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(),
+                                                          ldf, C.byref(stop), float(restart_growth))
         if not loop._h:
             raise NKAError("nka_batch_loop_create returned NULL: CUDA refused the residual graph or the driver "
                            "has no conditional graph nodes (the reason is printed on stderr)")
@@ -219,7 +222,7 @@ class BatchNKA:
         return ld
 
     def fixed_point_queue(self, residual, X, F, slot_problem, X0, Xout=None, atol=0.0, rtol=1e-8,
-                          maxit=100, dtol: float = 0.0, scale=None) -> "FixedPointQueue":
+                          maxit=100, dtol: float = 0.0, scale=None, restart_growth: float = 0.0) -> "FixedPointQueue":
         """Solve nproblems = X0.shape[0] problems x_p = G_p(x_p) on the members as slots, in one graph launch
         (INTEGRATION.md section 9).  When a slot's problem stops, the launch writes its final iterate to
         Xout[p], loads the next problem's X0 row into the slot and restarts the slot's accelerator.
@@ -230,8 +233,10 @@ class BatchNKA:
         (slot b solves problem b) and kept by the queue.  X0, Xout: CUDA float64 [nproblems, vlen] with unit
         column stride; Xout=None solves in place (Xout is X0).  The stopping rule is fixed_point_loop's,
         with tensor atol, rtol and maxit holding one entry per problem (nproblems), found through
-        slot_problem; scale is per slot, [nbatch, vlen], like F."""
+        slot_problem; scale is per slot, [nbatch, vlen], like F.  restart_growth is fixed_point_loop's,
+        applied to each problem's own norms (INTEGRATION.md section 9b)."""
         _check_stopping(atol, rtol, maxit, dtol)
+        _check_restart_growth(restart_growth)
         sp_bad = "slot_problem must be a contiguous CUDA int32 tensor of length nbatch = %d" % self.nbatch
         if not _is_torch(slot_problem):
             raise ValueError(sp_bad)
@@ -260,9 +265,10 @@ class BatchNKA:
         graph = _capture(residual, F.device)
         queue = FixedPointQueue(self, graph, X, F, slot_problem, X0, Xout, nproblems)
         queue._stop = (atol, rtol, maxit, scale)
-        queue._h = self._lib.nka_batch_queue_create_stop(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(), ldf,
-                                                         slot_problem.data_ptr(), X0.data_ptr(), ldx0, Xout.data_ptr(),
-                                                         ldxout, nproblems, C.byref(stop))
+        queue._h = self._lib.nka_batch_queue_create_restart(h, graph.raw_cuda_graph(), X.data_ptr(), ldx, F.data_ptr(),
+                                                            ldf, slot_problem.data_ptr(), X0.data_ptr(), ldx0,
+                                                            Xout.data_ptr(), ldxout, nproblems, C.byref(stop),
+                                                            float(restart_growth))
         if not queue._h:
             raise NKAError("nka_batch_queue_create returned NULL: CUDA refused the residual graph or the driver "
                            "has no conditional graph nodes (the reason is printed on stderr)")
@@ -287,6 +293,12 @@ def _check_stopping(atol, rtol, maxit, dtol):
         raise ValueError("maxit must be an integer >= 0")
     if isinstance(dtol, bool) or not isinstance(dtol, (int, float)) or not (dtol == 0.0 or dtol >= 1.0):
         raise ValueError("dtol must be 0 (off) or a number >= 1")
+
+
+def _check_restart_growth(restart_growth):
+    if isinstance(restart_growth, bool) or not isinstance(restart_growth, (int, float, np.integer, np.floating)) \
+            or not 0.0 <= restart_growth < float("inf"):
+        raise ValueError("restart_growth must be 0 (off) or a finite number > 0")
 
 
 def _check_lengths(count: int, what: str, *values):
@@ -370,6 +382,14 @@ class FixedPointLoop:
                                          norm.ctypes.data_as(C.POINTER(C.c_double)))
         return it, st, norm
 
+    def restarts(self) -> np.ndarray:
+        """Restarts the residual-growth rule made per member in the last launch (int32; zeros when
+        restart_growth is 0).  Synchronises."""
+        h = self._handle("restarts", "it copies the loop's restart counts to the host and synchronises")
+        out = np.zeros(self._batch.nbatch, dtype=np.int32)
+        self._lib.nka_batch_loop_restarts(h, out.ctypes.data_as(C.POINTER(C.c_int)))
+        return out
+
     def history(self) -> np.ndarray:
         """[(maxit+1), nbatch]: row k holds each member's norm at check k, NaN where it made none.  Synchronises."""
         h = self._handle("history", "it copies the loop's history to the host and synchronises")
@@ -425,6 +445,14 @@ class FixedPointQueue:
         self._lib.nka_batch_queue_results(h, it.ctypes.data_as(C.POINTER(C.c_int)), st.ctypes.data_as(C.POINTER(C.c_int)),
                                           norm.ctypes.data_as(C.POINTER(C.c_double)))
         return it, st, norm
+
+    def restarts(self) -> np.ndarray:
+        """Restarts the residual-growth rule made per problem in the last launch (int32; the restart of a slot
+        taking a problem is not counted; zeros when restart_growth is 0).  Synchronises."""
+        h = self._handle("restarts", "it copies the queue's restart counts to the host and synchronises")
+        out = np.zeros(self.nproblems, dtype=np.int32)
+        self._lib.nka_batch_queue_restarts(h, out.ctypes.data_as(C.POINTER(C.c_int)))
+        return out
 
     def destroy(self) -> None:
         if self._h:

@@ -50,6 +50,14 @@ void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, cons
 void nka_stop_test_require(const char* call, const nka_stop_test* stop, size_t vlen);
 void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
                          size_t n, int nbatch, const unsigned char* active, int* iters);
+// The residual-growth restart (nka_batch_guard.cu): the prologue's reset of the restart counts nrst (nbatch)
+// and, in a queue, p_restarts (nproblems; NULL and 0 in a loop); and the body's guard followed by the
+// batch's restart of its mask rmask, queued on the capturing `s`.  claimed, move_out and p_restarts are
+// the queue's (NULL in a loop).
+void nka_loop_guard_reset_launch(cudaStream_t s, int* nrst, int nbatch, int* p_restarts, size_t nproblems);
+void nka_loop_guard_restart(nka_batch* bt, cudaStream_t s, double gamma, const unsigned char* active, const int* iters,
+                            const double* rlast, const unsigned char* claimed, const int* move_out, double* rprev,
+                            int* nrst, int* p_restarts, unsigned char* rmask);
 // The graph  prologue -> WHILE (cond) { residual graph, cloned as a child -> body }, instantiated and
 // uploaded on `s`.  prologue and body queue their kernels on `s` while it captures.  A graph CUDA
 // refuses gives nullptr, after printing CUDA's reason under `call`, with no error left behind.

@@ -14,6 +14,7 @@
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <string.h>
 
 #include <algorithm>
 #include <vector>
@@ -164,13 +165,17 @@ struct nka_batch_loop {
   double* hist = nullptr;                 // device, (maxit+1) x nbatch
   double* partials = nullptr;             // device, nbatch x prow
   unsigned* tickets = nullptr;            // device, nbatch
+  double* rprev = nullptr;                // device, nbatch: the previous check's norm (restart_growth > 0 only)
+  int* nrst = nullptr;                    // device, nbatch: restarts in this launch (restart_growth > 0 only)
+  unsigned char* rmask = nullptr;         // device, nbatch: the guard's restart mask (restart_growth > 0 only)
 };
 
 static void loop_free(NKABATCHLOOP L)
 {
   if (L->exec) cudaGraphExecDestroy(L->exec);
   cudaFree(L->iters); cudaFree(L->status); cudaFree(L->active); cudaFree(L->r0); cudaFree(L->rlast);
-  cudaFree(L->hist); cudaFree(L->partials); cudaFree(L->tickets);
+  cudaFree(L->hist); cudaFree(L->partials); cudaFree(L->tickets); cudaFree(L->rprev); cudaFree(L->nrst);
+  cudaFree(L->rmask);
   delete L;
 }
 
@@ -310,12 +315,22 @@ extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph,
 extern "C" NKABATCHLOOP nka_batch_loop_create_stop(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
                                                   size_t ldf, const nka_stop_test* stop_in)
 {
+  return nka_batch_loop_create_restart(bt, residual_graph, x, ldx, f, ldf, stop_in, 0.0);
+}
+
+extern "C" NKABATCHLOOP nka_batch_loop_create_restart(NKABATCH bt, void* residual_graph, double* x, size_t ldx,
+                                                     double* f, size_t ldf, const nka_stop_test* stop_in,
+                                                     double restart_growth)
+{
   NKA_REQUIRE(bt != NULL, "nka_batch_loop_create: null handle");
   NKA_REQUIRE(residual_graph != NULL, "nka_batch_loop_create: null residual graph");
   NKA_REQUIRE(x != NULL && f != NULL, "nka_batch_loop_create: null x or f");
   NKA_REQUIRE(ldx >= bt->vlen && ldf >= bt->vlen, "nka_batch_loop_create: ldx and ldf must be >= vlen");
   nka_stop_test_require("nka_batch_loop_create", stop_in, bt->vlen);
+  NKA_REQUIRE(restart_growth >= 0.0 && isfinite(restart_growth),
+              "nka_batch_loop_create: restart_growth must be 0 (off) or a finite number > 0");
   const nka_stop_test stop = *stop_in;
+  const bool guarded = restart_growth > 0.0;
   const int maxit = stop.maxit;
   DeviceGuard guard(bt->device);
   nka_refuse_capture(bt->stream, "nka_batch_loop_create", "it builds and uploads a graph and synchronises");
@@ -339,6 +354,11 @@ extern "C" NKABATCHLOOP nka_batch_loop_create_stop(NKABATCH bt, void* residual_g
   CUDA_CHECK(cudaMalloc(&L->hist, nhist * sizeof(double)));
   CUDA_CHECK(cudaMalloc(&L->partials, nb * prow * sizeof(double)));
   CUDA_CHECK(cudaMalloc(&L->tickets, nb * sizeof(unsigned)));
+  if (guarded) {
+    CUDA_CHECK(cudaMalloc(&L->rprev, nb * sizeof(double)));
+    CUDA_CHECK(cudaMalloc(&L->nrst, nb * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&L->rmask, nb));
+  }
 
   cudaStream_t s = nullptr;               // private: the batch's own stream may be the legacy default
   CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
@@ -346,22 +366,28 @@ extern "C" NKABATCHLOOP nka_batch_loop_create_stop(NKABATCH bt, void* residual_g
   if (bt->poison) {
     CUDA_CHECK(cudaMemsetAsync(L->partials, 0xFF, nb * prow * sizeof(double), s));
     CUDA_CHECK(cudaMemsetAsync(L->r0, 0xFF, nb * sizeof(double), s));
+    if (guarded) CUDA_CHECK(cudaMemsetAsync(L->rprev, 0xFF, nb * sizeof(double), s));
   }
   const unsigned greset = (unsigned)((nhist + NKA_THREADS - 1) / NKA_THREADS < 1024 ? (nhist + NKA_THREADS - 1) / NKA_THREADS : 1024);
   // before any launch: every member RUNNING at 0 steps, as the results of a loop never launched read
   nka_loop_reset<<<greset, NKA_THREADS, 0, s>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
   CUDA_CHECK(cudaGetLastError());
+  if (guarded) nka_loop_guard_reset_launch(s, L->nrst, bt->nbatch, nullptr, 0);
 
-  // reset, then the WHILE node: { residual, check, decide, update, step }
+  // reset [, guard reset], then the WHILE node: { residual, check, decide, [guard, restart,] update, step }
   auto prologue = [&](cudaStream_t cs, cudaGraphConditionalHandle) {
     nka_loop_reset<<<greset, NKA_THREADS, 0, cs>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
     CUDA_CHECK(cudaGetLastError());
+    if (guarded) nka_loop_guard_reset_launch(cs, L->nrst, bt->nbatch, nullptr, 0);
   };
   auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
     nka_loop_queue_check(Vc, gc, bt->nbatch, cs, f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active, L->r0, L->rlast,
                          L->hist, L->partials, prow, L->tickets, stop, /*index=*/nullptr);
     nka_loop_decide<<<1, 1024, 0, cs>>>(L->active, bt->nbatch, cond);
     CUDA_CHECK(cudaGetLastError());
+    if (guarded)
+      nka_loop_guard_restart(bt, cs, restart_growth, L->active, L->iters, L->rlast, nullptr, nullptr, L->rprev, L->nrst,
+                             nullptr, L->rmask);
     nka_batch_update_captured(bt, f, ldf, L->active, cs);
     nka_loop_queue_step(Vs, gs, cs, x, ldx, f, ldf, bt->vlen, bt->nbatch, L->active, L->iters);
   };
@@ -406,6 +432,21 @@ extern "C" void nka_batch_loop_history(NKABATCHLOOP L, double* norms)
   nka_refuse_capture(bt->stream, "nka_batch_loop_history", "it copies the loop's history to the host and synchronises");
   const size_t bytes = (size_t)(L->maxit + 1) * (size_t)bt->nbatch * sizeof(double);
   CUDA_CHECK(cudaMemcpyAsync(norms, L->hist, bytes, cudaMemcpyDeviceToHost, bt->stream));
+  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+}
+
+extern "C" void nka_batch_loop_restarts(NKABATCHLOOP L, int* restarts)
+{
+  NKA_REQUIRE(L != NULL && restarts != NULL, "nka_batch_loop_restarts: null argument");
+  NKABATCH bt = L->bt;
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, "nka_batch_loop_restarts", "it copies the loop's restart counts to the host and synchronises");
+  const size_t nb = (size_t)bt->nbatch;
+  if (!L->nrst) {
+    memset(restarts, 0, nb * sizeof(int));
+    return;
+  }
+  CUDA_CHECK(cudaMemcpyAsync(restarts, L->nrst, nb * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
   CUDA_CHECK(cudaStreamSynchronize(bt->stream));
 }
 

@@ -16,7 +16,9 @@
 #include <cuda_runtime.h>
 #include <limits.h>
 #include <stdint.h>
+#include <math.h>
 #include <stdio.h>
+#include <string.h>
 
 #include "../../include/nka_b200.h"
 #include "nka_internal.h"
@@ -180,6 +182,10 @@ struct nka_batch_queue {
   int* p_iters = nullptr;                 // device, nproblems
   int* p_status = nullptr;                // device, nproblems
   double* p_norm = nullptr;               // device, nproblems
+  double* rprev = nullptr;                // device, nbatch: the previous check's norm (restart_growth > 0 only)
+  int* nrst = nullptr;                    // device, nbatch: the slot's problem's restarts (restart_growth > 0 only)
+  unsigned char* rmask = nullptr;         // device, nbatch: claimed | the rule (restart_growth > 0 only)
+  int* p_restarts = nullptr;              // device, nproblems (restart_growth > 0 only)
 };
 
 static void queue_free(NKABATCHQUEUE Q)
@@ -188,6 +194,7 @@ static void queue_free(NKABATCHQUEUE Q)
   cudaFree(Q->iters); cudaFree(Q->status); cudaFree(Q->active); cudaFree(Q->claimed); cudaFree(Q->r0);
   cudaFree(Q->rlast); cudaFree(Q->hist); cudaFree(Q->partials); cudaFree(Q->tickets); cudaFree(Q->move_out);
   cudaFree(Q->move_in); cudaFree(Q->next); cudaFree(Q->p_iters); cudaFree(Q->p_status); cudaFree(Q->p_norm);
+  cudaFree(Q->rprev); cudaFree(Q->nrst); cudaFree(Q->rmask); cudaFree(Q->p_restarts);
   delete Q;
 }
 
@@ -208,6 +215,15 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual
                                                     double* xout, size_t ldxout, size_t nproblems,
                                                     const nka_stop_test* stop_in)
 {
+  return nka_batch_queue_create_restart(bt, residual_graph, x, ldx, f, ldf, slot_problem, x0, ldx0, xout, ldxout,
+                                        nproblems, stop_in, 0.0);
+}
+
+extern "C" NKABATCHQUEUE nka_batch_queue_create_restart(NKABATCH bt, void* residual_graph, double* x, size_t ldx,
+                                                       double* f, size_t ldf, int* slot_problem, const double* x0,
+                                                       size_t ldx0, double* xout, size_t ldxout, size_t nproblems,
+                                                       const nka_stop_test* stop_in, double restart_growth)
+{
   NKA_REQUIRE(bt != NULL, "nka_batch_queue_create: null handle");
   NKA_REQUIRE(residual_graph != NULL, "nka_batch_queue_create: null residual graph");
   NKA_REQUIRE(x != NULL && f != NULL && slot_problem != NULL && x0 != NULL && xout != NULL,
@@ -216,7 +232,10 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual
               "nka_batch_queue_create: ldx, ldf, ldx0 and ldxout must be >= vlen");
   NKA_REQUIRE(nproblems >= 1 && nproblems <= (size_t)INT_MAX, "nka_batch_queue_create: nproblems must be in 1..INT_MAX");
   nka_stop_test_require("nka_batch_queue_create", stop_in, bt->vlen);
+  NKA_REQUIRE(restart_growth >= 0.0 && isfinite(restart_growth),
+              "nka_batch_queue_create: restart_growth must be 0 (off) or a finite number > 0");
   const nka_stop_test stop = *stop_in;
+  const bool guarded = restart_growth > 0.0;
   DeviceGuard guard(bt->device);
   nka_refuse_capture(bt->stream, "nka_batch_queue_create", "it builds and uploads a graph and synchronises");
   if (nka_loop_driver_refused("nka_batch_queue_create")) return nullptr;
@@ -246,6 +265,12 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual
   CUDA_CHECK(cudaMalloc(&Q->p_iters, nproblems * sizeof(int)));
   CUDA_CHECK(cudaMalloc(&Q->p_status, nproblems * sizeof(int)));
   CUDA_CHECK(cudaMalloc(&Q->p_norm, nproblems * sizeof(double)));
+  if (guarded) {
+    CUDA_CHECK(cudaMalloc(&Q->rprev, nb * sizeof(double)));
+    CUDA_CHECK(cudaMalloc(&Q->nrst, nb * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&Q->rmask, nb));
+    CUDA_CHECK(cudaMalloc(&Q->p_restarts, nproblems * sizeof(int)));
+  }
 
   cudaStream_t s = nullptr;               // private: the batch's own stream may be the legacy default
   CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
@@ -255,6 +280,7 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual
     CUDA_CHECK(cudaMemsetAsync(Q->r0, 0xFF, nb * sizeof(double), s));
     CUDA_CHECK(cudaMemsetAsync(Q->rlast, 0xFF, nb * sizeof(double), s));
     CUDA_CHECK(cudaMemsetAsync(Q->hist, 0xFF, nb * sizeof(double), s));
+    if (guarded) CUDA_CHECK(cudaMemsetAsync(Q->rprev, 0xFF, nb * sizeof(double), s));
   }
   const size_t nreset = nproblems > nb ? nproblems : nb;
   const unsigned greset = (unsigned)((nreset + NKA_THREADS - 1) / NKA_THREADS < 1024 ? (nreset + NKA_THREADS - 1) / NKA_THREADS : 1024);
@@ -265,6 +291,7 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual
   };
   // before any launch: every problem RUNNING at 0 steps (slot_problem is the caller's until a launch)
   reset(s, 0);
+  if (guarded) nka_loop_guard_reset_launch(s, Q->nrst, bt->nbatch, Q->p_restarts, nproblems);
 
   const dim3 grows(gr, (unsigned)nb);
   auto claim_rows_restart = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
@@ -277,11 +304,17 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_stop(NKABATCH bt, void* residual
     else
       nka_queue_rows<1><<<grows, NKA_THREADS, 0, cs>>>(x, ldx, x0, ldx0, xout, ldxout, bt->vlen, Q->move_out, Q->move_in);
     CUDA_CHECK(cudaGetLastError());
-    nka_batch_restart_captured(bt, Q->claimed, cs);
+    if (guarded)    // restart the claimed slots and the running ones the rule picks: rmask = claimed | rule
+      nka_loop_guard_restart(bt, cs, restart_growth, Q->active, Q->iters, Q->rlast, Q->claimed, Q->move_out, Q->rprev,
+                             Q->nrst, Q->p_restarts, Q->rmask);
+    else
+      nka_batch_restart_captured(bt, Q->claimed, cs);
   };
-  // reset, claim, rows, restart; then the WHILE node: { residual, check, claim, rows, restart, update, step }
+  // reset [, guard reset], claim, rows, [guard,] restart; then the WHILE node:
+  //   { residual, check, claim, rows, [guard,] restart, update, step }
   auto prologue = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
     reset(cs, bt->nbatch);
+    if (guarded) nka_loop_guard_reset_launch(cs, Q->nrst, bt->nbatch, Q->p_restarts, nproblems);
     claim_rows_restart(cs, cond);
   };
   auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
@@ -323,6 +356,21 @@ extern "C" void nka_batch_queue_results(NKABATCHQUEUE Q, int* iters, int* status
   CUDA_CHECK(cudaMemcpyAsync(iters, Q->p_iters, np * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
   CUDA_CHECK(cudaMemcpyAsync(status, Q->p_status, np * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
   CUDA_CHECK(cudaMemcpyAsync(norm, Q->p_norm, np * sizeof(double), cudaMemcpyDeviceToHost, bt->stream));
+  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+}
+
+extern "C" void nka_batch_queue_restarts(NKABATCHQUEUE Q, int* restarts)
+{
+  NKA_REQUIRE(Q != NULL && restarts != NULL, "nka_batch_queue_restarts: null argument");
+  NKABATCH bt = Q->bt;
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, "nka_batch_queue_restarts", "it copies the queue's restart counts to the host and synchronises");
+  const size_t np = Q->nproblems;
+  if (!Q->p_restarts) {
+    memset(restarts, 0, np * sizeof(int));
+    return;
+  }
+  CUDA_CHECK(cudaMemcpyAsync(restarts, Q->p_restarts, np * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
   CUDA_CHECK(cudaStreamSynchronize(bt->stream));
 }
 

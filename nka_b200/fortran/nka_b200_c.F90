@@ -486,6 +486,58 @@ module nka_b200_c
       type(c_ptr) :: handle
     end function
 
+    !! ---- residual-growth restarts (include/nka_b200.h): the _stop creates with restart_growth
+
+    !! NKABATCHLOOP nka_batch_loop_create_restart (NKABATCH, void *residual_graph, double *x_dev, size_t ldx,
+    !!     double *f_dev, size_t ldf, const nka_stop_test *stop, double restart_growth)
+    !! restart_growth: 0 (off) or finite and > 0.  c_null_ptr if CUDA refuses the graph.
+    function nka_batch_loop_create_restart(batch, residual_graph, x_dev, ldx, f_dev, ldf, stop, restart_growth) &
+        bind(C, name='nka_batch_loop_create_restart') result(handle)
+      import :: c_ptr, c_double, c_size_t
+      type(c_ptr), value :: batch, residual_graph
+      real(c_double), intent(inout) :: x_dev(*)
+      integer(c_size_t), value :: ldx
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      type(c_ptr), value :: stop
+      real(c_double), value :: restart_growth
+      type(c_ptr) :: handle
+    end function
+
+    !! NKABATCHQUEUE nka_batch_queue_create_restart (NKABATCH, void *residual_graph, double *x_dev, size_t ldx,
+    !!     double *f_dev, size_t ldf, int *slot_problem_dev, const double *x0_dev, size_t ldx0,
+    !!     double *xout_dev, size_t ldxout, size_t nproblems, const nka_stop_test *stop, double restart_growth)
+    function nka_batch_queue_create_restart(batch, residual_graph, x_dev, ldx, f_dev, ldf, slot_problem_dev, x0_dev, &
+                                            ldx0, xout_dev, ldxout, nproblems, stop, restart_growth) &
+        bind(C, name='nka_batch_queue_create_restart') result(handle)
+      import :: c_ptr, c_double, c_size_t
+      type(c_ptr), value :: batch, residual_graph
+      real(c_double), intent(inout) :: x_dev(*)
+      integer(c_size_t), value :: ldx
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      type(c_ptr), value :: slot_problem_dev
+      real(c_double), intent(in) :: x0_dev(*)
+      integer(c_size_t), value :: ldx0
+      real(c_double), intent(inout) :: xout_dev(*)
+      integer(c_size_t), value :: ldxout, nproblems
+      type(c_ptr), value :: stop
+      real(c_double), value :: restart_growth
+      type(c_ptr) :: handle
+    end function
+
+    !! restarts: c_loc of an integer(c_int) array of nbatch elements on the host
+    subroutine nka_batch_loop_restarts(handle, restarts) bind(C, name='nka_batch_loop_restarts')
+      import :: c_ptr
+      type(c_ptr), value :: handle, restarts
+    end subroutine
+
+    !! restarts: c_loc of an integer(c_int) array of nproblems elements on the host
+    subroutine nka_batch_queue_restarts(handle, restarts) bind(C, name='nka_batch_queue_restarts')
+      import :: c_ptr
+      type(c_ptr), value :: handle, restarts
+    end subroutine
+
   end interface
 
 end module nka_b200_c
