@@ -377,6 +377,52 @@ void nka_batch_loop_restarts (struct nka_batch_loop *L, int *restarts);
 /* nproblems ints on the host; synchronises */
 void nka_batch_queue_restarts (struct nka_batch_queue *Q, int *restarts);
 
+/* ---- interleaved batched accelerators: one thread per member ------------ */
+/* One handle holds nbatch (1..2^31-1, limited only by memory) independent
+ * accelerators that share vlen, mvec (1..32) and vtol, stored component-major:
+ * element i of member b is at f_dev[i*ldf + b] (ldf >= nbatch), the layout of a
+ * Fortran array f(ncell, nvar) with one member per cell.  One update is one
+ * kernel launch whatever nbatch is; each member runs on its own thread.
+ *
+ * Member b's correction vectors, num_vec, lists, Gram factor entries among
+ * list slots, coefficients c, min_margin, ndrop_last, evicted_last and
+ * relaxed_last are bit for bit what the reference's C nka_accel_update /
+ * nka_relax / nka_restart give when fed that member's calls: its dot products
+ * are the reference's serial sums, and no multiply-add is contracted.  They do
+ * not depend on nbatch, the member's index, the other members' data or masks,
+ * ldf, or f_dev's alignment.
+ *
+ * active_dev / mask_dev: NULL (every member) or nbatch device bytes, nonzero =
+ * selected; an unselected member's column of f is neither read nor written and
+ * its state is untouched.  Update, relax, restart and set_vec_tol can be
+ * captured in a CUDA graph (the handle keeps no host-side shape state; vtol
+ * lives on the device); the queries, set_stream and synchronize abort while the
+ * handle's stream captures.  Device-only, single-GPU, no dot-product callback.
+ *
+ * nka_ibatch_get_state fills mvec, subspace, pending, first, last, free_slot,
+ * next, prev, c, h (h[r*(mvec+1)+c]), vtol, min_margin, ndrop_last,
+ * evicted_last and relaxed_last; every other field is zero.
+ *
+ * The prototypes spell the handle as `struct nka_ibatch *`, which NKAIBATCH is. */
+typedef struct nka_ibatch *NKAIBATCH;
+struct nka_ibatch *nka_ibatch_init (int nbatch, size_t vlen, int mvec, double vtol, int device, void *stream);
+void nka_ibatch_delete (struct nka_ibatch *b);
+void nka_ibatch_accel_update (struct nka_ibatch *b, double *f_dev, size_t ldf, const unsigned char *active_dev);
+void nka_ibatch_relax (struct nka_ibatch *b, const unsigned char *mask_dev);
+void nka_ibatch_restart (struct nka_ibatch *b, const unsigned char *mask_dev);
+void nka_ibatch_set_vec_tol (struct nka_ibatch *b, double vtol);
+/* nbatch ints on the host; synchronises */
+void nka_ibatch_num_vec (struct nka_ibatch *b, int *out);
+/* 1 if every member passes the invariant check of nka_defined; synchronises */
+int nka_ibatch_defined (struct nka_ibatch *b);
+void nka_ibatch_get_state (struct nka_ibatch *b, int member, nka_state_view *out);
+void nka_ibatch_set_stream (struct nka_ibatch *b, void *stream);
+void nka_ibatch_synchronize (struct nka_ibatch *b);
+/* as nka_stream_capturing */
+int nka_ibatch_stream_capturing (struct nka_ibatch *b);
+/* kernel launches run eagerly so far; captured kernels are not counted */
+unsigned long long nka_ibatch_launch_count (struct nka_ibatch *b);
+
 #ifdef __cplusplus
 }
 #endif

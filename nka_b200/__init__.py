@@ -6,8 +6,9 @@ layers), and this Python mirror of the reference interface for tests and
 benchmarks.
 """
 from .batch import BatchNKA
+from .ibatch import InterleavedBatchNKA
 from .nka import (NKA, NKAError, comm_unique_id, nka_accel_update, nka_delete, nka_init, nka_max_vec,
                   nka_num_vec, nka_relax, nka_restart, nka_vec_len, nka_vec_tol)
 
-__all__ = ["NKA", "BatchNKA", "NKAError", "comm_unique_id", "nka_init", "nka_delete", "nka_accel_update", "nka_restart",
-           "nka_relax", "nka_num_vec", "nka_max_vec", "nka_vec_len", "nka_vec_tol"]
+__all__ = ["NKA", "BatchNKA", "InterleavedBatchNKA", "NKAError", "comm_unique_id", "nka_init", "nka_delete",
+           "nka_accel_update", "nka_restart", "nka_relax", "nka_num_vec", "nka_max_vec", "nka_vec_len", "nka_vec_tol"]

@@ -132,6 +132,20 @@ SYMBOLS = {
                                                     C.POINTER(StopTest), C.c_double]),
     "nka_batch_loop_restarts": (None, [C.c_void_p, C.POINTER(C.c_int)]),
     "nka_batch_queue_restarts": (None, [C.c_void_p, C.POINTER(C.c_int)]),
+    # include/nka_b200.h: interleaved batched accelerators
+    "nka_ibatch_init": (C.c_void_p, [C.c_int, C.c_size_t, C.c_int, C.c_double, C.c_int, C.c_void_p]),
+    "nka_ibatch_delete": (None, [C.c_void_p]),
+    "nka_ibatch_accel_update": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "nka_ibatch_relax": (None, [C.c_void_p, C.c_void_p]),
+    "nka_ibatch_restart": (None, [C.c_void_p, C.c_void_p]),
+    "nka_ibatch_set_vec_tol": (None, [C.c_void_p, C.c_double]),
+    "nka_ibatch_num_vec": (None, [C.c_void_p, C.POINTER(C.c_int)]),
+    "nka_ibatch_defined": (C.c_int, [C.c_void_p]),
+    "nka_ibatch_get_state": (None, [C.c_void_p, C.c_int, C.POINTER(StateView)]),
+    "nka_ibatch_set_stream": (None, [C.c_void_p, C.c_void_p]),
+    "nka_ibatch_synchronize": (None, [C.c_void_p]),
+    "nka_ibatch_stream_capturing": (C.c_int, [C.c_void_p]),
+    "nka_ibatch_launch_count": (C.c_ulonglong, [C.c_void_p]),
     # include/nka_example.h
     "nka_system_init": (C.c_void_p, [C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),
     "nka_system_init_slab": (C.c_void_p, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_void_p]),

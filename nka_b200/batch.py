@@ -75,16 +75,7 @@ class BatchNKA:
         return h
 
     def _mask(self, mask, what: str):
-        """The device address of a length-nbatch CUDA bool / uint8 tensor, or None for every member."""
-        if mask is None:
-            return None
-        if not _is_torch(mask):
-            raise ValueError("%s must be a CUDA bool or uint8 tensor of length nbatch" % what)
-        import torch
-        if mask.dtype not in (torch.bool, torch.uint8) or not mask.is_cuda or mask.dim() != 1 \
-                or mask.numel() != self.nbatch or (self.nbatch > 1 and mask.stride(0) != 1):
-            raise ValueError("%s must be a contiguous CUDA bool or uint8 tensor of length nbatch" % what)
-        return mask.data_ptr()
+        return _mask_address(mask, self.nbatch, what)
 
     def _rows(self, T, name: str) -> int:
         """The row stride of T, a CUDA float64 tensor [nbatch, vlen] with unit column stride."""
@@ -145,15 +136,7 @@ class BatchNKA:
         v = _lib.StateView()
         self._lib.nka_batch_get_state(self._uncaptured("state", "it copies the device state to the host and synchronises"),
                                       b, C.byref(v))
-        n = v.mvec + 1
-        return {
-            "subspace": v.subspace, "pending": v.pending, "first": v.first, "last": v.last,
-            "free": v.free_slot, "next": list(v.next[:n]), "prev": list(v.prev[:n]),
-            "chained": list(v.chained[:n]), "ndrop_last": v.ndrop_last, "evicted_last": v.evicted_last,
-            "relaxed_last": v.relaxed_last, "error": v.error, "vtol": v.vtol, "min_margin": v.min_margin,
-            "s_last": v.s_last, "c": np.array(v.c[:n]), "s": np.array(v.s[:n]),
-            "h": np.array(v.h[: n * n]).reshape(n, n), "ncalls": v.ncalls,
-        }
+        return _state_dict(v)
 
     def set_stream(self, stream: int | None):
         """The stream every later call is queued on; set the capture stream here before a capture begins."""
@@ -274,6 +257,32 @@ class BatchNKA:
                            "has no conditional graph nodes (the reason is printed on stderr)")
         self._loops.add(queue)
         return queue
+
+
+def _mask_address(mask, nbatch: int, what: str):
+    """The device address of a length-nbatch CUDA bool / uint8 tensor, or None for every member."""
+    if mask is None:
+        return None
+    if not _is_torch(mask):
+        raise ValueError("%s must be a CUDA bool or uint8 tensor of length nbatch" % what)
+    import torch
+    if mask.dtype not in (torch.bool, torch.uint8) or not mask.is_cuda or mask.dim() != 1 \
+            or mask.numel() != nbatch or (nbatch > 1 and mask.stride(0) != 1):
+        raise ValueError("%s must be a contiguous CUDA bool or uint8 tensor of length nbatch" % what)
+    return mask.data_ptr()
+
+
+def _state_dict(v: _lib.StateView) -> dict:
+    """An nka_state_view as the dict NKA.state() returns."""
+    n = v.mvec + 1
+    return {
+        "subspace": v.subspace, "pending": v.pending, "first": v.first, "last": v.last,
+        "free": v.free_slot, "next": list(v.next[:n]), "prev": list(v.prev[:n]),
+        "chained": list(v.chained[:n]), "ndrop_last": v.ndrop_last, "evicted_last": v.evicted_last,
+        "relaxed_last": v.relaxed_last, "error": v.error, "vtol": v.vtol, "min_margin": v.min_margin,
+        "s_last": v.s_last, "c": np.array(v.c[:n]), "s": np.array(v.s[:n]),
+        "h": np.array(v.h[: n * n]).reshape(n, n), "ncalls": v.ncalls,
+    }
 
 
 def _check_stopping(atol, rtol, maxit, dtol):

@@ -538,6 +538,95 @@ module nka_b200_c
       type(c_ptr), value :: handle, restarts
     end subroutine
 
+    !! ---- interleaved batched accelerators (include/nka_b200.h): the handle is a struct nka_ibatch * in a c_ptr.
+    !! A Fortran f(ncell, nvar) with one member per cell is f_dev with ldf = ncell (>= nbatch).
+
+    !! NKAIBATCH nka_ibatch_init (int nbatch, size_t vlen, int mvec, double vtol, int device, void *stream)
+    function nka_ibatch_init(nbatch, vlen, mvec, vtol, device, stream) bind(C, name='nka_ibatch_init') result(handle)
+      import :: c_ptr, c_size_t, c_int, c_double
+      integer(c_int),    value :: nbatch
+      integer(c_size_t), value :: vlen
+      integer(c_int),    value :: mvec
+      real(c_double),    value :: vtol
+      integer(c_int),    value :: device
+      type(c_ptr),       value :: stream
+      type(c_ptr) :: handle
+    end function
+
+    subroutine nka_ibatch_delete(handle) bind(C, name='nka_ibatch_delete')
+      import :: c_ptr
+      type(c_ptr), value :: handle
+    end subroutine
+
+    !! void nka_ibatch_accel_update (NKAIBATCH, double *f_dev, size_t ldf, const unsigned char *active_dev)
+    !! f_dev: the device array f(ldf, vlen), element i of member b at f(b, i) (CUDA Fortran: a device array,
+    !! passed by address); active_dev: c_null_ptr or the device address of nbatch bytes
+    subroutine nka_ibatch_accel_update(handle, f_dev, ldf, active_dev) bind(C, name='nka_ibatch_accel_update')
+      import :: c_ptr, c_double, c_size_t
+      type(c_ptr), value :: handle
+      real(c_double), intent(inout) :: f_dev(*)
+      integer(c_size_t), value :: ldf
+      type(c_ptr), value :: active_dev
+    end subroutine
+
+    subroutine nka_ibatch_relax(handle, mask_dev) bind(C, name='nka_ibatch_relax')
+      import :: c_ptr
+      type(c_ptr), value :: handle, mask_dev
+    end subroutine
+
+    subroutine nka_ibatch_restart(handle, mask_dev) bind(C, name='nka_ibatch_restart')
+      import :: c_ptr
+      type(c_ptr), value :: handle, mask_dev
+    end subroutine
+
+    subroutine nka_ibatch_set_vec_tol(handle, vtol) bind(C, name='nka_ibatch_set_vec_tol')
+      import :: c_ptr, c_double
+      type(c_ptr), value :: handle
+      real(c_double), value :: vtol
+    end subroutine
+
+    !! out: c_loc of an integer(c_int) array of nbatch elements on the host
+    subroutine nka_ibatch_num_vec(handle, out) bind(C, name='nka_ibatch_num_vec')
+      import :: c_ptr
+      type(c_ptr), value :: handle, out
+    end subroutine
+
+    function nka_ibatch_defined(handle) bind(C, name='nka_ibatch_defined') result(ok)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int) :: ok
+    end function
+
+    !! out: c_loc of an nka_state_view on the host
+    subroutine nka_ibatch_get_state(handle, member, out) bind(C, name='nka_ibatch_get_state')
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int), value :: member
+      type(c_ptr), value :: out
+    end subroutine
+
+    subroutine nka_ibatch_set_stream(handle, stream) bind(C, name='nka_ibatch_set_stream')
+      import :: c_ptr
+      type(c_ptr), value :: handle, stream
+    end subroutine
+
+    subroutine nka_ibatch_synchronize(handle) bind(C, name='nka_ibatch_synchronize')
+      import :: c_ptr
+      type(c_ptr), value :: handle
+    end subroutine
+
+    function nka_ibatch_stream_capturing(handle) bind(C, name='nka_ibatch_stream_capturing') result(c)
+      import :: c_ptr, c_int
+      type(c_ptr), value :: handle
+      integer(c_int) :: c
+    end function
+
+    function nka_ibatch_launch_count(handle) bind(C, name='nka_ibatch_launch_count') result(n)
+      import :: c_ptr, c_long_long
+      type(c_ptr), value :: handle
+      integer(c_long_long) :: n
+    end function
+
   end interface
 
 end module nka_b200_c
