@@ -1,9 +1,12 @@
 // nka_batch.h -- the batched accelerator's handle and kernel tables (nka_batch.cu, nka_batch_pass_a.cu,
 // nka_batch_pass_b.cu), shared with its device-side fixed-point loops (nka_batch_loop.cu) and work
-// queues (nka_batch_queue.cu).
+// queues (nka_batch_queue.cu); and the solve core both build on (NkaSolve: nka_batch_loop.cu, whose
+// guard launchers are in nka_batch_guard.cu).
 #pragma once
 #include <cuda_runtime.h>
+#include <stdint.h>
 #include <functional>
+#include <initializer_list>
 #include "nka_dispatch.h"
 #include "../../include/nka_b200.h"
 
@@ -34,36 +37,73 @@ void nka_batch_update_captured(nka_batch* bt, double* f, size_t ldf, const unsig
 // nka_batch_restart of the masked members, queued on a capturing `stream` likewise.
 void nka_batch_restart_captured(nka_batch* bt, const unsigned char* mask, cudaStream_t stream);
 
-// ---- shared by the device-side loops and queues (nka_batch_loop.cu) ----
-// 0 if the driver has conditional graph nodes (12.4); otherwise prints why `call` cannot build its graph.
-int nka_loop_driver_refused(const char* call);
+// ---- the solve core shared by the device-side loops and queues (nka_batch_loop.cu, nka_batch_guard.cu) ----
+// A device-side solve over a batch: its graph, the per-slot state (slot b is member b) and what every body
+// launch needs.  nka_batch_loop and nka_batch_queue derive from it; deleting one frees everything.
+struct NkaSolve {
+  NKABATCH bt = nullptr;
+  cudaGraphExec_t exec = nullptr;
+  int* iters = nullptr;                   // device, nbatch: the slot's steps
+  int* status = nullptr;                  // device, nbatch: NKA_LOOP_* (or a queue's NKA_QUEUE_IDLE)
+  unsigned char* active = nullptr;        // device, nbatch: status == RUNNING, the update's and step's mask
+  double* r0 = nullptr;                   // device, nbatch: each slot's norm at check 0
+  double* rlast = nullptr;                // device, nbatch: each slot's latest norm
+  double* hist = nullptr;                 // device, nhist: check k of slot b at hist[k * hstride + b]
+  double* partials = nullptr;             // device, nbatch x prow
+  unsigned* tickets = nullptr;            // device, nbatch
+  double* rprev = nullptr;                // device, nbatch: the previous check's norm (gamma > 0 only)
+  int* nrst = nullptr;                    // device, nbatch: restarts (gamma > 0 only)
+  unsigned char* rmask = nullptr;         // device, nbatch: the guard's restart mask (gamma > 0 only)
+  double* x = nullptr;                    // the caller's X and F rows
+  const double* f = nullptr;
+  size_t ldx = 0, ldf = 0;
+  size_t nhist = 0, prow = 0;
+  int hstride = 0;                        // a loop's nbatch (maxit+1 rows of history); a queue's 0 (one scratch row)
+  int Vc = 1, Vs = 1;                     // access widths of check (F) and step (X, F)
+  unsigned gc = 0, gs = 0;                // their CTAs per slot
+  nka_stop_test stop = {};
+  double gamma = 0.0;                     // restart_growth; 0: no guard
+  virtual ~NkaSolve();
+};
+
+// The graph's prologue or body: its kernels queued on the capturing stream.
+typedef std::function<void(cudaStream_t, cudaGraphConditionalHandle)> NkaCaptureFn;
+// The create steps loops and queues share, under `call`, for H (a new handle with bt set): the stop test's
+// and gamma's checks, the capture refusal, the driver check, the slot state for x, f and a history of
+// maxit+1 rows (history) or one scratch row, a private stream on which the tickets are zeroed, the state
+// poisoned (NKA_POISON_ALLOC), then `init` allocates and resets the rest, and the graph
+//   prologue -> WHILE (cond) { residual graph, cloned as a child -> body },
+// instantiated, uploaded and synchronised.  A driver or graph CUDA refuses deletes H and gives nullptr,
+// after printing why on stderr.
+NkaSolve* nka_solve_create(const char* call, NkaSolve* H, void* residual, double* x, size_t ldx, const double* f,
+                           size_t ldf, const nka_stop_test* stop, double gamma, bool history,
+                           const std::function<void(cudaStream_t)>& init, const NkaCaptureFn& prologue,
+                           const NkaCaptureFn& body);
+// The body's nka_loop_check<Vc> over dim3(gc, nbatch) on the capturing `s`; it applies the stop test with
+// the per-problem entries of row b at index[b] (index NULL: at b).
+void nka_solve_check(const NkaSolve& H, cudaStream_t s, const int* index);
+// The body's nka_loop_step<Vs> over dim3(gs, nbatch): X_b += F_b of the active slots.
+void nka_solve_step(const NkaSolve& H, cudaStream_t s);
+// The residual-growth restart (nka_batch_guard.cu): the reset of the restart counts nrst and, in a queue,
+// p_restarts (nproblems; NULL and 0 in a loop); and the body's guard followed by the batch's restart of
+// its mask rmask.  claimed, move_out and p_restarts are the queue's (NULL in a loop).
+void nka_solve_guard_reset(const NkaSolve& H, cudaStream_t s, int* p_restarts, size_t nproblems);
+void nka_solve_guard_restart(const NkaSolve& H, cudaStream_t s, const unsigned char* claimed, const int* move_out,
+                             int* p_restarts);
+// The graph launch on the batch's stream, refused (under `call`) while that stream captures.
+void nka_solve_launch(const NkaSolve* H, const char* call);
+// The device-to-host copies of a results query on the batch's stream, refused (call, why) while it captures,
+// then a synchronise.  A copy from NULL zeroes dst instead; with no copy left nothing is synchronised.
+struct NkaCopy { void* dst; const void* src; size_t bytes; };
+void nka_solve_copy_out(const NkaSolve* H, const char* call, const char* why, std::initializer_list<NkaCopy> copies);
+// Waits for the batch's stream and deletes H (NULL: nothing).
+void nka_solve_destroy(NkaSolve* H);
 // CTAs per member of the loop's check and step kernels at access width V (vlen only, as the batch's fix-up)
 int nka_loop_grid(nka_batch* bt, int V);
-// nka_loop_check<V> / nka_loop_step<V> queued on `s` over dim3(grid, nbatch) (nka_batch_loop.cu documents
-// them); check k of member b is recorded at hist[k * hstride + b].  check applies `stop` with the per-problem
-// entries of row b at index[b] (index NULL: at b).
-void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, const double* F, size_t ldf, size_t n,
-                          int hstride, const int* iters, int* status, unsigned char* active, double* r0, double* rlast,
-                          double* hist, double* partials, size_t prow, unsigned* tickets, const nka_stop_test& stop,
-                          const int* index);
-// Aborts (file:line, under `call`) unless `stop` is a valid nka_stop_test for members of length vlen.
-void nka_stop_test_require(const char* call, const nka_stop_test* stop, size_t vlen);
-void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
-                         size_t n, int nbatch, const unsigned char* active, int* iters);
-// The residual-growth restart (nka_batch_guard.cu): the prologue's reset of the restart counts nrst (nbatch)
-// and, in a queue, p_restarts (nproblems; NULL and 0 in a loop); and the body's guard followed by the
-// batch's restart of its mask rmask, queued on the capturing `s`.  claimed, move_out and p_restarts are
-// the queue's (NULL in a loop).
-void nka_loop_guard_reset_launch(cudaStream_t s, int* nrst, int nbatch, int* p_restarts, size_t nproblems);
-void nka_loop_guard_restart(nka_batch* bt, cudaStream_t s, double gamma, const unsigned char* active, const int* iters,
-                            const double* rlast, const unsigned char* claimed, const int* move_out, double* rprev,
-                            int* nrst, int* p_restarts, unsigned char* rmask);
-// The graph  prologue -> WHILE (cond) { residual graph, cloned as a child -> body }, instantiated and
-// uploaded on `s`.  prologue and body queue their kernels on `s` while it captures.  A graph CUDA
-// refuses gives nullptr, after printing CUDA's reason under `call`, with no error left behind.
-typedef std::function<void(cudaStream_t, cudaGraphConditionalHandle)> NkaCaptureFn;
-cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t residual, const NkaCaptureFn& prologue,
-                                const NkaCaptureFn& body);
+// ceil(n / NKA_THREADS) CTAs, clamped to 1..1024: the grid of the solves' element-wise reset kernels
+unsigned nka_grid_clamp(size_t n);
+// Whether rows at p with stride ld are all 16-byte aligned: the base address and an even row stride.
+inline bool nka_aligned16(const void* p, size_t ld) { return (uintptr_t)p % 16 == 0 && ld % 2 == 0; }
 
 // (F, ldf, W, wstride, ld, n, S, partials, prow, tickets, dots, active)
 typedef void (*NkaBatchPassAFn)(const double*, size_t, const double*, size_t, size_t, size_t, const NkaDevState*, double*,

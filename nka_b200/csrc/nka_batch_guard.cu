@@ -11,6 +11,7 @@
 // check recorded (rlast), kept per slot in rprev.  rprev is read only when k >= 1 and written at every
 // check of a running member, so r_{k-1} is always this launch's (loop) or this problem's (queue).  The
 // guard is per slot and reads only the slot's own values, so a problem's bits do not depend on its slot.
+// Its launchers take the solve core's handle (nka_batch.h: NkaSolve), whose rprev, nrst and rmask it uses.
 #include <cuda_runtime.h>
 
 #include "nka_internal.h"
@@ -65,25 +66,20 @@ nka_loop_guard(const unsigned char* __restrict__ active, const int* __restrict__
 // ---------------------------------------------------------------------------
 // launchers (nka_batch.h)
 // ---------------------------------------------------------------------------
-static unsigned grid_for(size_t n)
+void nka_solve_guard_reset(const NkaSolve& H, cudaStream_t s, int* p_restarts, size_t nproblems)
 {
-  const size_t g = (n + NKA_THREADS - 1) / NKA_THREADS;
-  return (unsigned)(g < 1024 ? (g < 1 ? 1 : g) : 1024);
-}
-
-void nka_loop_guard_reset_launch(cudaStream_t s, int* nrst, int nbatch, int* p_restarts, size_t nproblems)
-{
+  const int nbatch = H.bt->nbatch;
   const size_t n = nproblems > (size_t)nbatch ? nproblems : (size_t)nbatch;
-  nka_loop_guard_reset<<<grid_for(n), NKA_THREADS, 0, s>>>(nrst, nbatch, p_restarts, nproblems);
+  nka_loop_guard_reset<<<nka_grid_clamp(n), NKA_THREADS, 0, s>>>(H.nrst, nbatch, p_restarts, nproblems);
   CUDA_CHECK(cudaGetLastError());
 }
 
-void nka_loop_guard_restart(nka_batch* bt, cudaStream_t s, double gamma, const unsigned char* active, const int* iters,
-                            const double* rlast, const unsigned char* claimed, const int* move_out, double* rprev,
-                            int* nrst, int* p_restarts, unsigned char* rmask)
+void nka_solve_guard_restart(const NkaSolve& H, cudaStream_t s, const unsigned char* claimed, const int* move_out,
+                             int* p_restarts)
 {
-  nka_loop_guard<<<grid_for((size_t)bt->nbatch), NKA_THREADS, 0, s>>>(active, iters, rlast, claimed, move_out, gamma,
-                                                                      rprev, nrst, p_restarts, rmask, bt->nbatch);
+  nka_loop_guard<<<nka_grid_clamp((size_t)H.bt->nbatch), NKA_THREADS, 0, s>>>(H.active, H.iters, H.rlast, claimed, move_out,
+                                                                            H.gamma, H.rprev, H.nrst, p_restarts, H.rmask,
+                                                                            H.bt->nbatch);
   CUDA_CHECK(cudaGetLastError());
-  nka_batch_restart_captured(bt, rmask, s);
+  nka_batch_restart_captured(H.bt, H.rmask, s);
 }

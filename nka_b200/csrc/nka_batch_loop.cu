@@ -10,6 +10,8 @@
 //     nka_grid_reduce folds its partial rows in a fixed order, so a norm depends on the row alone;
 //   - the update is nka_batch_accel_update's own launch sequence, with check's mask;
 //   - step is X_b + F_b element by element, as X[b] += F[b] computes it.
+// The host side is the solve core the work queues share (nka_batch.h: NkaSolve, nka_solve_create): the
+// per-slot state, the create steps, the check and step launchers and the entry points' common parts.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -151,69 +153,26 @@ nka_loop_step(double* __restrict__ X, size_t ldx, const double* __restrict__ F, 
 }
 
 // ---------------------------------------------------------------------------
-// the handle
+// the solve core, shared with the work queues (nka_batch_queue.cu)
 // ---------------------------------------------------------------------------
-struct nka_batch_loop {
-  NKABATCH bt = nullptr;
-  int maxit = 0;
-  cudaGraphExec_t exec = nullptr;
-  int* iters = nullptr;                   // device, nbatch
-  int* status = nullptr;                  // device, nbatch
-  unsigned char* active = nullptr;        // device, nbatch: status == RUNNING, the update's mask
-  double* r0 = nullptr;                   // device, nbatch: each member's norm at check 0
-  double* rlast = nullptr;                // device, nbatch: each member's latest norm
-  double* hist = nullptr;                 // device, (maxit+1) x nbatch
-  double* partials = nullptr;             // device, nbatch x prow
-  unsigned* tickets = nullptr;            // device, nbatch
-  double* rprev = nullptr;                // device, nbatch: the previous check's norm (restart_growth > 0 only)
-  int* nrst = nullptr;                    // device, nbatch: restarts in this launch (restart_growth > 0 only)
-  unsigned char* rmask = nullptr;         // device, nbatch: the guard's restart mask (restart_growth > 0 only)
-};
-
-static void loop_free(NKABATCHLOOP L)
+NkaSolve::~NkaSolve()
 {
-  if (L->exec) cudaGraphExecDestroy(L->exec);
-  cudaFree(L->iters); cudaFree(L->status); cudaFree(L->active); cudaFree(L->r0); cudaFree(L->rlast);
-  cudaFree(L->hist); cudaFree(L->partials); cudaFree(L->tickets); cudaFree(L->rprev); cudaFree(L->nrst);
-  cudaFree(L->rmask);
-  delete L;
+  if (exec) cudaGraphExecDestroy(exec);
+  cudaFree(iters); cudaFree(status); cudaFree(active); cudaFree(r0); cudaFree(rlast); cudaFree(hist);
+  cudaFree(partials); cudaFree(tickets); cudaFree(rprev); cudaFree(nrst); cudaFree(rmask);
 }
 
-// ---------------------------------------------------------------------------
-// shared with the work queues (nka_batch_queue.cu)
-// ---------------------------------------------------------------------------
-int nka_loop_driver_refused(const char* call)
-{
-  int driver = 0;
-  CUDA_CHECK(cudaDriverGetVersion(&driver));
-  if (driver >= 12040) return 0;
-  fprintf(stderr, "nka_b200: %s: conditional graph nodes need a CUDA 12.4 driver, this one is %d.%d: %s\n", call,
-          driver / 1000, (driver % 1000) / 10, cudaGetErrorString(cudaErrorInsufficientDriver));
-  fflush(stderr);
-  return 1;
-}
-
-// CTAs per member of check and step: the batch's rule for a one-accumulator sweep of vlen (its fix-up's)
 int nka_loop_grid(NKABATCH bt, int V) { return nka_grid_for(bt->geom, 4, bt->vlen, V, NKA_THREADS); }
 
-void nka_loop_queue_check(int V, unsigned grid, int nbatch, cudaStream_t s, const double* F, size_t ldf, size_t n,
-                          int hstride, const int* iters, int* status, unsigned char* active, double* r0, double* rlast,
-                          double* hist, double* partials, size_t prow, unsigned* tickets, const nka_stop_test& stop,
-                          const int* index)
+unsigned nka_grid_clamp(size_t n)
 {
-  const dim3 g(grid, (unsigned)nbatch);
-  // the scale's load width follows its own rows' alignment; V and grid follow F's alone
-  const int scale16 = stop.scale_dev && (uintptr_t)stop.scale_dev % 16 == 0 && stop.ldscale % 2 == 0;
-  if (V == 2)
-    nka_loop_check<2><<<g, NKA_THREADS, 0, s>>>(F, ldf, n, hstride, iters, status, active, r0, rlast, hist, partials, prow,
-                                                tickets, stop, index, scale16);
-  else
-    nka_loop_check<1><<<g, NKA_THREADS, 0, s>>>(F, ldf, n, hstride, iters, status, active, r0, rlast, hist, partials, prow,
-                                                tickets, stop, index, scale16);
-  CUDA_CHECK(cudaGetLastError());
+  const size_t g = (n + NKA_THREADS - 1) / NKA_THREADS;
+  return (unsigned)(g < 1024 ? (g < 1 ? 1 : g) : 1024);
 }
 
-void nka_stop_test_require(const char* call, const nka_stop_test* stop, size_t vlen)
+// Aborts (file:line, under `call`) unless `stop` is a valid nka_stop_test for members of length vlen and
+// gamma a valid restart_growth.
+static void solve_require(const char* call, const nka_stop_test* stop, size_t vlen, double gamma)
 {
   char msg[160];
   const auto require = [&](bool ok, const char* what) {
@@ -226,17 +185,19 @@ void nka_stop_test_require(const char* call, const nka_stop_test* stop, size_t v
   require(stop->maxit >= 0, "maxit must be >= 0");
   require(stop->dtol == 0.0 || stop->dtol >= 1.0, "dtol must be 0 (off) or >= 1");
   require(!stop->scale_dev || stop->ldscale >= vlen, "ldscale must be >= vlen");
+  require(gamma >= 0.0 && isfinite(gamma), "restart_growth must be 0 (off) or a finite number > 0");
 }
 
-void nka_loop_queue_step(int V, unsigned grid, cudaStream_t s, double* X, size_t ldx, const double* F, size_t ldf,
-                         size_t n, int nbatch, const unsigned char* active, int* iters)
+// 0 if the driver has conditional graph nodes (12.4); otherwise prints why `call` cannot build its graph.
+static int driver_refused(const char* call)
 {
-  const dim3 g(grid, (unsigned)nbatch);
-  if (V == 2)
-    nka_loop_step<2><<<g, NKA_THREADS, 0, s>>>(X, ldx, F, ldf, n, active, iters);
-  else
-    nka_loop_step<1><<<g, NKA_THREADS, 0, s>>>(X, ldx, F, ldf, n, active, iters);
-  CUDA_CHECK(cudaGetLastError());
+  int driver = 0;
+  CUDA_CHECK(cudaDriverGetVersion(&driver));
+  if (driver >= 12040) return 0;
+  fprintf(stderr, "nka_b200: %s: conditional graph nodes need a CUDA 12.4 driver, this one is %d.%d: %s\n", call,
+          driver / 1000, (driver % 1000) / 10, cudaGetErrorString(cudaErrorInsufficientDriver));
+  fflush(stderr);
+  return 1;
 }
 
 // CUDA refused the graph: the caller's residual graph or the driver.  Not a library fault: print CUDA's
@@ -250,8 +211,11 @@ static cudaGraphExec_t graph_refused(const char* call, cudaGraph_t g, const char
   return nullptr;
 }
 
-cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t residual, const NkaCaptureFn& prologue,
-                                const NkaCaptureFn& body_fn)
+// The graph  prologue -> WHILE (cond) { residual graph, cloned as a child -> body }, instantiated and
+// uploaded on `s`.  A graph CUDA refuses gives nullptr, after printing CUDA's reason under `call`, with no
+// error left behind.
+static cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t residual,
+                                       const NkaCaptureFn& prologue, const NkaCaptureFn& body_fn)
 {
   cudaGraph_t g = nullptr;
   CUDA_CHECK(cudaGraphCreate(&g, 0));
@@ -302,9 +266,129 @@ cudaGraphExec_t nka_while_graph(const char* call, cudaStream_t s, cudaGraph_t re
   return exec;
 }
 
+NkaSolve* nka_solve_create(const char* call, NkaSolve* H, void* residual, double* x, size_t ldx, const double* f,
+                           size_t ldf, const nka_stop_test* stop, double gamma, bool history,
+                           const std::function<void(cudaStream_t)>& init, const NkaCaptureFn& prologue,
+                           const NkaCaptureFn& body)
+{
+  NKABATCH bt = H->bt;
+  solve_require(call, stop, bt->vlen, gamma);
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, call, "it builds and uploads a graph and synchronises");
+  if (driver_refused(call)) {
+    delete H;
+    return nullptr;
+  }
+  const size_t nb = (size_t)bt->nbatch;
+  H->x = x, H->ldx = ldx, H->f = f, H->ldf = ldf;
+  H->stop = *stop;
+  H->gamma = gamma;
+  H->hstride = history ? bt->nbatch : 0;
+  H->nhist = history ? (size_t)(stop->maxit + 1) * nb : nb;
+  // the 16-byte paths need every row 16-byte aligned
+  H->Vc = nka_aligned16(f, ldf) ? 2 : 1;
+  H->Vs = H->Vc == 2 && nka_aligned16(x, ldx) ? 2 : 1;
+  H->gc = (unsigned)nka_loop_grid(bt, H->Vc);
+  H->gs = (unsigned)nka_loop_grid(bt, H->Vs);
+  H->prow = H->gc;
+  CUDA_CHECK(cudaMalloc(&H->iters, nb * sizeof(int)));
+  CUDA_CHECK(cudaMalloc(&H->status, nb * sizeof(int)));
+  CUDA_CHECK(cudaMalloc(&H->active, nb));
+  CUDA_CHECK(cudaMalloc(&H->r0, nb * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&H->rlast, nb * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&H->hist, H->nhist * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&H->partials, nb * H->prow * sizeof(double)));
+  CUDA_CHECK(cudaMalloc(&H->tickets, nb * sizeof(unsigned)));
+  if (gamma > 0.0) {
+    CUDA_CHECK(cudaMalloc(&H->rprev, nb * sizeof(double)));
+    CUDA_CHECK(cudaMalloc(&H->nrst, nb * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&H->rmask, nb));
+  }
+
+  cudaStream_t s = nullptr;               // private: the batch's own stream may be the legacy default
+  CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+  CUDA_CHECK(cudaMemsetAsync(H->tickets, 0, nb * sizeof(unsigned), s));
+  if (bt->poison) {
+    CUDA_CHECK(cudaMemsetAsync(H->partials, 0xFF, nb * H->prow * sizeof(double), s));
+    CUDA_CHECK(cudaMemsetAsync(H->r0, 0xFF, nb * sizeof(double), s));
+    CUDA_CHECK(cudaMemsetAsync(H->rlast, 0xFF, nb * sizeof(double), s));
+    CUDA_CHECK(cudaMemsetAsync(H->hist, 0xFF, H->nhist * sizeof(double), s));
+    if (gamma > 0.0) CUDA_CHECK(cudaMemsetAsync(H->rprev, 0xFF, nb * sizeof(double), s));
+  }
+  init(s);
+  H->exec = nka_while_graph(call, s, (cudaGraph_t)residual, prologue, body);
+  if (!H->exec) {
+    cudaStreamDestroy(s);
+    delete H;
+    return nullptr;
+  }
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  CUDA_CHECK(cudaStreamDestroy(s));
+  return H;
+}
+
+void nka_solve_check(const NkaSolve& H, cudaStream_t s, const int* index)
+{
+  const dim3 g(H.gc, (unsigned)H.bt->nbatch);
+  // the scale's load width follows its own rows' alignment; Vc and gc follow F's alone
+  const int scale16 = H.stop.scale_dev && nka_aligned16(H.stop.scale_dev, H.stop.ldscale);
+  if (H.Vc == 2)
+    nka_loop_check<2><<<g, NKA_THREADS, 0, s>>>(H.f, H.ldf, H.bt->vlen, H.hstride, H.iters, H.status, H.active, H.r0,
+                                                H.rlast, H.hist, H.partials, H.prow, H.tickets, H.stop, index, scale16);
+  else
+    nka_loop_check<1><<<g, NKA_THREADS, 0, s>>>(H.f, H.ldf, H.bt->vlen, H.hstride, H.iters, H.status, H.active, H.r0,
+                                                H.rlast, H.hist, H.partials, H.prow, H.tickets, H.stop, index, scale16);
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void nka_solve_step(const NkaSolve& H, cudaStream_t s)
+{
+  const dim3 g(H.gs, (unsigned)H.bt->nbatch);
+  if (H.Vs == 2)
+    nka_loop_step<2><<<g, NKA_THREADS, 0, s>>>(H.x, H.ldx, H.f, H.ldf, H.bt->vlen, H.active, H.iters);
+  else
+    nka_loop_step<1><<<g, NKA_THREADS, 0, s>>>(H.x, H.ldx, H.f, H.ldf, H.bt->vlen, H.active, H.iters);
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void nka_solve_launch(const NkaSolve* H, const char* call)
+{
+  DeviceGuard guard(H->bt->device);
+  if (nka_capture_status(H->bt->stream) != 0)
+    nka_capture_fail(call, "a graph with conditional nodes cannot become a child of another graph");
+  CUDA_CHECK(cudaGraphLaunch(H->exec, H->bt->stream));
+}
+
+void nka_solve_copy_out(const NkaSolve* H, const char* call, const char* why, std::initializer_list<NkaCopy> copies)
+{
+  NKABATCH bt = H->bt;
+  DeviceGuard guard(bt->device);
+  nka_refuse_capture(bt->stream, call, why);
+  bool queued = false;
+  for (const NkaCopy& c : copies) {
+    if (!c.src) {
+      memset(c.dst, 0, c.bytes);
+      continue;
+    }
+    CUDA_CHECK(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, bt->stream));
+    queued = true;
+  }
+  if (queued) CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+}
+
+void nka_solve_destroy(NkaSolve* H)
+{
+  if (!H) return;
+  DeviceGuard guard(H->bt->device);
+  cudaStreamSynchronize(H->bt->stream);
+  delete H;
+}
+
 // ---------------------------------------------------------------------------
-// the handle's entry points
+// the handle and its entry points
 // ---------------------------------------------------------------------------
+struct nka_batch_loop : NkaSolve {};
+
 extern "C" NKABATCHLOOP nka_batch_loop_create(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
                                              size_t ldf, double atol, double rtol, int maxit)
 {
@@ -326,134 +410,58 @@ extern "C" NKABATCHLOOP nka_batch_loop_create_restart(NKABATCH bt, void* residua
   NKA_REQUIRE(residual_graph != NULL, "nka_batch_loop_create: null residual graph");
   NKA_REQUIRE(x != NULL && f != NULL, "nka_batch_loop_create: null x or f");
   NKA_REQUIRE(ldx >= bt->vlen && ldf >= bt->vlen, "nka_batch_loop_create: ldx and ldf must be >= vlen");
-  nka_stop_test_require("nka_batch_loop_create", stop_in, bt->vlen);
-  NKA_REQUIRE(restart_growth >= 0.0 && isfinite(restart_growth),
-              "nka_batch_loop_create: restart_growth must be 0 (off) or a finite number > 0");
-  const nka_stop_test stop = *stop_in;
-  const bool guarded = restart_growth > 0.0;
-  const int maxit = stop.maxit;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_loop_create", "it builds and uploads a graph and synchronises");
-  if (nka_loop_driver_refused("nka_batch_loop_create")) return nullptr;
-
   NKABATCHLOOP L = new nka_batch_loop();
   L->bt = bt;
-  L->maxit = maxit;
-  const size_t nb = (size_t)bt->nbatch;
-  const size_t nhist = (size_t)(maxit + 1) * nb;
-  // the 16-byte paths need every row 16-byte aligned: the base address and an even row stride
-  const int Vc = ((uintptr_t)f % 16 == 0 && ldf % 2 == 0) ? 2 : 1;
-  const int Vs = Vc == 2 && (uintptr_t)x % 16 == 0 && ldx % 2 == 0 ? 2 : 1;
-  const unsigned gc = (unsigned)nka_loop_grid(bt, Vc), gs = (unsigned)nka_loop_grid(bt, Vs);
-  const size_t prow = gc;
-  CUDA_CHECK(cudaMalloc(&L->iters, nb * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&L->status, nb * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&L->active, nb));
-  CUDA_CHECK(cudaMalloc(&L->r0, nb * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&L->rlast, nb * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&L->hist, nhist * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&L->partials, nb * prow * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&L->tickets, nb * sizeof(unsigned)));
-  if (guarded) {
-    CUDA_CHECK(cudaMalloc(&L->rprev, nb * sizeof(double)));
-    CUDA_CHECK(cudaMalloc(&L->nrst, nb * sizeof(int)));
-    CUDA_CHECK(cudaMalloc(&L->rmask, nb));
-  }
-
-  cudaStream_t s = nullptr;               // private: the batch's own stream may be the legacy default
-  CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-  CUDA_CHECK(cudaMemsetAsync(L->tickets, 0, nb * sizeof(unsigned), s));
-  if (bt->poison) {
-    CUDA_CHECK(cudaMemsetAsync(L->partials, 0xFF, nb * prow * sizeof(double), s));
-    CUDA_CHECK(cudaMemsetAsync(L->r0, 0xFF, nb * sizeof(double), s));
-    if (guarded) CUDA_CHECK(cudaMemsetAsync(L->rprev, 0xFF, nb * sizeof(double), s));
-  }
-  const unsigned greset = (unsigned)((nhist + NKA_THREADS - 1) / NKA_THREADS < 1024 ? (nhist + NKA_THREADS - 1) / NKA_THREADS : 1024);
-  // before any launch: every member RUNNING at 0 steps, as the results of a loop never launched read
-  nka_loop_reset<<<greset, NKA_THREADS, 0, s>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
-  CUDA_CHECK(cudaGetLastError());
-  if (guarded) nka_loop_guard_reset_launch(s, L->nrst, bt->nbatch, nullptr, 0);
-
-  // reset [, guard reset], then the WHILE node: { residual, check, decide, [guard, restart,] update, step }
-  auto prologue = [&](cudaStream_t cs, cudaGraphConditionalHandle) {
-    nka_loop_reset<<<greset, NKA_THREADS, 0, cs>>>(L->iters, L->status, L->active, L->rlast, L->hist, nhist, bt->nbatch);
+  // reset [, guard reset]; at create time too: every member RUNNING at 0 steps, as the results of a loop
+  // never launched read
+  const auto reset = [&](cudaStream_t cs) {
+    nka_loop_reset<<<nka_grid_clamp(L->nhist), NKA_THREADS, 0, cs>>>(L->iters, L->status, L->active, L->rlast, L->hist,
+                                                                     L->nhist, bt->nbatch);
     CUDA_CHECK(cudaGetLastError());
-    if (guarded) nka_loop_guard_reset_launch(cs, L->nrst, bt->nbatch, nullptr, 0);
+    if (L->gamma > 0.0) nka_solve_guard_reset(*L, cs, nullptr, 0);
   };
-  auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
-    nka_loop_queue_check(Vc, gc, bt->nbatch, cs, f, ldf, bt->vlen, bt->nbatch, L->iters, L->status, L->active, L->r0, L->rlast,
-                         L->hist, L->partials, prow, L->tickets, stop, /*index=*/nullptr);
+  // then the WHILE node: { residual, check, decide, [guard, restart,] update, step }
+  const auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
+    nka_solve_check(*L, cs, /*index=*/nullptr);
     nka_loop_decide<<<1, 1024, 0, cs>>>(L->active, bt->nbatch, cond);
     CUDA_CHECK(cudaGetLastError());
-    if (guarded)
-      nka_loop_guard_restart(bt, cs, restart_growth, L->active, L->iters, L->rlast, nullptr, nullptr, L->rprev, L->nrst,
-                             nullptr, L->rmask);
+    if (L->gamma > 0.0) nka_solve_guard_restart(*L, cs, nullptr, nullptr, nullptr);
     nka_batch_update_captured(bt, f, ldf, L->active, cs);
-    nka_loop_queue_step(Vs, gs, cs, x, ldx, f, ldf, bt->vlen, bt->nbatch, L->active, L->iters);
+    nka_solve_step(*L, cs);
   };
-  L->exec = nka_while_graph("nka_batch_loop_create", s, (cudaGraph_t)residual_graph, prologue, body);
-  if (!L->exec) {
-    cudaStreamDestroy(s);
-    loop_free(L);
-    return nullptr;
-  }
-  CUDA_CHECK(cudaStreamSynchronize(s));
-  CUDA_CHECK(cudaStreamDestroy(s));
-  return L;
+  return static_cast<NKABATCHLOOP>(nka_solve_create("nka_batch_loop_create", L, residual_graph, x, ldx, f, ldf, stop_in,
+                                                    restart_growth, /*history=*/true, reset,
+                                                    [&](cudaStream_t cs, cudaGraphConditionalHandle) { reset(cs); },
+                                                    body));
 }
 
 extern "C" void nka_batch_loop_launch(NKABATCHLOOP L)
 {
   NKA_REQUIRE(L != NULL, "nka_batch_loop_launch: null loop");
-  DeviceGuard guard(L->bt->device);
-  if (nka_capture_status(L->bt->stream) != 0)
-    nka_capture_fail("nka_batch_loop_launch", "a graph with conditional nodes cannot become a child of another graph");
-  CUDA_CHECK(cudaGraphLaunch(L->exec, L->bt->stream));
+  nka_solve_launch(L, "nka_batch_loop_launch");
 }
 
 extern "C" void nka_batch_loop_results(NKABATCHLOOP L, int* iters, int* status, double* norm)
 {
   NKA_REQUIRE(L != NULL && iters != NULL && status != NULL && norm != NULL, "nka_batch_loop_results: null argument");
-  NKABATCH bt = L->bt;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_loop_results", "it copies the loop's results to the host and synchronises");
-  const size_t nb = (size_t)bt->nbatch;
-  CUDA_CHECK(cudaMemcpyAsync(iters, L->iters, nb * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaMemcpyAsync(status, L->status, nb * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaMemcpyAsync(norm, L->rlast, nb * sizeof(double), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+  const size_t nb = (size_t)L->bt->nbatch;
+  nka_solve_copy_out(L, "nka_batch_loop_results", "it copies the loop's results to the host and synchronises",
+                     {{iters, L->iters, nb * sizeof(int)}, {status, L->status, nb * sizeof(int)},
+                      {norm, L->rlast, nb * sizeof(double)}});
 }
 
 extern "C" void nka_batch_loop_history(NKABATCHLOOP L, double* norms)
 {
   NKA_REQUIRE(L != NULL && norms != NULL, "nka_batch_loop_history: null argument");
-  NKABATCH bt = L->bt;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_loop_history", "it copies the loop's history to the host and synchronises");
-  const size_t bytes = (size_t)(L->maxit + 1) * (size_t)bt->nbatch * sizeof(double);
-  CUDA_CHECK(cudaMemcpyAsync(norms, L->hist, bytes, cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+  nka_solve_copy_out(L, "nka_batch_loop_history", "it copies the loop's history to the host and synchronises",
+                     {{norms, L->hist, L->nhist * sizeof(double)}});
 }
 
 extern "C" void nka_batch_loop_restarts(NKABATCHLOOP L, int* restarts)
 {
   NKA_REQUIRE(L != NULL && restarts != NULL, "nka_batch_loop_restarts: null argument");
-  NKABATCH bt = L->bt;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_loop_restarts", "it copies the loop's restart counts to the host and synchronises");
-  const size_t nb = (size_t)bt->nbatch;
-  if (!L->nrst) {
-    memset(restarts, 0, nb * sizeof(int));
-    return;
-  }
-  CUDA_CHECK(cudaMemcpyAsync(restarts, L->nrst, nb * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+  nka_solve_copy_out(L, "nka_batch_loop_restarts", "it copies the loop's restart counts to the host and synchronises",
+                     {{restarts, L->nrst, (size_t)L->bt->nbatch * sizeof(int)}});
 }
 
-extern "C" void nka_batch_loop_destroy(NKABATCHLOOP L)
-{
-  if (!L) return;
-  DeviceGuard guard(L->bt->device);
-  cudaStreamSynchronize(L->bt->stream);
-  loop_free(L);
-}
+extern "C" void nka_batch_loop_destroy(NKABATCHLOOP L) { nka_solve_destroy(L); }

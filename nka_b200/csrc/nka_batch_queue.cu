@@ -12,13 +12,13 @@
 // initial guess in; restart restarts the claimed slots' accelerators.  A claimed slot is not checked
 // until the next body, whose check sees the residual at its initial guess and sets r0 there, as the
 // loop's first check does.  Every kernel is per slot or element-wise, so a problem's bits are those
-// of the loop on a just-restarted member, whatever slot it lands in and whatever surrounds it.
+// of the loop on a just-restarted member, whatever slot it lands in and whatever surrounds it.  The
+// queue is built on the loop's solve core (nka_batch.h: NkaSolve, nka_solve_create); this file keeps
+// the queue's own arguments and per-problem arrays, its kernels, and its prologue and body.
 #include <cuda_runtime.h>
 #include <limits.h>
-#include <stdint.h>
 #include <math.h>
 #include <stdio.h>
-#include <string.h>
 
 #include "../../include/nka_b200.h"
 #include "nka_internal.h"
@@ -161,44 +161,24 @@ nka_queue_rows(double* __restrict__ X, size_t ldx, const double* X0, size_t ldx0
 }
 
 // ---------------------------------------------------------------------------
-// the handle
+// the handle: the solve core's slot state (nka_batch.h) and the queue's own arrays
 // ---------------------------------------------------------------------------
-struct nka_batch_queue {
-  NKABATCH bt = nullptr;
+struct nka_batch_queue : NkaSolve {
   size_t nproblems = 0;
-  cudaGraphExec_t exec = nullptr;
-  int* iters = nullptr;                   // device, nbatch: the slot's steps
-  int* status = nullptr;                  // device, nbatch: NKA_LOOP_* or NKA_QUEUE_IDLE
-  unsigned char* active = nullptr;        // device, nbatch: the update's and step's mask
   unsigned char* claimed = nullptr;       // device, nbatch: the restart's mask
-  double* r0 = nullptr;                   // device, nbatch
-  double* rlast = nullptr;                // device, nbatch
-  double* hist = nullptr;                 // device, nbatch: check's history, scratch (stride 0: one per slot)
-  double* partials = nullptr;             // device, nbatch x prow
-  unsigned* tickets = nullptr;            // device, nbatch
   int* move_out = nullptr;                // device, nbatch
   int* move_in = nullptr;                 // device, nbatch
   long long* next = nullptr;              // device: the next problem id to hand out
   int* p_iters = nullptr;                 // device, nproblems
   int* p_status = nullptr;                // device, nproblems
   double* p_norm = nullptr;               // device, nproblems
-  double* rprev = nullptr;                // device, nbatch: the previous check's norm (restart_growth > 0 only)
-  int* nrst = nullptr;                    // device, nbatch: the slot's problem's restarts (restart_growth > 0 only)
-  unsigned char* rmask = nullptr;         // device, nbatch: claimed | the rule (restart_growth > 0 only)
   int* p_restarts = nullptr;              // device, nproblems (restart_growth > 0 only)
+  ~nka_batch_queue() override
+  {
+    cudaFree(claimed); cudaFree(move_out); cudaFree(move_in); cudaFree(next); cudaFree(p_iters); cudaFree(p_status);
+    cudaFree(p_norm); cudaFree(p_restarts);
+  }
 };
-
-static void queue_free(NKABATCHQUEUE Q)
-{
-  if (Q->exec) cudaGraphExecDestroy(Q->exec);
-  cudaFree(Q->iters); cudaFree(Q->status); cudaFree(Q->active); cudaFree(Q->claimed); cudaFree(Q->r0);
-  cudaFree(Q->rlast); cudaFree(Q->hist); cudaFree(Q->partials); cudaFree(Q->tickets); cudaFree(Q->move_out);
-  cudaFree(Q->move_in); cudaFree(Q->next); cudaFree(Q->p_iters); cudaFree(Q->p_status); cudaFree(Q->p_norm);
-  cudaFree(Q->rprev); cudaFree(Q->nrst); cudaFree(Q->rmask); cudaFree(Q->p_restarts);
-  delete Q;
-}
-
-static bool aligned16(const void* p, size_t ld) { return (uintptr_t)p % 16 == 0 && ld % 2 == 0; }
 
 extern "C" NKABATCHQUEUE nka_batch_queue_create(NKABATCH bt, void* residual_graph, double* x, size_t ldx, double* f,
                                                size_t ldf, int* slot_problem, const double* x0, size_t ldx0,
@@ -231,69 +211,31 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_restart(NKABATCH bt, void* resid
   NKA_REQUIRE(ldx >= bt->vlen && ldf >= bt->vlen && ldx0 >= bt->vlen && ldxout >= bt->vlen,
               "nka_batch_queue_create: ldx, ldf, ldx0 and ldxout must be >= vlen");
   NKA_REQUIRE(nproblems >= 1 && nproblems <= (size_t)INT_MAX, "nka_batch_queue_create: nproblems must be in 1..INT_MAX");
-  nka_stop_test_require("nka_batch_queue_create", stop_in, bt->vlen);
-  NKA_REQUIRE(restart_growth >= 0.0 && isfinite(restart_growth),
-              "nka_batch_queue_create: restart_growth must be 0 (off) or a finite number > 0");
-  const nka_stop_test stop = *stop_in;
-  const bool guarded = restart_growth > 0.0;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_queue_create", "it builds and uploads a graph and synchronises");
-  if (nka_loop_driver_refused("nka_batch_queue_create")) return nullptr;
-
   NKABATCHQUEUE Q = new nka_batch_queue();
   Q->bt = bt;
   Q->nproblems = nproblems;
   const size_t nb = (size_t)bt->nbatch;
-  const int Vc = aligned16(f, ldf) ? 2 : 1;
-  const int Vs = Vc == 2 && aligned16(x, ldx) ? 2 : 1;
-  const int Vr = aligned16(x, ldx) && aligned16(x0, ldx0) && aligned16(xout, ldxout) ? 2 : 1;
-  const unsigned gc = (unsigned)nka_loop_grid(bt, Vc), gs = (unsigned)nka_loop_grid(bt, Vs);
-  const unsigned gr = (unsigned)nka_loop_grid(bt, Vr);
-  const size_t prow = gc;
-  CUDA_CHECK(cudaMalloc(&Q->iters, nb * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&Q->status, nb * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&Q->active, nb));
-  CUDA_CHECK(cudaMalloc(&Q->claimed, nb));
-  CUDA_CHECK(cudaMalloc(&Q->r0, nb * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&Q->rlast, nb * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&Q->hist, nb * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&Q->partials, nb * prow * sizeof(double)));
-  CUDA_CHECK(cudaMalloc(&Q->tickets, nb * sizeof(unsigned)));
-  CUDA_CHECK(cudaMalloc(&Q->move_out, nb * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&Q->move_in, nb * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&Q->next, sizeof(long long)));
-  CUDA_CHECK(cudaMalloc(&Q->p_iters, nproblems * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&Q->p_status, nproblems * sizeof(int)));
-  CUDA_CHECK(cudaMalloc(&Q->p_norm, nproblems * sizeof(double)));
-  if (guarded) {
-    CUDA_CHECK(cudaMalloc(&Q->rprev, nb * sizeof(double)));
-    CUDA_CHECK(cudaMalloc(&Q->nrst, nb * sizeof(int)));
-    CUDA_CHECK(cudaMalloc(&Q->rmask, nb));
-    CUDA_CHECK(cudaMalloc(&Q->p_restarts, nproblems * sizeof(int)));
-  }
-
-  cudaStream_t s = nullptr;               // private: the batch's own stream may be the legacy default
-  CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-  CUDA_CHECK(cudaMemsetAsync(Q->tickets, 0, nb * sizeof(unsigned), s));
-  if (bt->poison) {
-    CUDA_CHECK(cudaMemsetAsync(Q->partials, 0xFF, nb * prow * sizeof(double), s));
-    CUDA_CHECK(cudaMemsetAsync(Q->r0, 0xFF, nb * sizeof(double), s));
-    CUDA_CHECK(cudaMemsetAsync(Q->rlast, 0xFF, nb * sizeof(double), s));
-    CUDA_CHECK(cudaMemsetAsync(Q->hist, 0xFF, nb * sizeof(double), s));
-    if (guarded) CUDA_CHECK(cudaMemsetAsync(Q->rprev, 0xFF, nb * sizeof(double), s));
-  }
-  const size_t nreset = nproblems > nb ? nproblems : nb;
-  const unsigned greset = (unsigned)((nreset + NKA_THREADS - 1) / NKA_THREADS < 1024 ? (nreset + NKA_THREADS - 1) / NKA_THREADS : 1024);
-  auto reset = [&](cudaStream_t cs, int nslots) {
+  const int Vr = nka_aligned16(x, ldx) && nka_aligned16(x0, ldx0) && nka_aligned16(xout, ldxout) ? 2 : 1;
+  const dim3 grows((unsigned)nka_loop_grid(bt, Vr), (unsigned)nb);
+  const unsigned greset = nka_grid_clamp(nproblems > nb ? nproblems : nb);
+  const auto reset = [&](cudaStream_t cs, int nslots) {
     nka_queue_reset<<<greset, NKA_THREADS, 0, cs>>>(Q->p_iters, Q->p_status, Q->p_norm, nproblems, slot_problem, Q->status,
                                                    Q->active, nslots, Q->next);
     CUDA_CHECK(cudaGetLastError());
+    if (Q->gamma > 0.0) nka_solve_guard_reset(*Q, cs, Q->p_restarts, nproblems);
   };
-  // before any launch: every problem RUNNING at 0 steps (slot_problem is the caller's until a launch)
-  reset(s, 0);
-  if (guarded) nka_loop_guard_reset_launch(s, Q->nrst, bt->nbatch, Q->p_restarts, nproblems);
-
-  const dim3 grows(gr, (unsigned)nb);
+  const auto init = [&](cudaStream_t s) {
+    CUDA_CHECK(cudaMalloc(&Q->claimed, nb));
+    CUDA_CHECK(cudaMalloc(&Q->move_out, nb * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&Q->move_in, nb * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&Q->next, sizeof(long long)));
+    CUDA_CHECK(cudaMalloc(&Q->p_iters, nproblems * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&Q->p_status, nproblems * sizeof(int)));
+    CUDA_CHECK(cudaMalloc(&Q->p_norm, nproblems * sizeof(double)));
+    if (Q->gamma > 0.0) CUDA_CHECK(cudaMalloc(&Q->p_restarts, nproblems * sizeof(int)));
+    // before any launch: every problem RUNNING at 0 steps (slot_problem is the caller's until a launch)
+    reset(s, 0);
+  };
   auto claim_rows_restart = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
     nka_queue_claim<<<1, NKA_QUEUE_CLAIM_THREADS, 0, cs>>>(slot_problem, bt->nbatch, Q->next, (long long)nproblems, Q->iters,
                                                           Q->status, Q->active, Q->rlast, Q->p_iters, Q->p_status,
@@ -304,9 +246,8 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_restart(NKABATCH bt, void* resid
     else
       nka_queue_rows<1><<<grows, NKA_THREADS, 0, cs>>>(x, ldx, x0, ldx0, xout, ldxout, bt->vlen, Q->move_out, Q->move_in);
     CUDA_CHECK(cudaGetLastError());
-    if (guarded)    // restart the claimed slots and the running ones the rule picks: rmask = claimed | rule
-      nka_loop_guard_restart(bt, cs, restart_growth, Q->active, Q->iters, Q->rlast, Q->claimed, Q->move_out, Q->rprev,
-                             Q->nrst, Q->p_restarts, Q->rmask);
+    if (Q->gamma > 0.0)   // restart the claimed slots and the running ones the rule picks: rmask = claimed | rule
+      nka_solve_guard_restart(*Q, cs, Q->claimed, Q->move_out, Q->p_restarts);
     else
       nka_batch_restart_captured(bt, Q->claimed, cs);
   };
@@ -314,70 +255,40 @@ extern "C" NKABATCHQUEUE nka_batch_queue_create_restart(NKABATCH bt, void* resid
   //   { residual, check, claim, rows, [guard,] restart, update, step }
   auto prologue = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
     reset(cs, bt->nbatch);
-    if (guarded) nka_loop_guard_reset_launch(cs, Q->nrst, bt->nbatch, Q->p_restarts, nproblems);
     claim_rows_restart(cs, cond);
   };
   auto body = [&](cudaStream_t cs, cudaGraphConditionalHandle cond) {
     // check's history stride is 0: every check of slot b writes hist[b], which nothing reads.  It runs after
     // the residual and before claim, so slot_problem[b] is still the problem whose F it checks.
-    nka_loop_queue_check(Vc, gc, bt->nbatch, cs, f, ldf, bt->vlen, /*hstride=*/0, Q->iters, Q->status, Q->active, Q->r0, Q->rlast,
-                         Q->hist, Q->partials, prow, Q->tickets, stop, /*index=*/slot_problem);
+    nka_solve_check(*Q, cs, /*index=*/slot_problem);
     claim_rows_restart(cs, cond);
     nka_batch_update_captured(bt, f, ldf, Q->active, cs);
-    nka_loop_queue_step(Vs, gs, cs, x, ldx, f, ldf, bt->vlen, bt->nbatch, Q->active, Q->iters);
+    nka_solve_step(*Q, cs);
   };
-  Q->exec = nka_while_graph("nka_batch_queue_create", s, (cudaGraph_t)residual_graph, prologue, body);
-  if (!Q->exec) {
-    cudaStreamDestroy(s);
-    queue_free(Q);
-    return nullptr;
-  }
-  CUDA_CHECK(cudaStreamSynchronize(s));
-  CUDA_CHECK(cudaStreamDestroy(s));
-  return Q;
+  return static_cast<NKABATCHQUEUE>(nka_solve_create("nka_batch_queue_create", Q, residual_graph, x, ldx, f, ldf, stop_in,
+                                                     restart_growth, /*history=*/false, init, prologue, body));
 }
 
 extern "C" void nka_batch_queue_launch(NKABATCHQUEUE Q)
 {
   NKA_REQUIRE(Q != NULL, "nka_batch_queue_launch: null queue");
-  DeviceGuard guard(Q->bt->device);
-  if (nka_capture_status(Q->bt->stream) != 0)
-    nka_capture_fail("nka_batch_queue_launch", "a graph with conditional nodes cannot become a child of another graph");
-  CUDA_CHECK(cudaGraphLaunch(Q->exec, Q->bt->stream));
+  nka_solve_launch(Q, "nka_batch_queue_launch");
 }
 
 extern "C" void nka_batch_queue_results(NKABATCHQUEUE Q, int* iters, int* status, double* norm)
 {
   NKA_REQUIRE(Q != NULL && iters != NULL && status != NULL && norm != NULL, "nka_batch_queue_results: null argument");
-  NKABATCH bt = Q->bt;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_queue_results", "it copies the queue's results to the host and synchronises");
   const size_t np = Q->nproblems;
-  CUDA_CHECK(cudaMemcpyAsync(iters, Q->p_iters, np * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaMemcpyAsync(status, Q->p_status, np * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaMemcpyAsync(norm, Q->p_norm, np * sizeof(double), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+  nka_solve_copy_out(Q, "nka_batch_queue_results", "it copies the queue's results to the host and synchronises",
+                     {{iters, Q->p_iters, np * sizeof(int)}, {status, Q->p_status, np * sizeof(int)},
+                      {norm, Q->p_norm, np * sizeof(double)}});
 }
 
 extern "C" void nka_batch_queue_restarts(NKABATCHQUEUE Q, int* restarts)
 {
   NKA_REQUIRE(Q != NULL && restarts != NULL, "nka_batch_queue_restarts: null argument");
-  NKABATCH bt = Q->bt;
-  DeviceGuard guard(bt->device);
-  nka_refuse_capture(bt->stream, "nka_batch_queue_restarts", "it copies the queue's restart counts to the host and synchronises");
-  const size_t np = Q->nproblems;
-  if (!Q->p_restarts) {
-    memset(restarts, 0, np * sizeof(int));
-    return;
-  }
-  CUDA_CHECK(cudaMemcpyAsync(restarts, Q->p_restarts, np * sizeof(int), cudaMemcpyDeviceToHost, bt->stream));
-  CUDA_CHECK(cudaStreamSynchronize(bt->stream));
+  nka_solve_copy_out(Q, "nka_batch_queue_restarts", "it copies the queue's restart counts to the host and synchronises",
+                     {{restarts, Q->p_restarts, Q->nproblems * sizeof(int)}});
 }
 
-extern "C" void nka_batch_queue_destroy(NKABATCHQUEUE Q)
-{
-  if (!Q) return;
-  DeviceGuard guard(Q->bt->device);
-  cudaStreamSynchronize(Q->bt->stream);
-  queue_free(Q);
-}
+extern "C" void nka_batch_queue_destroy(NKABATCHQUEUE Q) { nka_solve_destroy(Q); }

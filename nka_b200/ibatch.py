@@ -7,69 +7,19 @@ calls (INTEGRATION.md section 10).  Device-only and single-GPU.
 """
 from __future__ import annotations
 
-import ctypes as C
-
-import numpy as np
-
-from . import _lib
-from .batch import _mask_address, _state_dict
+from .batch import _Batch
 from .nka import NKAError, _is_torch
 
 MAX_BATCH = 2**31 - 1
 
 
-class InterleavedBatchNKA:
-    """`nbatch` accelerators sharing vlen, mvec and vtol, stored interleaved and updated together."""
-
-    def __init__(self, nbatch: int | None = None, vlen: int | None = None, mvec: int | None = None,
-                 vtol: float = 0.01, device: int = -1, stream: int | None = None):
-        self._h = None
-        self._lib = _lib.load()
-        if nbatch is not None:
-            self.init(nbatch, vlen, mvec, vtol=vtol, device=device, stream=stream)
-
-    # -- life cycle -------------------------------------------------------
-    def init(self, nbatch: int, vlen: int, mvec: int, vtol: float = 0.01, device: int = -1,
-             stream: int | None = None):
-        """Re-initialising frees the previous storage.  Bad arguments raise ValueError before any CUDA call."""
-        if nbatch is None or not 1 <= nbatch <= MAX_BATCH:
-            raise ValueError("nbatch must be in 1..%d" % MAX_BATCH)
-        if vlen is None or vlen < 1:
-            raise ValueError("vlen must be >= 1")
-        if mvec is None or mvec <= 0:
-            raise ValueError("mvec must be > 0")
-        if mvec > _lib.MAX_MVEC:
-            raise ValueError("mvec > %d is not supported by this build" % _lib.MAX_MVEC)
-        if not vtol > 0.0:
-            raise ValueError("vtol must be > 0")
-        self.delete()
-        self._h = self._lib.nka_ibatch_init(nbatch, vlen, mvec, vtol, device, stream)
-        if not self._h:
-            raise NKAError("nka_ibatch_init returned NULL")
-        self.nbatch, self.vlen, self.mvec = nbatch, vlen, mvec
-        return self
-
-    def delete(self):
-        if self._h:
-            self._lib.nka_ibatch_delete(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.delete()
-        except Exception:
-            pass
-
-    def _handle(self):
-        if not self._h:
-            raise NKAError("interleaved batched accelerator is not initialised")
-        return self._h
-
-    def _uncaptured(self, call: str, why: str):
-        h = self._handle()
-        if self._lib.nka_ibatch_stream_capturing(h) != 0:
-            raise NKAError("%s cannot be captured in a CUDA graph: %s" % (call, why))
-        return h
+class InterleavedBatchNKA(_Batch):
+    """`nbatch` accelerators sharing vlen, mvec and vtol, stored interleaved and updated together.  state(b)
+    fills subspace, pending, first, last, free, next, prev, c, h, vtol, min_margin, ndrop_last, evicted_last
+    and relaxed_last; the rest are zero."""
+    _prefix = "nka_ibatch"
+    _max_batch = MAX_BATCH
+    _name = "interleaved batched accelerator"
 
     def _ldf(self, F) -> int:
         """The column stride of F, a CUDA float64 tensor [nbatch, vlen] with unit row stride."""
@@ -98,52 +48,5 @@ class InterleavedBatchNKA:
         overwritten with its accelerated correction.  active: optional length-nbatch CUDA bool / uint8
         tensor; an inactive member's elements of F and its state are left exactly as they are.  Capturable."""
         ldf = self._ldf(F)
-        a = _mask_address(active, self.nbatch, "active")
+        a = self._mask(active, "active")
         self._lib.nka_ibatch_accel_update(self._handle(), F.data_ptr(), ldf, a)
-
-    def relax(self, mask=None) -> None:
-        m = _mask_address(mask, self.nbatch, "mask")
-        self._lib.nka_ibatch_relax(self._handle(), m)
-
-    def restart(self, mask=None) -> None:
-        m = _mask_address(mask, self.nbatch, "mask")
-        self._lib.nka_ibatch_restart(self._handle(), m)
-
-    def set_vec_tol(self, vtol: float) -> None:
-        if not vtol > 0.0:
-            raise ValueError("vtol must be > 0")
-        self._lib.nka_ibatch_set_vec_tol(self._handle(), vtol)
-
-    # -- queries ----------------------------------------------------------
-    def num_vec(self) -> np.ndarray:
-        out = np.zeros(self.nbatch, dtype=np.int32)
-        self._lib.nka_ibatch_num_vec(self._uncaptured("num_vec", "it copies the device state to the host and synchronises"),
-                                     out.ctypes.data_as(C.POINTER(C.c_int)))
-        return out
-
-    def defined(self) -> bool:
-        return bool(self._h) and bool(self._lib.nka_ibatch_defined(
-            self._uncaptured("defined", "it copies the device state to the host and synchronises")))
-
-    def state(self, b: int) -> dict:
-        """Member b's state, with the keys and layout of NKA.state().  Filled: subspace, pending, first, last,
-        free, next, prev, c, h, vtol, min_margin, ndrop_last, evicted_last, relaxed_last; the rest are zero."""
-        if not 0 <= b < self.nbatch:
-            raise ValueError("member index out of range")
-        v = _lib.StateView()
-        self._lib.nka_ibatch_get_state(self._uncaptured("state", "it copies the device state to the host and synchronises"),
-                                       b, C.byref(v))
-        return _state_dict(v)
-
-    def set_stream(self, stream: int | None):
-        """The stream every later call is queued on; set the capture stream here before a capture begins."""
-        self._lib.nka_ibatch_set_stream(self._uncaptured("set_stream", "it synchronises the handle's stream"), stream)
-
-    def synchronize(self):
-        self._lib.nka_ibatch_synchronize(self._uncaptured("synchronize", "it synchronises the handle's stream"))
-
-    def stream_capturing(self) -> int:
-        return self._lib.nka_ibatch_stream_capturing(self._handle())
-
-    def launch_count(self) -> int:
-        return self._lib.nka_ibatch_launch_count(self._handle())
